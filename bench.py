@@ -35,6 +35,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "M alignments/s filter+besthit+profile"
 FILTER = dict(l=80, p=95, z=80)
@@ -565,6 +566,44 @@ def parity_check(m, cfg, plan, tlen, rank, world, local, dist, bcast):
     return ok, res
 
 
+# ------------------------------------------------------------------------------------------------ output dump
+DUMP_LIMIT = 64_000_000             # bytes of .npy files in all
+
+
+def step_outputs(ctx, cfg, out, kept):
+    """What a caller of the timed step receives, by name: the profile (abundance vector and statistics) or the coverage
+    summary of the whole step, whichever the config asks for, and the kept-record count and (when the config outputs
+    records) the filtered record bytes of the step's last chunk, the only chunk they are kept for."""
+    res = {"kept_records_last_chunk": kept}
+    if cfg["ctx"].get("profile"):
+        ab, st = out
+        res["abundance"] = ab
+        res.update({"profile_" + k: v for k, v in st.items()})
+    elif cfg["ctx"].get("coverage"):
+        res.update(zip(("coverage_covered", "coverage_touched", "coverage_total"), out))
+    if cfg["ctx"].get("records"):
+        res["records_last_chunk"] = ctx.pull_records()[0]
+    return res
+
+
+def dump_outputs(path, arrays):
+    """Every array as <path>/<name>.npy in float64 (byte data in float32; both hold the values exactly).  An array that does
+    not fit in what is left of DUMP_LIMIT is replaced by a sample of its elements at positions drawn with the workload's seed,
+    and the positions go to <name>_sample_index.npy, so that two builds run with the same arguments dump the same elements."""
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_LIMIT - 256 * (len(arrays) + 1)            # room for the .npy headers
+    for name, a in sorted(arrays.items(), key=lambda kv: np.size(kv[1])):
+        a = np.asarray(a)
+        dt = np.dtype(np.float32 if a.dtype == np.uint8 else np.float64)
+        if a.size * dt.itemsize > left:
+            idx = np.unique(np.random.default_rng(SEED).integers(0, a.size, left // (dt.itemsize + 8)))
+            np.save(os.path.join(path, name + "_sample_index.npy"), idx.astype(np.float64))
+            left -= idx.size * 8
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a.astype(dt))
+        left -= a.size * dt.itemsize
+
+
 # ------------------------------------------------------------------------------------------------ our arm
 def run_ours(args):
     import msamtools_b200 as m
@@ -711,6 +750,8 @@ def run_ours(args):
     wall_step_ms = max_over_ranks(wall_ms / args.steps)
     n_total = sum_over_ranks(n_local)
     value = n_total / (step_ms * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_outputs(ctx, cfg, out, kept_last))
 
     # the job's own result must be the same bits on every rank, and obey the conservation laws of the profile
     job_check = {}
@@ -853,7 +894,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-ingest", action="store_true", help="skip the BGZF file-to-result (host ingest) leg")
     ap.add_argument("--cpu-port", action="store_true", help="time the in-memory oracle port even when oracle/_ref exists")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as DIR/<name>.npy "
+                                                          "(float32/float64, at most 64 MB in all; a larger output is sampled): the "
+                                                          "step's profile or coverage summary, and the kept count and records of its "
+                                                          "last chunk")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

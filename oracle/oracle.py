@@ -4,6 +4,7 @@ Imported by tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl
 legs -- never by anything under msamtools_b200/.
 """
 import ctypes as C
+import json
 import os
 import subprocess
 
@@ -34,6 +35,16 @@ class OracleError(RuntimeError):
 
 
 _lib = None
+
+
+def reference_dir():
+    """The checkout of the reference msamtools sources that oracle/Makefile.ref compiles: MSAMTOOLS_REFERENCE if set, else
+    BASELINE.json's reference_path; None when that directory does not exist."""
+    d = os.environ.get("MSAMTOOLS_REFERENCE")
+    if not d:
+        with open(os.path.join(_HERE, "..", "BASELINE.json")) as fh:
+            d = json.load(fh).get("reference_path", "")
+    return d if d and os.path.isdir(d) else None
 
 
 def build():

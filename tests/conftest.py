@@ -8,20 +8,17 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
-REF_TESTS = "/root/reference/tests"           # only exists in the build container, never on the GPU box
+# The checkout of the reference msamtools v1.1.3 sources (not part of this repository), or None: the tests that run the
+# reference's shell suites need it and skip without it.
+from oracle import oracle as _orc  # noqa: E402
+
+REFERENCE = _orc.reference_dir()
+REF_TESTS = os.path.join(REFERENCE, "tests") if REFERENCE else ""
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu under gpurun)")
-
-
-def have_gpu():
-    try:
-        import msamtools_b200 as m
-        return m._lib.load().msg_device_count() > 0
-    except Exception:
-        return False
+    config.addinivalue_line("markers", "gpu: needs a B200")
 
 
 @pytest.fixture(scope="session")
@@ -32,4 +29,4 @@ def oracle():
     return orc
 
 
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="/root/reference not present (GPU box)")
+needs_reference = pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="the reference's sources are absent (MSAMTOOLS_REFERENCE, BASELINE.json reference_path)")

@@ -1,14 +1,16 @@
 #!/usr/bin/env python
-"""Generates tests/golden/fixtures.npz + cases.json.  Run in the build container only:
+"""Generates tests/golden/fixtures.npz + cases.json from a checkout of the reference's sources (MSAMTOOLS_REFERENCE, else
+BASELINE.json's reference_path):
 
     python tests/golden/make_golden.py
 
-Inputs are the reference's own test fixtures (tests/fixtures/*.sam, tests/tiny_aln.bam under
-/root/reference), re-encoded as raw BAM record streams (the C-ABI input layout).  Expected
+Inputs are the reference's own test fixtures (tests/fixtures/*.sam, tests/tiny_aln.bam of that
+checkout), re-encoded as raw BAM record streams (the C-ABI input layout).  Expected
 outputs are (a) the strings the reference's test scripts assert (restated with citations in
-tests/test_oracle_golden.py) and (b) the outputs of the pinned CPU oracle -- and, when
-oracle/_ref/msamtools has been built, of the reference's own object code (tests/test_ref_binary.py
-checks that (b) agrees with it).  /root/reference does not exist on the GPU box; these files travel.
+tests/test_oracle_golden.py, which asserts them again) and (b) the outputs of the pinned CPU
+oracle, which (a) pins.  The reference's object code itself is not run here: its outputs on
+seeded synthetic streams are what tests/golden/make_golden_streams.py stores.  The tests read
+these files, so they need no reference checkout.
 """
 import json
 import os
@@ -24,7 +26,7 @@ import samutil                                    # noqa: E402
 from oracle import oracle as orc                  # noqa: E402
 import test_oracle_golden as T                    # noqa: E402
 
-REF = "/root/reference/tests"
+REF = os.path.join(orc.reference_dir(), "tests")
 FIXTURES = ["filter", "cigar_eqx", "besthit", "besthit_rescore", "long_qname", "profile", "profile_empty",
             "profile_unmapped", "profile_fractional_mincount", "coverage", "integration", "qname_coordinate", "qname_reopened"]
 

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import msamtools_b200 as m
-from conftest import ROOT, have_gpu
+from conftest import ROOT
 
 
 def declared_symbols():
@@ -54,12 +54,23 @@ def test_struct_layout_matches_header(tmp_path):
             assert got[f"{cname}.{fname}"] == [f.offset, f.size], f"{cname}.{fname}"
 
 
-@pytest.mark.skipif(have_gpu(), reason="a GPU is present")
 def test_no_cpu_fallback():
-    with pytest.raises(m.MsgError) as e:
-        m.Context(l=80, n_targets=1)
-    assert e.value.code == m._lib.MSG_ENODEV
-    assert "no CPU fallback" in e.value.text
+    # in a child process that sees no CUDA device (none installed, or all of them hidden from it)
+    import subprocess
+    import sys
+    code = ("import msamtools_b200 as m\n"
+            "try:\n"
+            "    m.Context(l=80, n_targets=1)\n"
+            "    print('created')\n"
+            "except m.MsgError as e:\n"
+            "    print(e.code, e.text)\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, check=True)
+    out = r.stdout.strip()
+    assert out != "created", "a context was created without a CUDA device"
+    rc, text = out.split(" ", 1)
+    assert int(rc) == m._lib.MSG_ENODEV
+    assert "no CPU fallback" in text
 
 
 def test_product_does_not_import_oracle():

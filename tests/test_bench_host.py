@@ -46,6 +46,29 @@ def test_small_chunk_is_a_prefix_of_the_full_chunk():
     assert 5_000 <= n < 5_100 and np.array_equal(poff, foff[:n + 1]) and np.array_equal(part, full[:int(poff[-1])])
 
 
+def test_dump_outputs_exact_bounded_and_repeatable(tmp_path, monkeypatch):
+    """--dump-outputs: values exact in float64 (bytes in float32); an output past the size limit is replaced by a sample
+    taken at the same positions on every run"""
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 200_000)
+    rng = np.random.default_rng(3)
+    arrays = {"abundance": rng.random(5_000), "kept_records_last_chunk": 123_456, "profile_delta": [0.5, 0.25], "profile_converged": 1,
+              "records_last_chunk": rng.integers(0, 256, 1_000_000, dtype=np.uint8)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) == sorted([k + ".npy" for k in arrays] + ["records_last_chunk_sample_index.npy"])
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in names) <= 200_000
+    for f in names:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == (np.float32 if f == "records_last_chunk.npy" else np.float64) and np.array_equal(a, b)
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in names}
+    assert np.array_equal(got["abundance"], arrays["abundance"]) and got["kept_records_last_chunk"] == 123_456
+    assert got["profile_delta"].tolist() == [0.5, 0.25] and got["profile_converged"] == 1
+    idx = got["records_last_chunk_sample_index"].astype(np.int64)
+    assert len(idx) > 1000 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(got["records_last_chunk"], arrays["records_last_chunk"][idx])
+
+
 def test_reference_arm_runs_on_the_host(tmp_path):
     if not bench.have_ref_binary():
         pytest.skip("oracle/_ref not built")

@@ -1,6 +1,6 @@
 """CPU: the oracle must reproduce every committed golden case (tests/golden/), so the bundle the
 GPU parity tests rely on cannot drift from the pinned oracle.  Runs everywhere (no GPU, no
-/root/reference)."""
+reference sources)."""
 import numpy as np
 import pytest
 

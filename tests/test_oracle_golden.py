@@ -1,19 +1,14 @@
 """Pins the CPU oracle against the expected values written in the reference's OWN test
-scripts, on the reference's own fixtures (read in place from /root/reference/tests; these
-tests skip on the GPU box, where tests/golden/ carries the same vectors).
+scripts, on the reference's own fixtures (tests/fixtures/*.sam and tests/tiny_aln.bam of
+msamtools v1.1.3, stored as record streams in tests/golden/fixtures.npz).
 
 Every expected string below is restated from the cited reference test, not computed here.
 """
-import os
-
 import numpy as np
 import pytest
 
+import goldenutil as G
 import samutil
-from conftest import REF_TESTS, needs_reference
-
-pytestmark = needs_reference
-FX = os.path.join(REF_TESTS, "fixtures")
 
 # tests/test_filter.sh:15
 ALL_MAPPED = ("clip80:0,clip90:0,del99:0,id97:0,id98:0,ins99:0,len80:0,md99:0,md_precedence:0,pairX:65,pairX:129,"
@@ -74,14 +69,14 @@ def _run_filter(oracle, sam, **opts):
 
 @pytest.mark.parametrize("opts,expected", FILTER_CASES)
 def test_filter_fixture(oracle, opts, expected):
-    sam = samutil.read_sam(os.path.join(FX, "filter.sam"))
+    sam = G.fixture("filter")
     idx, _ = _run_filter(oracle, sam, **opts)
     assert sam.name_flags(idx) == expected
 
 
 @pytest.mark.parametrize("opts,expected", EQX_CASES)
 def test_cigar_eqx_fixture(oracle, opts, expected):
-    sam = samutil.read_sam(os.path.join(FX, "cigar_eqx.sam"))
+    sam = G.fixture("cigar_eqx")
     idx, _ = _run_filter(oracle, sam, **opts)
     assert sam.name_flags(idx) == expected
 
@@ -108,7 +103,7 @@ def _aux_text(rec, tag):
 
 def test_filter_rescore_values(oracle):
     # tests/test_filter.sh:153-163: id98 -> AS:i:96, md_precedence -> AS:i:100
-    sam = samutil.read_sam(os.path.join(FX, "filter.sam"))
+    sam = G.fixture("filter")
     idx, cfg = _run_filter(oracle, sam, p=98, rescore=True)
     recs = samutil.split_records(oracle.emit_records(sam.raw, sam.off, idx, cfg))
     by_name = {sam.record_fields(int(i))[0]: r for i, r in zip(idx, recs)}
@@ -120,7 +115,7 @@ def test_filter_rescore_values(oracle):
 
 @pytest.mark.parametrize("fixture,opts,expected", BESTHIT_CASES)
 def test_besthit_fixture(oracle, fixture, opts, expected):
-    sam = samutil.read_sam(os.path.join(FX, fixture))
+    sam = G.fixture(fixture.replace(".sam", ""))
     idx, cfg = _run_filter(oracle, sam, **opts)
     assert sam.name_flags(idx) == expected
     if opts.get("rescore"):
@@ -132,7 +127,7 @@ def test_besthit_fixture(oracle, fixture, opts, expected):
 @pytest.mark.parametrize("opts", [dict(besthit=True), dict(p=90, besthit=True)])
 def test_long_qname_besthit(oracle, opts):
     # tests/test_besthit.sh:85-128: one winner per complete 127/128/254-char QNAME
-    sam = samutil.read_sam(os.path.join(FX, "long_qname.sam"))
+    sam = G.fixture("long_qname")
     idx, _ = _run_filter(oracle, sam, **opts)
     got = [(len(sam.record_fields(int(i))[0]), sam.record_fields(int(i))[1], sam.ref_names[sam.record_fields(int(i))[2]]) for i in idx]
     assert got == [(127, 0, "A"), (128, 0, "A"), (254, 0, "A"), (254, 0, "B")]
@@ -144,7 +139,7 @@ PROFILE_CASES = [("all", 0, 6, 2), ("equal", 0, 5.5, 1.5), ("ignore", 1, 5, 1), 
 
 @pytest.mark.parametrize("mode,unknown,a,b", PROFILE_CASES)
 def test_profile_fixture(oracle, mode, unknown, a, b):
-    sam = samutil.read_sam(os.path.join(FX, "profile.sam"))
+    sam = G.fixture("profile")
     share = {"all": 1, "equal": 2, "proportional": 3, "ignore": 4}[mode]
     ab, st, _, _ = oracle.profile(sam.raw, sam.off, None, len(sam.ref_names), share)
     assert (st["mapped_inserts"], st["multi"], st["uniq"]) == (7, 1, 6)             # test_profile.sh:38-46
@@ -156,7 +151,7 @@ def test_profile_fixture(oracle, mode, unknown, a, b):
 
 def test_profile_long_qname(oracle):
     # tests/test_profile.sh:69-97
-    sam = samutil.read_sam(os.path.join(FX, "long_qname.sam"))
+    sam = G.fixture("long_qname")
     ab, st, _, _ = oracle.profile(sam.raw, sam.off, None, len(sam.ref_names), 2)
     assert (st["mapped_inserts"], st["multi"], st["uniq"]) == (4, 4, 0)
     assert abs(ab[0] - 2) <= 1e-9 and abs(ab[1] - 2) <= 1e-9
@@ -165,7 +160,7 @@ def test_profile_long_qname(oracle):
 @pytest.mark.parametrize("fixture", ["profile_empty.sam", "profile_unmapped.sam"])
 def test_profile_zero(oracle, fixture):
     # tests/test_profile.sh:99-137
-    sam = samutil.read_sam(os.path.join(FX, fixture))
+    sam = G.fixture(fixture.replace(".sam", ""))
     ab, st, _, _ = oracle.profile(sam.raw, sam.off, None, len(sam.ref_names), 2)
     assert (st["mapped_inserts"], st["multi"], st["uniq"]) == (0, 0, 0)
     assert not ab.any()
@@ -173,14 +168,14 @@ def test_profile_zero(oracle, fixture):
 
 def test_profile_fractional(oracle):
     # tests/test_profile.sh:139-160: equal sharing -> A 1.3333 B 1.3333 C 0.3333
-    sam = samutil.read_sam(os.path.join(FX, "profile_fractional_mincount.sam"))
+    sam = G.fixture("profile_fractional_mincount")
     ab, st, _, _ = oracle.profile(sam.raw, sam.off, None, len(sam.ref_names), 2)
     assert np.allclose(ab[:3], [4 / 3, 4 / 3, 1 / 3], atol=1e-6)
 
 
 def test_coverage_fixture(oracle):
     # tests/test_coverage.sh:28-62
-    sam = samutil.read_sam(os.path.join(FX, "coverage.sam"))
+    sam = G.fixture("coverage")
     cov, touched, total, depth = oracle.coverage(sam.raw, sam.off, None, sam.target_len, want_depth=True)
     assert depth[0].tolist() == [1, 0, 1, 1, 2, 2, 1, 0, 0, 1]
     assert depth[1].tolist() == [0] * 5
@@ -196,7 +191,7 @@ def test_coverage_fixture(oracle):
 
 def test_integration(oracle):
     # tests/test_integration.sh:38-72: filter -p 95 | profile --multi equal
-    sam = samutil.read_sam(os.path.join(FX, "integration.sam"))
+    sam = G.fixture("integration")
     ab, st, _, _ = oracle.profile(sam.raw, sam.off, None, 2, 2)
     assert (st["multi"], st["uniq"]) == (2, 2) and np.allclose(ab, [2, 2], atol=1e-9)
     idx, _ = _run_filter(oracle, sam, p=95)
@@ -207,7 +202,7 @@ def test_integration(oracle):
 
 def test_tiny_aln_config1(oracle):
     # BASELINE.json configs[0]: filter -l 80 -p 95 -z 80 --besthit | profile --multi=proportional
-    sam = samutil.read_bam(os.path.join(REF_TESTS, "tiny_aln.bam"))
+    sam = G.fixture("tiny_aln")
     assert sam.n == 16 and len(sam.ref_names) == 2924
     idx, _ = _run_filter(oracle, sam, l=80, p=95, z=80, besthit=True)
     assert len(idx) == 14

@@ -1,30 +1,38 @@
 """oracle/_ref = the reference's OWN object code (its unmodified C sources compiled against the
-shims in oracle/shim/).  These tests run only where /root/reference exists (build container):
+shims in oracle/shim/ by oracle/Makefile.ref, where the reference's sources are present):
 
-1. the reference's ten `make check` suites pass against it  -> the shim is faithful;
-2. the CPU oracle (our restatement) agrees with it on seeded synthetic streams -> the oracle is
-   pinned against the reference itself, not only against its test fixtures.
+1. the reference's ten `make check` suites pass against it (needs the reference's sources) -> the shim is faithful;
+2. the CPU oracle (our restatement) agrees with it on seeded synthetic streams (needs the binary) -> the oracle is
+   pinned against the reference itself, not only against its test fixtures;
+3. on every machine, the oracle reproduces what (2) compares, as stored in tests/golden/streams.json
+   (tests/golden/make_golden_streams.py).  Where (2) runs too, the stored data is checked against the reference.
 """
 import gzip
+import hashlib
+import json
 import os
+import re
 import subprocess
 
 import numpy as np
 import pytest
 
 import samutil
-from conftest import REF_TESTS, ROOT, needs_reference
+from conftest import GOLDEN, REF_TESTS, REFERENCE, ROOT, needs_reference
 
-pytestmark = needs_reference
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "msamtools")
 
 
 @pytest.fixture(scope="module")
 def ref_bin():
-    subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "-f", "Makefile.ref"])
+    if REFERENCE:
+        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "-f", "Makefile.ref", "REF=" + REFERENCE])
+    if not os.access(REF_BIN, os.X_OK):
+        pytest.skip("no reference object code: oracle/_ref/msamtools is not built and the reference's sources are absent")
     return REF_BIN
 
 
+@needs_reference
 @pytest.mark.parametrize("suite", ["smoke", "filter", "besthit", "profile", "coverage", "integration", "qname_order",
                                    "errors", "streaming", "summary"])
 def test_reference_suite_passes_on_ref_binary(ref_bin, suite, tmp_path):
@@ -43,16 +51,22 @@ STREAMS = {"mixed": ("mixed", 40_000, 424242, {}),
 
 
 @pytest.fixture(scope="module", params=list(STREAMS))
-def synth_bam(request, tmp_path_factory):
+def synth_stream(request):
     from msamtools_b200 import synth
     preset, nrec, seed, over = STREAMS[request.param]
     p = synth.make_params(preset, n_records=nrec, seed=seed, **over)
     raw, off, _ = synth.generate(p)
     tlen = synth.target_lengths(p)
     names = [f"ref{i:04d}" for i in range(len(tlen))]
+    return request.param, raw, off, tlen, names
+
+
+@pytest.fixture(scope="module")
+def synth_bam(synth_stream, tmp_path_factory):
+    _, raw, off, tlen, names = synth_stream
     path = str(tmp_path_factory.mktemp("synth") / "in.bam")
     samutil.write_bam(path, samutil.synth_header(names, tlen), names, tlen, raw)
-    return path, raw, off, tlen, names
+    return (path,) + synth_stream[1:]
 
 
 FILTERS = [(["-l", "80", "-p", "95", "-z", "80"], dict(l=80, p=95, z=80)),
@@ -61,6 +75,8 @@ FILTERS = [(["-l", "80", "-p", "95", "-z", "80"], dict(l=80, p=95, z=80)),
            (["--ppt", "-990"], dict(ppt=-990)),
            (["-p", "99", "-v", "-k"], dict(p=99, invert=True, keep_unmapped=True)),
            (["-l", "100", "--rescore", "--besthit"], dict(l=100, rescore=True, besthit=True))]
+MODES = ["all", "equal", "proportional", "ignore"]
+PRE_ARGV, PRE_OPTS = ["-l", "80", "-p", "95", "-z", "80", "--besthit"], dict(l=80, p=95, z=80, besthit=True)   # filter | profile
 
 
 def _payload(bam_bytes):
@@ -75,53 +91,124 @@ def _payload(bam_bytes):
     return data[o:]
 
 
+# ---- one output of each command, from the reference's object code and from the oracle, in the same form
+def reference_filter(ref_bin, path, argv):
+    return _payload(subprocess.run([ref_bin, "filter", "-b", "-u"] + argv + [path], capture_output=True, check=True).stdout)
+
+
+def oracle_filter(oracle, raw, off, opts):
+    cfg = oracle.filter_cfg(**opts)
+    return bytes(oracle.emit_records(raw, off, oracle.filter_stream(raw, off, cfg), cfg))
+
+
+def reference_profile(ref_bin, path, names, mode, pre, outp):
+    """the three insert counts of the table's comments, every feature's value as printed, and for proportional sharing the
+    PropSharing iterations and purged inserts reported on stderr"""
+    prof = [ref_bin, "profile", "--label", "x", "--unit", "ab", "--nolen", "--multi", mode, "-o", outp]
+    if pre:
+        f = subprocess.Popen([ref_bin, "filter", "-b", "-u"] + PRE_ARGV + [path], stdout=subprocess.PIPE)
+        r = subprocess.run(prof + ["-"], stdin=f.stdout, capture_output=True, text=True)
+        f.wait()
+    else:
+        r = subprocess.run(prof + [path], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
+    comments, body = samutil.read_profile_gz(outp)
+    res = {}
+    for key, label in (("mapped_inserts", "Mapped inserts"), ("multi", "- Multiple mapped "), ("uniq", "- Uniquely mapped ")):
+        res[key] = int(next(l for l in comments if label in l).split(":")[1].split("(")[0])
+    got = {k: v for k, v in body[1:]}
+    res["values"] = [got[n] for n in names]
+    if mode == "proportional":
+        res["iterations"] = sum("PropSharing Iteration" in l for l in r.stderr.splitlines())
+        m = re.search(r"Purged (\d+) inserts", r.stderr)
+        res["purged"] = int(m.group(1)) if m else None
+    return res
+
+
+def oracle_profile(oracle, raw, off, n_targets, mode, pre):
+    idx = oracle.filter_stream(raw, off, oracle.filter_cfg(**PRE_OPTS)) if pre else None
+    ab, st, _, _ = oracle.profile(raw, off, idx, n_targets, {"all": 1, "equal": 2, "proportional": 3, "ignore": 4}[mode])
+    res = {"mapped_inserts": st["mapped_inserts"], "multi": st["multi"], "uniq": st["uniq"], "values": ["%.8g" % x for x in ab]}
+    if mode == "proportional":
+        res.update(iterations=st["iterations"], purged=st["purged"])
+    return res
+
+
+def reference_coverage(ref_bin, path, outp):
+    subprocess.run([ref_bin, "coverage", "--summary", "-o", outp, path], check=True)
+    with gzip.open(outp, "rt") as fh:
+        return fh.read().splitlines()
+
+
+def oracle_coverage(oracle, raw, off, tlen, names):
+    cov, touched, total, _ = oracle.coverage(raw, off, None, tlen)
+    return ["%s\t0\t0" % n if not cov[t] else "%s\t%.8f\t%.2f" % (n, touched[t] / int(tlen[t]), total[t] / int(tlen[t]))
+            for t, n in enumerate(names)]
+
+
+def stored_form(result):
+    """What tests/golden/streams.json keeps of one output: record bytes as count, size and SHA-256; a list of printed rows
+    as count, SHA-256 of the rows and 32 rows at seeded positions; the counters of a profile as they are."""
+    if isinstance(result, bytes):
+        return {"records": len(samutil.split_records(result)), "bytes": len(result), "sha256": hashlib.sha256(result).hexdigest()}
+    if isinstance(result, dict):
+        return {k: stored_form(v) if k == "values" else v for k, v in result.items()}
+    pick = np.sort(np.random.default_rng(97).choice(len(result), min(32, len(result)), replace=False))
+    return {"rows": len(result), "sha256": hashlib.sha256("\n".join(result).encode()).hexdigest(),
+            "sample": {str(i): result[i] for i in pick}}
+
+
+def filter_key(stream, argv):
+    return f"{stream} | filter {' '.join(argv)}"
+
+
+def profile_key(stream, mode, pre):
+    return f"{stream} | {'filter | ' if pre else ''}profile --multi {mode}"
+
+
+def coverage_key(stream):
+    return f"{stream} | coverage --summary"
+
+
+# ---- (2) the oracle against the reference's object code
 @pytest.mark.parametrize("argv,opts", FILTERS, ids=lambda x: " ".join(x) if isinstance(x, list) else "")
 def test_oracle_filter_equals_reference(ref_bin, oracle, synth_bam, argv, opts):
     path, raw, off, tlen, names = synth_bam
-    out = subprocess.run([ref_bin, "filter", "-b", "-u"] + argv + [path], capture_output=True, check=True).stdout
-    cfg = oracle.filter_cfg(**opts)
-    idx = oracle.filter_stream(raw, off, cfg)
-    assert _payload(out) == bytes(oracle.emit_records(raw, off, idx, cfg))
+    assert reference_filter(ref_bin, path, argv) == oracle_filter(oracle, raw, off, opts)
 
 
-@pytest.mark.parametrize("mode", ["all", "equal", "proportional", "ignore"])
+@pytest.mark.parametrize("mode", MODES)
 @pytest.mark.parametrize("pre", [None, 1], ids=["plain", "filter|profile"])
 def test_oracle_profile_equals_reference(ref_bin, oracle, synth_bam, mode, pre, tmp_path):
     path, raw, off, tlen, names = synth_bam
-    outp = str(tmp_path / "p.gz")
-    prof = [ref_bin, "profile", "--label", "x", "--unit", "ab", "--nolen", "--multi", mode, "-o", outp]
-    if pre:
-        f = subprocess.Popen([ref_bin, "filter", "-b", "-u", "-l", "80", "-p", "95", "-z", "80", "--besthit", path], stdout=subprocess.PIPE)
-        r = subprocess.run(prof + ["-"], stdin=f.stdout, capture_output=True, text=True)
-        f.wait()
-        idx = oracle.filter_stream(raw, off, oracle.filter_cfg(l=80, p=95, z=80, besthit=True))
-    else:
-        r = subprocess.run(prof + [path], capture_output=True, text=True)
-        idx = None
-    assert r.returncode == 0, r.stderr
-    share = {"all": 1, "equal": 2, "proportional": 3, "ignore": 4}[mode]
-    ab, st, _, _ = oracle.profile(raw, off, idx, len(tlen), share)
-    comments, body = samutil.read_profile_gz(outp)
-    text = "\n".join(comments)
-    for label, val in (("Mapped inserts", st["mapped_inserts"]), ("- Multiple mapped ", st["multi"]), ("- Uniquely mapped ", st["uniq"])):
-        line = next(l for l in comments if label in l)
-        assert int(line.split(":")[1].split("(")[0]) == val, line
-    got = {k: v for k, v in body[1:]}
-    for i, n in enumerate(names):
-        assert got[n] == "%.8g" % ab[i], (n, got[n], ab[i])
-    if mode == "proportional":
-        iters = [l for l in r.stderr.splitlines() if "PropSharing Iteration" in l]
-        assert len(iters) == st["iterations"]
-        assert f"Purged {st['purged']} inserts" in r.stderr
+    assert reference_profile(ref_bin, path, names, mode, pre, str(tmp_path / "p.gz")) == oracle_profile(oracle, raw, off, len(tlen), mode, pre)
 
 
 def test_oracle_coverage_equals_reference(ref_bin, oracle, synth_bam, tmp_path):
     path, raw, off, tlen, names = synth_bam
-    outp = str(tmp_path / "c.gz")
-    subprocess.run([ref_bin, "coverage", "--summary", "-o", outp, path], check=True)
-    cov, touched, total, _ = oracle.coverage(raw, off, None, tlen)
-    with gzip.open(outp, "rt") as fh:
-        lines = fh.read().splitlines()
-    exp = ["%s\t0\t0" % n if not cov[t] else "%s\t%.8f\t%.2f" % (n, touched[t] / int(tlen[t]), total[t] / int(tlen[t]))
-           for t, n in enumerate(names)]
-    assert lines == exp
+    assert reference_coverage(ref_bin, path, str(tmp_path / "c.gz")) == oracle_coverage(oracle, raw, off, tlen, names)
+
+
+# ---- (3) the oracle against the stored outputs, everywhere
+@pytest.fixture(scope="module")
+def stored():
+    with open(os.path.join(GOLDEN, "streams.json")) as fh:
+        return json.load(fh)["outputs"]
+
+
+@pytest.mark.parametrize("argv,opts", FILTERS, ids=lambda x: " ".join(x) if isinstance(x, list) else "")
+def test_oracle_filter_equals_stored(oracle, stored, synth_stream, argv, opts):
+    stream, raw, off, tlen, names = synth_stream
+    assert stored_form(oracle_filter(oracle, raw, off, opts)) == stored[filter_key(stream, argv)]
+
+
+@pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("pre", [None, 1], ids=["plain", "filter|profile"])
+def test_oracle_profile_equals_stored(oracle, stored, synth_stream, mode, pre):
+    stream, raw, off, tlen, names = synth_stream
+    assert stored_form(oracle_profile(oracle, raw, off, len(tlen), mode, pre)) == stored[profile_key(stream, mode, pre)]
+
+
+def test_oracle_coverage_equals_stored(oracle, stored, synth_stream):
+    stream, raw, off, tlen, names = synth_stream
+    assert stored_form(oracle_coverage(oracle, raw, off, tlen, names)) == stored[coverage_key(stream)]
