@@ -31,7 +31,21 @@
  * by block_size bytes (SAM spec 4.2) -- plus a host-built index
  * rec_off[0..nrec] of byte offsets of each record's block_size field
  * (rec_off[nrec] = end of the last record).  A chunk must end on a QNAME
- * boundary (see msg_split_point) so that no read group straddles chunks/GPUs.
+ * boundary (see msg_split_point) so that no read group straddles chunks/GPUs --
+ * except on a context created with `collate`, which takes records in any order.
+ *
+ * Collating contexts (msg_config.collate = 1)
+ *   - chunks need not end on a QNAME boundary; a read's records may be spread over any number of pushes.
+ *   - msg_push* append the records' heads (everything but SEQ/QUAL) to device memory and complete before returning.
+ *     More than 2^32-2 records (or 64 GiB of heads) in one scope: MSG_ERANGE; no room on the device: MSG_ENOMEM.
+ *   - the first msg_finish_profile / msg_finish_coverage / msg_pull_counts after pushes groups everything held by
+ *     QNAME (equal l_read_name and bytes) and runs the pipeline once for every consumer; later calls reuse it.
+ *     A push after that starts a new scope whose records add to the same accumulators.  msg_reset drops held records.
+ *   - integers equal, and f64 values agree to rounding with, those of the same records reordered so that each
+ *     QNAME's records are contiguous and keep their input order.
+ *   - msg_kept_count, msg_pull_kept, msg_pull_records and msg_pull_stats return MSG_ESTATE.
+ *   - errors found after grouping (MSG_ENOTAG, MSG_ENOAS, MSG_EFORMAT) name the record's input ordinal (0-based,
+ *     counted over the scope's pushes) in msg_last_error.
  */
 #ifndef MSAMTOOLS_B200_H
 #define MSAMTOOLS_B200_H
@@ -85,7 +99,12 @@ typedef struct msg_config {
     uint8_t  invert;             /* -v                                                 */
     uint8_t  keep_unmapped;      /* -k                                                 */
     uint8_t  rescore;            /* --rescore                                          */
-    uint8_t  reserved0[3];
+    uint8_t  collate;            /* records may come in any order (e.g. sorted by coordinate): the context keeps their
+                                    heads (no SEQ/QUAL) on the device and groups them by QNAME at the first
+                                    msg_finish_profile / msg_finish_coverage after pushes.  Needs want_profile and/or
+                                    want_coverage, n_ranks == 1; not with want_records / want_kept / want_stats.
+                                    Results equal those of the same records regrouped stably by QNAME (see below).    */
+    uint8_t  reserved0[2];
     int32_t  min_length;         /* -l  (MIN_LENGTH, msam_filter.c:449-457)            */
     int32_t  ppt;                /* 10*-p or --ppt (PPT, msam_filter.c:420-437)        */
     int32_t  max_clip;           /* 100 - z; 100 when -z absent (MAX_CLIP, :439-447)   */

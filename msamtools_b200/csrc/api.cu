@@ -9,6 +9,7 @@
 #include "coverage.cuh"
 #include "gather.cuh"
 #include "fused.cuh"
+#include "collate.cuh"
 
 #include <nccl.h>        // types only; the library itself is dlopen'ed (no link-time dependency)
 #include <dlfcn.h>
@@ -157,6 +158,13 @@ struct msg_ctx {
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev_decode, ev_total;
     std::vector<cudaEvent_t> ev_free;
     cudaEvent_t marks[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    uint32_t err_rec = 0xffffffffu;            // record index of the last error reported (d_err[1]), 0xffffffff if none
+
+    // collation (cfg.collate, collate.cuh): record heads held on the device until a finish groups them by QNAME
+    DevBuf coll_arena, coll_aoff, coll_keys, coll_keys2, coll_len, coll_hist, coll_bstart, coll_list, coll_grouped, coll_goff;
+    uint64_t coll_n = 0, coll_bytes = 0;       // records and head bytes held in this scope
+    bool coll_dirty = false;                   // pushes since the last collation
+    bool coll_done = false;                    // a finish collated this scope: the next push starts a new one
     double decode_ms = 0, total_ms = 0; uint64_t decode_launches = 0, kernel_launches = 0;
     uint64_t h2d_bytes = 0, d2h_bytes = 0;
 };
@@ -231,6 +239,7 @@ int check_device_errors(msg_ctx *c)
 
 int report_device_errors(msg_ctx *c, const uint32_t *h)
 {
+    c->err_rec = h[1];
     if (h[0]) {                   // reported once: the next chunk starts with a clean error word
         cudaMemsetAsync(c->d_err, 0, 4, c->stream);
         cudaMemsetAsync(c->d_err + 1, 0xff, 4, c->stream);
@@ -705,6 +714,197 @@ int push_chunk(msg_ctx *c, const uint8_t *h_raw, const uint8_t *dev_raw, size_t 
     return run_chunk_general(c, d_raw, nbytes, readable, sl.d_off, nrec, h_raw, h_off);
 }
 
+// ------------------------------------------------------------------------------------------------ collation (collate.cuh)
+// MSG_COLLATE_HASH_BITS=k keeps the top k bits of the 64-bit QNAME hash, so that tests can reach the collision path.
+unsigned long long coll_hash_mask()
+{
+    static const int bits = getenv("MSG_COLLATE_HASH_BITS") ? atoi(getenv("MSG_COLLATE_HASH_BITS")) : 64;
+    return bits >= 64 || bits < 1 ? ~0ull : ~0ull << (64 - bits);
+}
+
+int coll_grow(msg_ctx *c, DevBuf &b, size_t bytes, size_t keep, uint64_t nrec, uint64_t head_bytes)
+{
+    if (bytes <= b.cap && b.p) return MSG_OK;
+    size_t free_b = 0, total_b = 0;
+    cudaError_t e = cudaMemGetInfo(&free_b, &total_b);
+    if (e == cudaSuccess) e = bytes + bytes / 2 + 256 <= free_b ? b.reserve_keep(bytes, keep, c->stream) : cudaErrorMemoryAllocation;
+    if (e == cudaSuccess) return MSG_OK;
+    cudaGetLastError();
+    return fail(c, e == cudaErrorMemoryAllocation ? MSG_ENOMEM : MSG_ECUDA,
+                "cannot hold %llu records (%llu bytes of record heads) for collation in device memory (%zu bytes free): %s",
+                (unsigned long long)nrec, (unsigned long long)head_bytes, free_b, cudaGetErrorString(e));
+}
+
+// A push on a collating context: append the chunk's record heads and keys to the scope (msg_config.collate).
+int collate_push(msg_ctx *c, const uint8_t *h_raw, const uint8_t *dev_raw, size_t nbytes, const uint64_t *h_off, const uint64_t *dev_off, size_t nrec)
+{
+    { int rc0 = chunk_args_ok(c, nbytes, nrec); if (rc0) return rc0; }
+    if (c->coll_done) { c->coll_n = 0; c->coll_bytes = 0; c->coll_done = false; }
+    if (nrec == 0) return MSG_OK;
+    if (c->coll_n + nrec > 0xfffffffeull)
+        return fail(c, MSG_ERANGE, "collation holds at most 2^32-2 records per scope (%llu held, %zu pushed)", (unsigned long long)c->coll_n, nrec);
+    Slot &sl = c->slot[0];
+    const uint8_t *src = dev_raw; const uint64_t *offp = dev_off;
+    if (!dev_raw) {
+        CU(sl.off.reserve((nrec + 1) * 8));
+        CU(cudaMemcpyAsync(sl.off.p, h_off, (nrec + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+        offp = sl.off.as<uint64_t>();
+        c->h2d_bytes += (nrec + 1) * 8;
+        // pinned, mapped host memory is read in place (only the heads and aux blocks cross PCIe); anything else is staged
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, h_raw) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) {
+            src = static_cast<const uint8_t *>(at.devicePointer);
+            c->zc_chunks++;
+        } else {
+            cudaGetLastError();
+            CU(sl.raw.reserve(nbytes + 64));
+            CU(cudaMemcpyAsync(sl.raw.p, h_raw, nbytes, cudaMemcpyHostToDevice, c->stream));
+            src = sl.raw.as<uint8_t>();
+            c->h2d_bytes += nbytes;
+        }
+    }
+    const uint32_t base = (uint32_t)c->coll_n;
+    CU(c->coll_len.reserve(nrec * 4));
+    collate_size_kernel<<<nblocks(nrec, 256), 256, 0, c->stream>>>(src, offp, nrec, nbytes, base, c->need_stats || c->cov_fused,
+                                                                   c->coll_len.as<uint32_t>(), c->d_err); LAUNCHED(c);
+    { int rc = check_device_errors(c); if (rc) return rc; }
+    const uint64_t n_all = c->coll_n + nrec;
+    { int rc = coll_grow(c, c->coll_aoff, (n_all + 1) * 8, (c->coll_n + 1) * 8, n_all, c->coll_bytes); if (rc) return rc; }
+    unsigned long long tot = 0;
+    unsigned long long *aoff = c->coll_aoff.as<unsigned long long>();
+    int rc = run_scan<unsigned long long>(c, InLenU64{c->coll_len.as<uint32_t>()}, OutExclU64Add{aoff + c->coll_n, c->coll_bytes}, nrec, &tot);
+    if (rc) return rc;
+    const uint64_t bytes_all = c->coll_bytes + tot;
+    if (bytes_all >= (1ull << 36))      // the grouped stream is handed to the pipeline with offsets from its start
+        return fail(c, MSG_ERANGE, "collation holds at most 64 GiB of record heads per scope (%llu records held)", (unsigned long long)c->coll_n);
+    unsigned long long *h_end = reinterpret_cast<unsigned long long *>(c->h_pin + 84);
+    *h_end = bytes_all;
+    CU(cudaMemcpyAsync(aoff + n_all, h_end, 8, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = coll_grow(c, c->coll_arena, bytes_all + 64, c->coll_bytes, n_all, bytes_all))) return rc;
+    if ((rc = coll_grow(c, c->coll_keys, n_all * sizeof(CollKey), c->coll_n * sizeof(CollKey), n_all, bytes_all))) return rc;
+    collate_gather_kernel<<<std::min<uint32_t>(nblocks(nrec, 8), 148u * 64u), 256, 0, c->stream>>>(src, offp, nrec, aoff + c->coll_n, c->coll_len.as<uint32_t>(),
+                                                                  c->coll_arena.as<uint8_t>(), c->coll_keys.as<CollKey>() + c->coll_n, base, coll_hash_mask()); LAUNCHED(c);
+    CU(cudaStreamSynchronize(c->stream));             // the caller may reuse its buffers once the push returns
+    c->coll_n = n_all; c->coll_bytes = bytes_all; c->coll_dirty = true;
+    return MSG_OK;
+}
+
+// Largest grouped chunk handed to the pipeline: with at most 2^24 records per chunk no chunk can hold more than the
+// profile stage's 65536 groups of > 1024 records.
+constexpr uint64_t COLL_CHUNK_RECORDS = 1ull << 24;
+
+// Group everything held by QNAME and run the pipeline over it once (first finish after pushes).
+int collate_run(msg_ctx *c)
+{
+    if (!c->coll_dirty) return MSG_OK;
+    c->coll_dirty = false; c->coll_done = true;
+    const uint64_t n = c->coll_n;
+    if (n == 0) return MSG_OK;
+    static const bool trace = getenv("MSG_TRACE_FINISH") != nullptr;
+    cudaEvent_t tev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    auto tmark = [&](int k) { if (trace) { cudaEventCreate(&tev[k]); cudaEventRecord(tev[k], c->stream); } };
+    tmark(0);
+    const unsigned long long *aoff = c->coll_aoff.as<unsigned long long>();
+    const uint8_t *arena = c->coll_arena.as<uint8_t>();
+    int rc;
+    // ---- partition by the top bits of the hash
+    uint32_t bits = 0;
+    while (bits < 24 && ((uint64_t)COLL_BUCKET_AVG << bits) < n) bits++;
+    const uint32_t nb = 1u << bits;
+    if ((rc = coll_grow(c, c->coll_keys2, n * sizeof(CollKey), 0, n, c->coll_bytes))) return rc;
+    CU(c->coll_hist.reserve((size_t)nb * 4)); CU(c->coll_bstart.reserve((size_t)nb * 4));
+    CU(c->coll_list.reserve((size_t)nb * 4 + 8));
+    uint32_t *hist = c->coll_hist.as<uint32_t>(), *bstart = c->coll_bstart.as<uint32_t>();
+    CollKey *keys = c->coll_keys2.as<CollKey>();
+    CU(cudaMemsetAsync(hist, 0, (size_t)nb * 4, c->stream));
+    collate_hist_kernel<<<nblocks(n, 256), 256, 0, c->stream>>>(c->coll_keys.as<CollKey>(), n, bits, hist); LAUNCHED(c);
+    if ((rc = run_scan<uint32_t>(c, InU32{hist}, OutExclU32{bstart}, nb, (uint32_t *)nullptr))) return rc;
+    CU(cudaMemcpyAsync(hist, bstart, (size_t)nb * 4, cudaMemcpyDeviceToDevice, c->stream));
+    collate_scatter_kernel<<<nblocks(n, 256), 256, 0, c->stream>>>(c->coll_keys.as<CollKey>(), n, bits, hist, keys); LAUNCHED(c);
+    tmark(1);
+    // ---- sort every bucket by (hash, ordinal)
+    uint32_t *big = c->coll_list.as<uint32_t>(), *cnt = reinterpret_cast<uint32_t *>(c->d_total);
+    CU(cudaMemsetAsync(cnt, 0, 4, c->stream));
+    collate_bucket_sort_kernel<<<std::min<uint32_t>(nb, 148u * 8u), 256, 0, c->stream>>>(keys, bstart, nb, n, big, cnt); LAUNCHED(c);
+    uint32_t *h_cnt = c->h_pin + 88;
+    CU(cudaMemcpyAsync(h_cnt, cnt, 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (*h_cnt) { collate_sort_global_kernel<<<*h_cnt, 1024, 0, c->stream>>>(keys, bstart, nb, n, big, false, arena, aoff); LAUNCHED(c); }
+    // ---- runs of one hash that hold different names: sort them by (name bytes, ordinal).  Rare (64-bit hash).
+    for (;;) {
+        const uint32_t cap = (uint32_t)(c->coll_list.cap / 8);
+        CU(cudaMemsetAsync(cnt, 0, 4, c->stream));
+        collate_collide_kernel<<<nblocks(n, 256), 256, 0, c->stream>>>(keys, n, arena, aoff, c->coll_list.as<uint32_t>(), cap, cnt); LAUNCHED(c);
+        CU(cudaMemcpyAsync(h_cnt, cnt, 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        if (*h_cnt <= cap) break;
+        CU(c->coll_list.reserve((size_t)*h_cnt * 8));
+    }
+    if (*h_cnt) { collate_sort_global_kernel<<<*h_cnt, 1024, 0, c->stream>>>(keys, bstart, nb, n, c->coll_list.as<uint32_t>(), true, arena, aoff); LAUNCHED(c); }
+    tmark(2);
+    // ---- heads in grouped order; keys[g].ord maps a grouped position back to its input ordinal
+    unsigned long long tot = 0;
+    if ((rc = coll_grow(c, c->coll_goff, (n + 1) * 8, 0, n, c->coll_bytes))) return rc;
+    unsigned long long *goff = c->coll_goff.as<unsigned long long>();
+    if ((rc = run_scan<unsigned long long>(c, InGroupedLen{keys, aoff}, OutExclU64{goff}, n, &tot))) return rc;
+    unsigned long long *h_end = reinterpret_cast<unsigned long long *>(c->h_pin + 84);
+    *h_end = tot;
+    CU(cudaMemcpyAsync(goff + n, h_end, 8, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = coll_grow(c, c->coll_grouped, tot + 64, 0, n, tot))) return rc;
+    collate_grouped_gather_kernel<<<std::min<uint32_t>(nblocks(n, 8), 148u * 64u), 256, 0, c->stream>>>(keys, n, arena, aoff, goff, c->coll_grouped.as<uint8_t>()); LAUNCHED(c);
+    tmark(3);
+    // ---- the pipeline, one device chunk at a time.  Chunks are cut where the hash changes, which is a group start; any
+    // group start is a safe cut here because every name occurs in exactly one run of the grouped stream, so no pool or
+    // profile group can continue across it (the record before a cut can never share the next record's name, whatever
+    // its flags or tid).  The chunk's index holds absolute offsets into the grouped arena.
+    unsigned long long *dcut = reinterpret_cast<unsigned long long *>(c->d_total);
+    unsigned long long *h_cut = reinterpret_cast<unsigned long long *>(c->h_pin + 92);
+    std::vector<unsigned long long> hgo(1);
+    for (uint64_t lo = 0; lo < n;) {
+        uint64_t hi = n;
+        if (n - lo > COLL_CHUNK_RECORDS) {
+            // the last run start in (lo, lo + 2^24], else (one read with more alignments) the first one after it
+            const uint64_t want = lo + COLL_CHUNK_RECORDS, end = std::min<uint64_t>(n, want + COLL_CHUNK_RECORDS);
+            const unsigned long long init[2] = {0ull, ~0ull};
+            memcpy(h_cut, init, 16);
+            CU(cudaMemcpyAsync(dcut, h_cut, 16, cudaMemcpyHostToDevice, c->stream));
+            collate_cut_kernel<<<nblocks(end - lo - 1, 256), 256, 0, c->stream>>>(keys, lo, want, end, dcut, dcut + 1); LAUNCHED(c);
+            CU(cudaMemcpyAsync(h_cut, dcut, 16, cudaMemcpyDeviceToHost, c->stream));
+            CU(cudaStreamSynchronize(c->stream));
+            hi = h_cut[0] ? h_cut[0] : h_cut[1] != ~0ull ? h_cut[1] : end;
+            if (hi == end && end < n) return fail(c, MSG_ERANGE, "one read has more than %llu alignments", (unsigned long long)COLL_CHUNK_RECORDS);
+        }
+        CU(cudaMemcpyAsync(hgo.data(), goff + hi, 8, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        // Groups come in hash order rather than input order.  Per read, the filter, best-hit and uniq-hit selection (a set
+        // per mate class) and insert counting only see that read's records, which keep their input order; across reads,
+        // the order changes only the order of the multi-mapper lists, i.e. the summation order of the f64 PropSharing
+        // sums, which the f64 atomics already vary.  So every integer result equals that of the input regrouped stably
+        // by QNAME, and every f64 result equals it up to rounding.
+        rc = push_chunk(c, nullptr, c->coll_grouped.as<uint8_t>(), hgo[0], nullptr, reinterpret_cast<const uint64_t *>(goff + lo), hi - lo);
+        if (!rc) rc = wait_all(c);
+        if (rc) {
+            // errors found after grouping name the record's input ordinal, not its grouped position
+            if ((rc == MSG_ENOTAG || rc == MSG_ENOAS || rc == MSG_EFORMAT) && c->err_rec != 0xffffffffu && lo + c->err_rec < n) {
+                CollKey k;
+                if (cudaMemcpy(&k, keys + lo + c->err_rec, sizeof k, cudaMemcpyDeviceToHost) == cudaSuccess)
+                    c->err += " (input record " + std::to_string(k.ord) + ")";
+            }
+            return rc;
+        }
+        lo = hi;
+    }
+    if (trace) {
+        tmark(4); cudaEventSynchronize(tev[4]);
+        float ms[4] = {0, 0, 0, 0};
+        for (int k = 0; k < 4; k++) cudaEventElapsedTime(&ms[k], tev[k], tev[k + 1]);
+        fprintf(stderr, "[msg collate] %llu records, %llu head bytes: partition %.3f ms, sort %.3f ms, grouped gather %.3f ms, pipeline %.3f ms\n",
+                (unsigned long long)n, (unsigned long long)tot, ms[0], ms[1], ms[2], ms[3]);
+        for (auto e : tev) if (e) cudaEventDestroy(e);
+    }
+    return MSG_OK;
+}
+
 int allreduce(msg_ctx *c, void *buf, size_t count, ncclDataType_t dt, ncclRedOp_t op)
 {
     if (c->cfg.n_ranks <= 1) return MSG_OK;
@@ -750,6 +950,12 @@ int msg_create(const msg_config *cfg, msg_ctx **out)
     if (cfg->want_coverage && !cfg->target_len) return fail(c, MSG_EINVAL, "want_coverage requires target_len");
     if (cfg->do_filter && cfg->invert && cfg->hit_mode) return fail(c, MSG_EINVAL, "--invert cannot be combined with --besthit or --uniqhit");
     if (cfg->hit_mode > MSG_HIT_UNIQUE) return fail(c, MSG_EINVAL, "bad hit_mode");
+    if (cfg->collate) {
+        if (!cfg->want_profile && !cfg->want_coverage) return fail(c, MSG_EINVAL, "collate needs want_profile and/or want_coverage");
+        if (cfg->want_records || cfg->want_kept || cfg->want_stats)
+            return fail(c, MSG_EINVAL, "collate cannot be combined with want_records, want_kept or want_stats: results come per grouped chunk, not per pushed one");
+        if (cfg->n_ranks > 1) return fail(c, MSG_EINVAL, "collate needs n_ranks == 1");
+    }
     int ndev = 0;
     cudaError_t ce = cudaGetDeviceCount(&ndev);
     if (ce != cudaSuccess || ndev == 0) { cudaGetLastError(); return fail(c, MSG_ENODEV, "no CUDA device available (%s); libmsamtools_b200 has no CPU fallback", ce != cudaSuccess ? cudaGetErrorString(ce) : "device count 0"); }
@@ -951,6 +1157,7 @@ int msg_reset(msg_ctx *c)
         CU(cudaMemsetAsync(c->d_covered, 0, T, c->stream));
         c->cov_finished = false;
     }
+    c->coll_n = c->coll_bytes = 0; c->coll_dirty = c->coll_done = false;
     c->n_kept = 0; c->have_stream = false; c->out_bytes = 0; c->cur_n = 0;
     CU(cudaStreamSynchronize(c->stream));
     return MSG_OK;
@@ -1005,6 +1212,7 @@ int msg_push_async(msg_ctx *c, const uint8_t *raw, size_t nbytes, const uint64_t
 {
     if (!c || (nrec && (!raw || !rec_off))) return MSG_EINVAL;
     CU(cudaSetDevice(c->cfg.device));
+    if (c->cfg.collate) return collate_push(c, raw, nullptr, nbytes, rec_off, nullptr, nrec);
     return push_chunk(c, raw, nullptr, nbytes, rec_off, nullptr, nrec);
 }
 
@@ -1013,6 +1221,7 @@ int msg_push_device_async(msg_ctx *c, const uint8_t *d_raw, size_t nbytes, const
     if (!c || (nrec && (!d_raw || !d_rec_off))) return MSG_EINVAL;
     if ((uintptr_t)d_raw & 15u) return fail(c, MSG_EINVAL, "device chunk must be 16-byte aligned");
     CU(cudaSetDevice(c->cfg.device));
+    if (c->cfg.collate) return collate_push(c, nullptr, d_raw, nbytes, nullptr, d_rec_off, nrec);
     return push_chunk(c, nullptr, d_raw, nbytes, nullptr, d_rec_off, nrec);
 }
 
@@ -1035,9 +1244,12 @@ int msg_push_device(msg_ctx *c, const uint8_t *d_raw, size_t nbytes, const uint6
     return rc ? rc : wait_all(c);
 }
 
+static const char *k_collate_chunk = "per-chunk results are not available on a collating context (records are grouped at finish)";
+
 int msg_kept_count(msg_ctx *c, size_t *n_kept)
 {
     if (!c || !n_kept) return MSG_EINVAL;
+    if (c->cfg.collate) return fail(c, MSG_ESTATE, "%s", k_collate_chunk);
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
     *n_kept = c->n_kept;
@@ -1047,6 +1259,7 @@ int msg_kept_count(msg_ctx *c, size_t *n_kept)
 int msg_pull_kept(msg_ctx *c, uint32_t *idx, size_t cap, size_t *n_kept)
 {
     if (!c) return MSG_EINVAL;
+    if (c->cfg.collate) return fail(c, MSG_ESTATE, "%s", k_collate_chunk);
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
     if (n_kept) *n_kept = c->n_kept;
@@ -1064,6 +1277,7 @@ int msg_pull_kept(msg_ctx *c, uint32_t *idx, size_t cap, size_t *n_kept)
 int msg_pull_records(msg_ctx *c, uint8_t *out, size_t cap, size_t *nbytes, size_t *nrec)
 {
     if (!c) return MSG_EINVAL;
+    if (c->cfg.collate) return fail(c, MSG_ESTATE, "%s", k_collate_chunk);
     if (!c->cfg.want_records) return fail(c, MSG_ESTATE, "context was created without want_records");
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
@@ -1082,6 +1296,7 @@ int msg_pull_records(msg_ctx *c, uint8_t *out, size_t cap, size_t *nbytes, size_
 int msg_pull_stats(msg_ctx *c, size_t nrec, int32_t *alen, int32_t *qlen, int32_t *qclip, int32_t *edit, int32_t *score, uint8_t *flags)
 {
     if (!c) return MSG_EINVAL;
+    if (c->cfg.collate) return fail(c, MSG_ESTATE, "%s", k_collate_chunk);
     if (!c->cfg.want_stats) return fail(c, MSG_ESTATE, "context was created without want_stats");
     { int wrc = wait_all(c); if (wrc) return wrc; }
     if (nrec != c->cur_n) return fail(c, MSG_EINVAL, "nrec does not match the last chunk");
@@ -1106,6 +1321,7 @@ int msg_pull_counts(msg_ctx *c, uint32_t *ui, double *d)
     if (!c->cfg.want_profile) return fail(c, MSG_ESTATE, "context was created without want_profile");
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
+    { int crc = collate_run(c); if (crc) return crc; }
     const size_t F = (size_t)c->cfg.n_features;
     if (ui && F) CU(cudaMemcpyAsync(ui, c->d_ui, F * 4, cudaMemcpyDeviceToHost, c->stream));
     if (d && F)  CU(cudaMemcpyAsync(d, c->d_d, F * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -1119,6 +1335,7 @@ int msg_finish_profile(msg_ctx *c, double *abundance, msg_profile_stats *st)
     if (!c->cfg.want_profile) return fail(c, MSG_ESTATE, "context was created without want_profile");
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
+    { int crc = collate_run(c); if (crc) return crc; }
     const msg_config &g = c->cfg;
     const uint32_t F = (uint32_t)g.n_features;
     msg_profile_stats s; memset(&s, 0, sizeof s);
@@ -1327,6 +1544,7 @@ int msg_finish_coverage(msg_ctx *c, uint8_t *covered, int64_t *touched, int64_t 
     if (!c->cfg.want_coverage) return fail(c, MSG_ESTATE, "context was created without want_coverage");
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
+    { int crc = collate_run(c); if (crc) return crc; }
     const msg_config &g = c->cfg;
     const size_t T = (size_t)g.n_targets;
     int rc;

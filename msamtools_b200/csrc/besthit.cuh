@@ -82,6 +82,17 @@ __device__ __forceinline__ bool pool_winner(int32_t *sb, uint32_t lane, bool act
     return tie && sb[slot] == 1;
 }
 
+// the first record of pool [i, end) that the best-hit writers read without an AS tag (for the error message)
+__device__ __forceinline__ uint32_t noas_record(const uint32_t *fb, uint64_t i, uint64_t end, bool paired)
+{
+    for (uint64_t j = i; j < end; j++) {
+        const uint32_t f = fb[j];
+        const int c = mate_class(f);
+        if ((f & FB_INPOOL) && !(f & FB_HAS_AS) && (paired ? (c == 1 || c == 2) : c == 0)) return (uint32_t)j;
+    }
+    return 0xffffffffu;
+}
+
 __global__ void __launch_bounds__(256) besthit_warp_select_kernel(const BestHitParams p)
 {
     __shared__ __align__(16) int32_t s_best[8][128];
@@ -103,7 +114,7 @@ __global__ void __launch_bounds__(256) besthit_warp_select_kernel(const BestHitP
     // pool pairedness (msam_filter.c:196-204) and the classes the reference visits (:247-254)
     const bool paired = (__ballot_sync(0xffffffffu, pooled && cls != 0) & v.segmask) != 0;
     const bool act = pooled && (paired ? (cls == 1 || cls == 2) : true);
-    if (act && !(f & FB_HAS_AS)) atomicOr(p.err, DERR_NOAS);                       // :219-221
+    if (act && !(f & FB_HAS_AS)) { atomicOr(p.err, DERR_NOAS); atomicMin(p.err + 1, (uint32_t)i); }       // :219-221
     const int32_t sc = act ? p.score[i] : INT32_MIN;
     const bool keep = pool_winner(s_best[threadIdx.x >> 5], lane, act, sc, v.s * 4u + (uint32_t)cls, p.uniq);
     if (mine) {
@@ -140,7 +151,7 @@ __global__ void __launch_bounds__(256) besthit_walk_select_kernel(const BestHitP
             if (!(f & FB_EQPREV)) break;
         }
         const uint64_t end = j;
-        if (paired ? (noas & 6u) : (noas & 1u)) atomicOr(p.err, DERR_NOAS);
+        if (paired ? (noas & 6u) : (noas & 1u)) { atomicOr(p.err, DERR_NOAS); atomicMin(p.err + 1, noas_record(p.fb, i, end, paired)); }
         for (j = i; j < end; j++) {
             f = p.fb[j];
             bool keep = false;

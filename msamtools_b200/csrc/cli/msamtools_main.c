@@ -604,7 +604,9 @@ static int filter_main(int argc, char *argv[])
     struct arg_lit *a_v = arg_lit0("v", "invert", "invert the effect of the filter: report the complement among mapped alignments (default: false)");
     struct arg_lit *a_rescore = arg_lit0(NULL, "rescore", "rescore alignments using MD or NM fields, in that order (default: false)\n\n"
                                          "Special filters (need name-grouped input and AS, unless --rescore; cannot be combined with -v):\n");
-    struct arg_lit *a_best = arg_lit0(NULL, "besthit", "keep all highest scoring hit(s) per read (default: false)");
+    struct arg_lit *a_best = arg_lit0(NULL, "besthit", "keep all highest scoring hit(s) per read (default: false); input in any other order (e.g. sorted by\n"
+                                      "coordinate) stays refused, as the output records would need SEQ/QUAL held on the GPU: filter it without\n"
+                                      "--besthit and pipe it into 'profile --collate'");
     struct arg_lit *a_uniq = arg_lit0(NULL, "uniqhit", "keep only one highest scoring hit per read, only if it is unique (default: false)");
     struct arg_end *end = arg_end(16);
     void *argtable[] = { a_b, a_u, a_h, a_S, a_file, a_help, a_l, a_p, a_ppt, a_z, a_k, a_v, a_rescore, a_best, a_uniq, end };
@@ -775,8 +777,10 @@ static int profile_main(int argc, char *argv[])
                                        "An insert hitting N features adds 1 to each (all), 1/N to each (equal), a share proportional to the\n"
                                        "features' current abundances (proportional), or nothing (ignore). Input must be grouped by QNAME and\n"
                                        "already filtered (see 'filter').");
+    struct arg_lit *a_collate = arg_lit0(NULL, "collate", "input need not be grouped by QNAME (e.g. sorted by coordinate): the records are grouped on the GPU\n"
+                                         "(default: false; without it, input must be grouped by QNAME)");
     struct arg_end *end = arg_end(20);
-    void *argtable[] = { a_S, a_file, a_help, a_out, a_label, a_genome, a_total, a_mincount, a_unit, a_pandas, a_nopandas, a_nolen, a_multi, end };
+    void *argtable[] = { a_S, a_file, a_help, a_out, a_label, a_genome, a_total, a_mincount, a_unit, a_pandas, a_nopandas, a_nolen, a_multi, a_collate, end };
 
     if (arg_nullcheck(argtable) != 0) mDie("insufficient memory");
     int nerrors = arg_parse(argc, argv, argtable);
@@ -798,7 +802,8 @@ static int profile_main(int argc, char *argv[])
     open_input(&r, a_file->filename[0]);
     phase(sub, "open + header");
     chunk_fill(&r.chunk, r.in, r.hdr, COORD_ORDER_CHECK_RECORDS, (size_t)-1, &r.eof);
-    qn_result qn = qname_preflight(r.hdr, &r.chunk);
+    qn_result qn = { QN_NOT_REQUIRED, 0, 0, 0 };
+    if (a_collate->count == 0) qn = qname_preflight(r.hdr, &r.chunk);
 
     /* any prefix matches, first hit in this order (msam_profile.c:712-748) */
     int share_type = MSG_MULTI_PROPORTIONAL, unit_type = 1;
@@ -856,6 +861,7 @@ static int profile_main(int argc, char *argv[])
     }
 
     r.cfg.do_filter = 0; r.cfg.want_profile = 1; r.cfg.share_type = (uint8_t)share_type;
+    r.cfg.collate = a_collate->count > 0;
     r.cfg.n_targets = n_targets; r.cfg.n_features = n_features; r.cfg.fmap = fmap;
     phase(sub, "pre-flight + feature map");
     msg_ctx *ctx = run_stream(&r);

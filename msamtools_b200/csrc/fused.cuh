@@ -72,7 +72,7 @@ __global__ void __launch_bounds__(256) fused_warp_kernel(const FusedParams p)
         const int cls = mate_class(f);
         const bool paired = (__ballot_sync(0xffffffffu, pooled && cls != 0) & v.segmask) != 0;
         const bool act = pooled && (paired ? (cls == 1 || cls == 2) : true);
-        if (act && !(f & FB_HAS_AS)) atomicOr(p.err, DERR_NOAS);
+        if (act && !(f & FB_HAS_AS)) { atomicOr(p.err, DERR_NOAS); atomicMin(p.err + 1, (uint32_t)i); }
         const int32_t sc = act ? p.score[i] : INT32_MIN;
         const bool keep = pool_winner(s_best[threadIdx.x >> 5], lane, act, sc, v.s * 4u + (uint32_t)cls, p.uniq);
 
@@ -225,7 +225,7 @@ __global__ void __launch_bounds__(128) fused_walk_kernel(const FusedParams p)
 #pragma unroll
         for (int k = 0; k < FUSED_PF; k++) if ((uint32_t)k < len) pass1(fr[k], sr[k]);
         for (uint64_t j = i + FUSED_PF; j < end; j++) pass1(p.fb[j], p.score[j]);
-        if (paired ? (noas & 6u) : (noas & 1u)) atomicOr(p.err, DERR_NOAS);
+        if (paired ? (noas & 6u) : (noas & 1u)) { atomicOr(p.err, DERR_NOAS); atomicMin(p.err + 1, noas_record(p.fb, i, end, paired)); }
         // pass 2: the winners' features, distinct, in the order READ1-class winners then READ2-class winners, each in input
         // order (msam_filter.c:247-254 -> msam_profile.c:136-142).  Two sweeps over the run (the usual short pool sits in the
         // prefetched registers); the first FUSED_DR distinct features live in registers (compare / insert fully unrolled),
