@@ -35,7 +35,8 @@
  * except on a context created with `collate`, which takes records in any order.
  *
  * Collating contexts (msg_config.collate = 1)
- *   - chunks need not end on a QNAME boundary; a read's records may be spread over any number of pushes.
+ *   - chunks need not end on a QNAME boundary; a read's records may be spread over any number of pushes, and a read
+ *     may have any number of records.
  *   - msg_push* append the records' heads (everything but SEQ/QUAL) to device memory and complete before returning.
  *     More than 2^32-2 records (or 64 GiB of heads) in one scope: MSG_ERANGE; no room on the device: MSG_ENOMEM.
  *   - the first msg_finish_profile / msg_finish_coverage / msg_pull_counts after pushes groups everything held by

@@ -790,8 +790,13 @@ int collate_push(msg_ctx *c, const uint8_t *h_raw, const uint8_t *dev_raw, size_
 }
 
 // Largest grouped chunk handed to the pipeline: with at most 2^24 records per chunk no chunk can hold more than the
-// profile stage's 65536 groups of > 1024 records.
-constexpr uint64_t COLL_CHUNK_RECORDS = 1ull << 24;
+// profile stage's 65536 groups of > 1024 records.  A single read larger than that is a chunk of its own (one group).
+// MSG_COLLATE_CHUNK_RECORDS=C (clamped to [1, 2^24]) lowers the limit, so that tests reach every cut with few records.
+uint64_t coll_chunk_records()
+{
+    static const long long env = getenv("MSG_COLLATE_CHUNK_RECORDS") ? atoll(getenv("MSG_COLLATE_CHUNK_RECORDS")) : 1ll << 24;
+    return (uint64_t)std::min<long long>(std::max<long long>(env, 1), 1ll << 24);
+}
 
 // Group everything held by QNAME and run the pipeline over it once (first finish after pushes).
 int collate_run(msg_ctx *c)
@@ -860,19 +865,25 @@ int collate_run(msg_ctx *c)
     unsigned long long *dcut = reinterpret_cast<unsigned long long *>(c->d_total);
     unsigned long long *h_cut = reinterpret_cast<unsigned long long *>(c->h_pin + 92);
     std::vector<unsigned long long> hgo(1);
+    const uint64_t C = coll_chunk_records();
     for (uint64_t lo = 0; lo < n;) {
         uint64_t hi = n;
-        if (n - lo > COLL_CHUNK_RECORDS) {
-            // the last run start in (lo, lo + 2^24], else (one read with more alignments) the first one after it
-            const uint64_t want = lo + COLL_CHUNK_RECORDS, end = std::min<uint64_t>(n, want + COLL_CHUNK_RECORDS);
-            const unsigned long long init[2] = {0ull, ~0ull};
-            memcpy(h_cut, init, 16);
-            CU(cudaMemcpyAsync(dcut, h_cut, 16, cudaMemcpyHostToDevice, c->stream));
-            collate_cut_kernel<<<nblocks(end - lo - 1, 256), 256, 0, c->stream>>>(keys, lo, want, end, dcut, dcut + 1); LAUNCHED(c);
-            CU(cudaMemcpyAsync(h_cut, dcut, 16, cudaMemcpyDeviceToHost, c->stream));
-            CU(cudaStreamSynchronize(c->stream));
-            hi = h_cut[0] ? h_cut[0] : h_cut[1] != ~0ull ? h_cut[1] : end;
-            if (hi == end && end < n) return fail(c, MSG_ERANGE, "one read has more than %llu alignments", (unsigned long long)COLL_CHUNK_RECORDS);
+        if (n - lo > C) {
+            // the last run start in (lo, lo + C]; else (one read of more than C records) the first one after lo + C,
+            // searched in windows that double until one is found or n is reached
+            const uint64_t want = lo + C;
+            uint64_t from = lo, end = std::min<uint64_t>(n, want + C + 1), step = C;
+            for (;;) {
+                const unsigned long long init[2] = {0ull, ~0ull};
+                memcpy(h_cut, init, 16);
+                CU(cudaMemcpyAsync(dcut, h_cut, 16, cudaMemcpyHostToDevice, c->stream));
+                collate_cut_kernel<<<nblocks(end - from - 1, 256), 256, 0, c->stream>>>(keys, from, want, end, dcut, dcut + 1); LAUNCHED(c);
+                CU(cudaMemcpyAsync(h_cut, dcut, 16, cudaMemcpyDeviceToHost, c->stream));
+                CU(cudaStreamSynchronize(c->stream));
+                if (h_cut[0] || h_cut[1] != ~0ull || end == n) break;
+                from = end - 1; step *= 2; end = std::min<uint64_t>(n, end + step);
+            }
+            hi = h_cut[0] ? h_cut[0] : h_cut[1] != ~0ull ? h_cut[1] : n;
         }
         CU(cudaMemcpyAsync(hgo.data(), goff + hi, 8, cudaMemcpyDeviceToHost, c->stream));
         CU(cudaStreamSynchronize(c->stream));
