@@ -1340,6 +1340,178 @@ int msg_pull_counts(msg_ctx *c, uint32_t *ui, double *d)
     return MSG_OK;
 }
 
+// MSG_TRACE_FINISH=1: device-side time of each phase of msg_finish_profile, printed to stderr (diagnostics only).
+// Events: 0 start, 1 counts combined over NCCL, 2 em_init done, 3 cooperative loop launched, 4 end.
+struct FinishTrace {
+    bool on;
+    cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    void mark(int k, cudaStream_t s) { if (on) { if (!ev[k]) cudaEventCreate(&ev[k]); cudaEventRecord(ev[k], s); } }
+};
+
+// With n_ranks > 1: ONE allreduce over NVLink for everything that is additive across ranks (per-reference counts, the
+// insert counters and the number of multi-mapper lists, packed as u32[F + 8]) and one for the MSG_MULTI_EQUAL shares,
+// on copies, so that finish can be called again after more chunks; ui and dd then point at the sums.  The insert
+// counters (and, with n_ranks > 1, the list total) are copied to hc.
+static int finish_combine_counts(msg_ctx *c, uint32_t *&ui, double *&dd, uint32_t *hc, FinishTrace &tr)
+{
+    const msg_config &g = c->cfg;
+    const uint32_t F = (uint32_t)g.n_features;
+    int rc;
+    if (g.n_ranks <= 1) { CU(cudaMemcpyAsync(hc, c->d_counters, 16, cudaMemcpyDeviceToHost, c->stream)); return MSG_OK; }
+    CU(c->t_ui.reserve(((size_t)F + 8) * 4));
+    ui = c->t_ui.as<uint32_t>();
+    uint32_t *cnt = ui + F;
+    CU(cudaMemcpyAsync(ui, c->d_ui, (size_t)F * 4, cudaMemcpyDeviceToDevice, c->stream));
+    CU(cudaMemcpyAsync(cnt, c->d_counters, 16, cudaMemcpyDeviceToDevice, c->stream));
+    const uint32_t nl_lo[2] = {(uint32_t)(c->csr_lists & 0xffffu), (uint32_t)(c->csr_lists >> 16)};   // two 16-bit halves: sums stay exact in u32 for up to 65536 ranks
+    CU(cudaMemcpyAsync(cnt + 4, nl_lo, 8, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = allreduce(c, ui, (size_t)F + 6, ncclUint32, ncclSum))) return rc;
+    if (g.share_type == MSG_MULTI_EQUAL) {
+        CU(c->t_d.reserve((size_t)(F ? F : 1) * 8));
+        CU(cudaMemcpyAsync(c->t_d.p, c->d_d, (size_t)F * 8, cudaMemcpyDeviceToDevice, c->stream));
+        dd = c->t_d.as<double>();
+        if ((rc = allreduce(c, dd, F, ncclFloat64, ncclSum))) return rc;
+    }
+    tr.mark(1, c->stream);
+    CU(cudaMemcpyAsync(hc, cnt, 24, cudaMemcpyDeviceToHost, c->stream));
+    return MSG_OK;
+}
+
+// The whole PropSharing loop in one cooperative launch: grid-wide barriers, no host round trips.  With n_ranks > 1 the
+// kernel also combines the counts (hc receives the insert counters and the list total) and runs every iteration's
+// exchange through peer memory.  The loop's iterations, deltas and purged count go to res / h_delta.  *ran stays false
+// when one GPU cannot co-schedule a CTA per SM: the caller then runs the host loop.
+static int em_coop_loop(msg_ctx *c, uint32_t *hc, int32_t *res, double *h_delta, FinishTrace &tr, bool *ran)
+{
+    const msg_config &g = c->cfg;
+    const uint32_t F = (uint32_t)g.n_features;
+    const bool multi = g.n_ranks > 1, sm = F <= EM_SMEM_F;
+    const bool rsag = multi && F + 8 > EM_XCHG_CTA0;               // gene catalogues: reduce-scatter / all-gather exchange
+    const size_t shm = em_smem_bytes(F);
+    int rc;
+    // the argument arrays below hold the addresses of these; partial is set once the grid size is known
+    const uint32_t *a0 = c->csr_off.as<uint32_t>(), *a1 = c->csr_len.as<uint32_t>(); const int32_t *a2 = c->csr_fid.as<int32_t>();
+    uint32_t nl_arg = (uint32_t)c->csr_lists, F_arg = F;
+    double *U = c->d_U, *av = c->d_a, *inc = c->d_inc, *dout = c->d_delta, *partial = nullptr;
+    int32_t *d_res = reinterpret_cast<int32_t *>(c->d_total);
+    const uint32_t *ui_arg = c->d_ui, *cnt_arg = c->d_counters;
+    uint32_t nl_lo = (uint32_t)(c->csr_lists & 0xffffu), nl_hi = (uint32_t)(c->csr_lists >> 16);   // two 16-bit halves, as in the NCCL path
+    uint32_t *hc_dev = nullptr, *bflag = c->d_bflag;
+    double *totbuf = nullptr;
+    unsigned long long *d_trace = nullptr;
+    PeerTable pt = c->peer_tab; int nr = g.n_ranks, rk = g.rank; uint32_t epoch = c->em_epoch;
+    static const double peer_timeout_s = getenv("MSG_PEER_TIMEOUT_S") ? atof(getenv("MSG_PEER_TIMEOUT_S")) : 120.0;
+    unsigned long long timeout_ns = (unsigned long long)(peer_timeout_s * 1e9);
+    if (multi) {
+        CU(c->t_cnt.reserve(64)); hc_dev = c->t_cnt.as<uint32_t>();
+        CU(c->t_d.reserve((size_t)F * 16)); totbuf = c->t_d.as<double>();
+        if (tr.on) { CU(c->t_ui.reserve(20 * 8 * 8)); d_trace = c->t_ui.as<unsigned long long>(); CU(cudaMemsetAsync(d_trace, 0, 20 * 8 * 8, c->stream)); }
+    }
+    void *largs[] = {&a0, &a1, &a2, &nl_arg, &U, &av, &inc, &partial, &F_arg, &dout, &d_res};
+    void *sargs[] = {&a0, &a1, &a2, &nl_arg, &U, &av, &inc, &F_arg, &dout, &d_res};
+    void *margs[] = {&a0, &a1, &a2, &nl_arg, &ui_arg, &cnt_arg, &nl_lo, &nl_hi, &U, &av, &inc, &partial, &F_arg, &dout, &d_res, &hc_dev,
+                     &totbuf, &bflag, &pt, &nr, &rk, &epoch, &timeout_ns};
+    void *rargs[] = {&a0, &a1, &a2, &nl_arg, &ui_arg, &cnt_arg, &nl_lo, &nl_hi, &U, &av, &inc, &F_arg, &dout, &d_res, &hc_dev,
+                     &pt, &nr, &rk, &epoch, &timeout_ns, &d_trace};
+    const void *fn; void **args;
+    if (rsag)       { fn = (const void *)em_loop_rsag_kernel; args = rargs; }
+    else if (multi) { fn = sm ? (const void *)em_loop_multi_kernel<true> : (const void *)em_loop_multi_kernel<false>; args = margs; }
+    else if (sm)    { fn = (const void *)em_loop_smem_kernel; args = sargs; }
+    else            { fn = (const void *)em_loop_kernel; args = largs; }
+    int per_sm = 0, nsm = 0;
+    CU(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, g.device));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, 256, shm));
+    if (per_sm < 1) {
+        if (multi) return fail(c, MSG_ECUDA, "cannot launch the cooperative PropSharing kernel (F = %u needs too much shared memory?)", F);
+        return MSG_OK;
+    }
+    const int want_ctas = EM_CTAS_ENV > 0 ? EM_CTAS_ENV : (sm ? 3 : 4);
+    if (per_sm > want_ctas) per_sm = want_ctas;
+    const uint32_t grid = (uint32_t)(nsm * per_sm);
+    CU(c->tile_sums.reserve((size_t)grid * 8 + 16));
+    partial = c->tile_sums.as<double>();
+    // one GPU: inc[3F], delta and d_res were cleared by em_init_kernel; the multi-GPU kernels clear their own state
+    if (multi) {
+        // The kernels of all ranks wait for one another inside the loop: line the ranks up first (a 4-byte NCCL
+        // allreduce on the same stream; it waits, on the device, for however long the slowest rank's ingest takes),
+        // so that the wall-clock limit inside the kernel (MSG_PEER_TIMEOUT_S, default 120 s) only ever measures a
+        // peer that died, not one that is merely late.
+        CU(cudaMemsetAsync(d_res, 0, 16, c->stream));
+        if ((rc = allreduce(c, c->t_cnt.as<uint32_t>() + 8, 1, ncclUint32, ncclSum))) return rc;
+        if (rsag) CU(cudaMemsetAsync(c->d_inc, 0, (size_t)F * 8, c->stream));
+    }
+    CU(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(256), args, shm, c->stream));
+    LAUNCHED(c);
+    if (multi) {
+        c->em_epoch += 32;
+        CU(cudaMemcpyAsync(hc, hc_dev, 24, cudaMemcpyDeviceToHost, c->stream));
+    }
+    tr.mark(3, c->stream);
+    CU(cudaMemcpyAsync(res, d_res, 16, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(h_delta, c->d_delta, 8 * 20, cudaMemcpyDeviceToHost, c->stream));
+    c->d2h_bytes += 176;
+    *ran = true;
+    return MSG_OK;
+}
+
+// The PropSharing loop with one launch per phase and a host read of delta per iteration: the NCCL fallback of the
+// multi-GPU loop (MSG_EM_HOST_LOOP=1 selects it on one GPU too).  The purged count lands in *h_purged at the caller's
+// stream sync.
+static int em_host_loop(msg_ctx *c, msg_profile_stats &s, uint32_t *h_purged)
+{
+    const uint32_t F = (uint32_t)c->cfg.n_features, nb = nblocks(F, 256), nl32 = (uint32_t)c->csr_lists;
+    const uint32_t em_grid = nl32 ? (nblocks(nl32, 256) < 148u * 8u ? nblocks(nl32, 256) : 148u * 8u) : 0;
+    const uint32_t *off = c->csr_off.as<uint32_t>(), *len = c->csr_len.as<uint32_t>(); const int32_t *fid = c->csr_fid.as<int32_t>();
+    int rc;
+    for (int k = 1; k < 20; k++) {                                                                      // msam_profile.c:331
+        CU(cudaMemsetAsync(c->d_inc, 0, (size_t)F * 8, c->stream));
+        if (nl32) { em_gather_kernel<<<em_grid, 256, em_smem_bytes(F), c->stream>>>(off, len, fid, nl32, c->d_a, c->d_inc, F); LAUNCHED(c); }
+        if ((rc = allreduce(c, c->d_inc, F, ncclFloat64, ncclSum))) return rc;
+        double delta = 0;
+        if (F) {
+            em_update_kernel<<<nb, 256, 0, c->stream>>>(c->d_U, c->d_inc, c->d_a, c->d_partial, F); LAUNCHED(c);
+            em_delta_kernel<<<1, 256, 0, c->stream>>>(c->d_partial, nb, F, c->d_delta + (k - 1)); LAUNCHED(c);
+            CU(cudaMemcpyAsync(&delta, c->d_delta + (k - 1), 8, cudaMemcpyDeviceToHost, c->stream));
+            CU(cudaStreamSynchronize(c->stream));
+            c->d2h_bytes += 8;
+        } else delta = nan("");                                                                     // reference divides by n_features == 0
+        s.em_delta[k - 1] = delta; s.em_iterations = k;
+        if (delta < 1e-10) { s.em_converged = 1; break; }                                               // :383
+    }
+    CU(cudaMemsetAsync(c->d_purged, 0, 4, c->stream));
+    if (nl32) { em_purged_kernel<<<em_grid, 256, 0, c->stream>>>(off, len, fid, nl32, c->d_a, c->d_purged); LAUNCHED(c); }
+    if ((rc = allreduce(c, c->d_purged, 1, ncclUint32, ncclSum))) return rc;
+    CU(cudaMemcpyAsync(h_purged, c->d_purged, 4, cudaMemcpyDeviceToHost, c->stream));
+    return MSG_OK;
+}
+
+static void finish_trace_report(msg_ctx *c, FinishTrace &tr, bool rsag_trace)
+{
+    const msg_config &g = c->cfg;
+    tr.mark(4, c->stream); cudaEventSynchronize(tr.ev[4]);
+    float ms[4] = {0, 0, 0, 0};
+    for (int k = 0; k < 4; k++) if (tr.ev[k] && tr.ev[k + 1]) cudaEventElapsedTime(&ms[k], tr.ev[k], tr.ev[k + 1]);
+    if (tr.ev[0] && tr.ev[2] && !tr.ev[1]) cudaEventElapsedTime(&ms[1], tr.ev[0], tr.ev[2]);
+    float chunk = 0, gap = 0, dec = 0;
+    if (!c->ev_total.empty()) { cudaEventElapsedTime(&chunk, c->ev_total.back().first, c->ev_total.back().second); cudaEventElapsedTime(&gap, c->ev_total.back().second, tr.ev[0]); }
+    if (!c->ev_decode.empty()) cudaEventElapsedTime(&dec, c->ev_decode.back().first, c->ev_decode.back().second);
+    fprintf(stderr, "[msg finish rank %d] last chunk %.3f ms (decode %.3f), gap %.3f ms, allreduce %.3f ms, init %.3f ms, loop %.3f ms, tail %.3f ms\n",
+            g.rank, chunk, dec, gap, ms[0], ms[1], ms[2], ms[3]);
+    if (rsag_trace) {
+        // CTA 0's view of the exchanges (ns): RS stores | fence+flags | owner blocks | announce | AG wait | grid barrier | delta ; gather = gap to the next exchange
+        unsigned long long t[160]; cudaMemcpy(t, c->t_ui.p, sizeof t, cudaMemcpyDeviceToHost);
+        double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}; int nx = 0;
+        for (int k = 1; k < 20 && t[k * 8 + 7]; k++) {
+            for (int j = 0; j < 7; j++) acc[j] += (double)(t[k * 8 + j + 1] - t[k * 8 + j]);
+            if (k + 1 < 20 && t[(k + 1) * 8]) acc[7] += (double)(t[(k + 1) * 8] - t[k * 8 + 7]);
+            nx++;
+        }
+        if (nx) fprintf(stderr, "[msg finish rank %d] rsag exchange, mean over %d (us): rs-store %.1f fence+flags %.1f owner %.1f announce %.1f ag-wait %.1f barrier %.1f delta %.1f | gather+barrier %.1f\n",
+                        g.rank, nx, acc[0] / nx / 1e3, acc[1] / nx / 1e3, acc[2] / nx / 1e3, acc[3] / nx / 1e3, acc[4] / nx / 1e3, acc[5] / nx / 1e3, acc[6] / nx / 1e3, acc[7] / nx / 1e3);
+    }
+    for (auto e : tr.ev) if (e) cudaEventDestroy(e);
+}
+
 int msg_finish_profile(msg_ctx *c, double *abundance, msg_profile_stats *st)
 {
     if (!c) return MSG_EINVAL;
@@ -1351,200 +1523,43 @@ int msg_finish_profile(msg_ctx *c, double *abundance, msg_profile_stats *st)
     const uint32_t F = (uint32_t)g.n_features;
     msg_profile_stats s; memset(&s, 0, sizeof s);
     int rc;
-    // work on copies so that finish can be called again after more chunks
-    uint32_t *ui = c->d_ui; double *dd = c->d_d; uint32_t *cnt = c->d_counters;
-    DevBuf &t_ui = c->t_ui, &t_d = c->t_d;
-    unsigned long long nl_global = c->csr_lists;
-    // MSG_TRACE_FINISH=1: device-side time of each phase, printed to stderr (diagnostics only)
     static const bool trace = getenv("MSG_TRACE_FINISH") != nullptr;
-    cudaEvent_t tev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    auto tmark = [&](int k) { if (trace) { if (!tev[k]) cudaEventCreate(&tev[k]); cudaEventRecord(tev[k], c->stream); } };
-    tmark(0);
+    FinishTrace tr{trace};
+    tr.mark(0, c->stream);
     // every small result is copied into pinned memory and read after ONE stream sync at the end
     uint32_t *hc = c->h_pin + 20; int32_t *res = reinterpret_cast<int32_t *>(c->h_pin + 16); uint32_t *h_purged = c->h_pin + 26;
     double *h_delta = reinterpret_cast<double *>(c->h_pin + 32);
     memset(c->h_pin + 16, 0, 4 * (72 - 16));
-    // proportional sharing over peer memory: the loop kernel also exchanges the counts, so no NCCL call and no em_init
-    const bool coop_multi = g.n_ranks > 1 && c->p2p_ok && F > 0 && g.share_type == MSG_MULTI_PROPORTIONAL && !getenv("MSG_EM_HOST_LOOP");
-    if (coop_multi) {
-    } else if (g.n_ranks > 1) {
-        // ONE allreduce over NVLink for everything that is additive across ranks: per-reference counts,
-        // the insert counters and the number of multi-mapper lists, packed as u32[F + 8]
-        CU(t_ui.reserve(((size_t)F + 8) * 4));
-        ui = t_ui.as<uint32_t>(); cnt = ui + F;
-        CU(cudaMemcpyAsync(ui, c->d_ui, (size_t)F * 4, cudaMemcpyDeviceToDevice, c->stream));
-        CU(cudaMemcpyAsync(cnt, c->d_counters, 16, cudaMemcpyDeviceToDevice, c->stream));
-        const uint32_t nl_lo[2] = {(uint32_t)(c->csr_lists & 0xffffu), (uint32_t)(c->csr_lists >> 16)};   // two 16-bit halves: sums stay exact in u32 for up to 65536 ranks
-        CU(cudaMemcpyAsync(cnt + 4, nl_lo, 8, cudaMemcpyHostToDevice, c->stream));
-        if ((rc = allreduce(c, ui, (size_t)F + 6, ncclUint32, ncclSum))) return rc;
-        if (g.share_type == MSG_MULTI_EQUAL) {
-            CU(t_d.reserve((size_t)(F ? F : 1) * 8));
-            CU(cudaMemcpyAsync(t_d.p, c->d_d, (size_t)F * 8, cudaMemcpyDeviceToDevice, c->stream));
-            dd = t_d.as<double>();
-            if ((rc = allreduce(c, dd, F, ncclFloat64, ncclSum))) return rc;
+    const bool em = g.share_type == MSG_MULTI_PROPORTIONAL;
+    const bool coop = em && F > 0 && (g.n_ranks <= 1 || c->p2p_ok) && !getenv("MSG_EM_HOST_LOOP");
+    // with n_ranks > 1 the cooperative loop kernel also combines the counts, so no NCCL call and no em_init
+    if (!coop || g.n_ranks <= 1) {
+        uint32_t *ui = c->d_ui; double *dd = c->d_d;
+        if ((rc = finish_combine_counts(c, ui, dd, hc, tr))) return rc;
+        if (F) {
+            em_init_kernel<<<nblocks(F, 256), 256, 0, c->stream>>>(ui, dd, g.share_type == MSG_MULTI_EQUAL, c->d_U, c->d_a, F, c->d_inc, c->d_delta,
+                                                                  reinterpret_cast<int32_t *>(c->d_total));
+            LAUNCHED(c);
         }
-        tmark(1);
-        CU(cudaMemcpyAsync(hc, cnt, 24, cudaMemcpyDeviceToHost, c->stream));
-    } else CU(cudaMemcpyAsync(hc, cnt, 16, cudaMemcpyDeviceToHost, c->stream));
-    if (F && !coop_multi) {
-        em_init_kernel<<<nblocks(F, 256), 256, 0, c->stream>>>(ui, dd, g.share_type == MSG_MULTI_EQUAL, c->d_U, c->d_a, F, c->d_inc, c->d_delta,
-                                                              reinterpret_cast<int32_t *>(c->d_total));
-        LAUNCHED(c);
     }
-    tmark(2);
-    const uint64_t ne_local = c->csr_ent;
-    const uint32_t nl32 = (uint32_t)c->csr_lists;
-    const uint32_t em_grid = nl32 ? (nblocks(nl32, 256) < 148u * 8u ? nblocks(nl32, 256) : 148u * 8u) : 0;
-    bool purged_done = false;
-    if (g.share_type == MSG_MULTI_PROPORTIONAL) {
-        const uint32_t nb = nblocks(F, 256);
-        bool looped = false;
-        if ((g.n_ranks <= 1 || c->p2p_ok) && F > 0 && !getenv("MSG_EM_HOST_LOOP")) {
-            // the whole loop is one cooperative launch (grid-wide barriers, no host round trips; with n_ranks > 1 the exchange is inside)
-            const bool sm = F <= EM_SMEM_F;
-            const size_t shm = sm ? (size_t)F * 8 * (1 + em_copies(F)) : 0;
-            int per_sm = 0, nsm = 0;
-            CU(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, g.device));
-            const bool rsag = g.n_ranks > 1 && F + 8 > EM_XCHG_CTA0;       // gene catalogues: reduce-scatter / all-gather exchange
-            if (rsag) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_loop_rsag_kernel, 256, 0));
-            else if (g.n_ranks > 1) {
-                if (sm) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_loop_multi_kernel<true>, 256, shm));
-                else    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_loop_multi_kernel<false>, 256, shm));
-            } else {
-                if (sm) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_loop_smem_kernel, 256, shm));
-                else    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, em_loop_kernel<false>, 256, shm));
-            }
-            if (per_sm < 1 && coop_multi) return fail(c, MSG_ECUDA, "cannot launch the cooperative PropSharing kernel (F = %u needs too much shared memory?)", F);
-            const int want_ctas = EM_CTAS_ENV > 0 ? EM_CTAS_ENV : (sm ? 3 : 4);
-            if (per_sm > want_ctas) per_sm = want_ctas;
-            if (per_sm >= 1) {
-                uint32_t grid = (uint32_t)(nsm * per_sm);
-                CU(c->tile_sums.reserve((size_t)grid * 8 + 16));
-                double *partial = c->tile_sums.as<double>();
-                int32_t *d_res = reinterpret_cast<int32_t *>(c->d_total);
-                const uint32_t *a0 = c->csr_off.as<uint32_t>(), *a1 = c->csr_len.as<uint32_t>(); const int32_t *a2 = c->csr_fid.as<int32_t>();
-                uint32_t nl_arg = nl32, F_arg = F;
-                const double *U = c->d_U; double *av = c->d_a, *inc = c->d_inc, *dout = c->d_delta;
-                PeerTable pt = c->peer_tab; int nr = g.n_ranks, rk = g.rank; uint32_t epoch = c->em_epoch;
-                void *args[] = {&a0, &a1, &a2, &nl_arg, &U, &av, &inc, &partial, &F_arg, &dout, &d_res};
-                // multi-GPU kernel: (lists..., ui, counters, nl_lo, nl_hi, U, a, inc, partial, F, delta, result, hc_out, peers, n_ranks, rank, epoch)
-                const uint32_t *ui_arg = c->d_ui, *cnt_arg = c->d_counters; double *Uw = c->d_U;
-                uint32_t nl_lo = (uint32_t)(c->csr_lists & 0xffffu), nl_hi = (uint32_t)(c->csr_lists >> 16);   // two 16-bit halves, as in the NCCL path
-                uint32_t *hc_dev = nullptr;
-                if (g.n_ranks > 1) { CU(c->t_cnt.reserve(64)); hc_dev = c->t_cnt.as<uint32_t>(); }
-                double *totbuf = nullptr; uint32_t *bflag = c->d_bflag;
-                if (g.n_ranks > 1) { CU(c->t_d.reserve((size_t)F * 16)); totbuf = c->t_d.as<double>(); }
-                static const double peer_timeout_s = getenv("MSG_PEER_TIMEOUT_S") ? atof(getenv("MSG_PEER_TIMEOUT_S")) : 120.0;
-                unsigned long long timeout_ns = (unsigned long long)(peer_timeout_s * 1e9);
-                void *margs[] = {&a0, &a1, &a2, &nl_arg, &ui_arg, &cnt_arg, &nl_lo, &nl_hi, &Uw, &av, &inc, &partial, &F_arg, &dout, &d_res, &hc_dev,
-                                 &totbuf, &bflag, &pt, &nr, &rk, &epoch, &timeout_ns};
-                unsigned long long *d_trace = nullptr;
-                if (trace && g.n_ranks > 1) { CU(c->t_ui.reserve(20 * 8 * 8)); d_trace = c->t_ui.as<unsigned long long>(); CU(cudaMemsetAsync(d_trace, 0, 20 * 8 * 8, c->stream)); }
-                void *rargs[] = {&a0, &a1, &a2, &nl_arg, &ui_arg, &cnt_arg, &nl_lo, &nl_hi, &Uw, &av, &inc, &F_arg, &dout, &d_res, &hc_dev,
-                                 &pt, &nr, &rk, &epoch, &timeout_ns, &d_trace};
-                // single GPU: inc[3F], delta and d_res were cleared by em_init_kernel; the multi-GPU kernel clears its own state
-                if (g.n_ranks > 1) {
-                    // The kernels of all ranks wait for one another inside the loop: line the ranks up first (a 4-byte NCCL
-                    // allreduce on the same stream; it waits, on the device, for however long the slowest rank's ingest takes),
-                    // so that the wall-clock limit inside the kernel (MSG_PEER_TIMEOUT_S, default 120 s) only ever measures a
-                    // peer that died, not one that is merely late.
-                    CU(cudaMemsetAsync(d_res, 0, 16, c->stream));
-                    CU(c->t_cnt.reserve(64));
-                    if ((rc = allreduce(c, c->t_cnt.as<uint32_t>() + 8, 1, ncclUint32, ncclSum))) return rc;
-                    if (rsag) {
-                        CU(cudaMemsetAsync(c->d_inc, 0, (size_t)F * 8, c->stream));
-                        CU(cudaLaunchCooperativeKernel((void *)em_loop_rsag_kernel, dim3(grid), dim3(256), rargs, 0, c->stream));
-                    }
-                    // compute + collective in one kernel: increments are exchanged through peer memory inside the loop
-                    else if (sm) CU(cudaLaunchCooperativeKernel((void *)em_loop_multi_kernel<true>, dim3(grid), dim3(256), margs, shm, c->stream));
-                    else         CU(cudaLaunchCooperativeKernel((void *)em_loop_multi_kernel<false>, dim3(grid), dim3(256), margs, shm, c->stream));
-                    c->em_epoch += 32;
-                    CU(cudaMemcpyAsync(hc, hc_dev, 24, cudaMemcpyDeviceToHost, c->stream));
-                } else {
-                    void *sargs[] = {&a0, &a1, &a2, &nl_arg, &U, &av, &inc, &F_arg, &dout, &d_res};
-                    if (sm) CU(cudaLaunchCooperativeKernel((void *)em_loop_smem_kernel, dim3(grid), dim3(256), sargs, shm, c->stream));
-                    else    CU(cudaLaunchCooperativeKernel((void *)em_loop_kernel<false>, dim3(grid), dim3(256), args, shm, c->stream));
-                }
-                LAUNCHED(c);
-                tmark(3);
-                CU(cudaMemcpyAsync(res, d_res, 16, cudaMemcpyDeviceToHost, c->stream));
-                CU(cudaMemcpyAsync(h_delta, c->d_delta, 8 * 20, cudaMemcpyDeviceToHost, c->stream));
-                c->d2h_bytes += 176;
-                purged_done = true;                              // both loop kernels count the purged lists themselves
-                looped = true;
-            }
-        }
-        for (int k = 1; !looped && k < 20; k++) {                                                            // msam_profile.c:331
-            CU(cudaMemsetAsync(c->d_inc, 0, (size_t)F * 8, c->stream));
-            if (nl32) {
-                if (F <= EM_SMEM_F) {
-                    em_gather_smem_kernel<<<em_grid, 256, (size_t)F * 16, c->stream>>>(c->csr_off.as<uint32_t>(), c->csr_len.as<uint32_t>(), c->csr_fid.as<int32_t>(), nl32, c->d_a, c->d_inc, F);
-                } else {
-                    em_gather_kernel<<<em_grid, 256, 0, c->stream>>>(c->csr_off.as<uint32_t>(), c->csr_len.as<uint32_t>(), c->csr_fid.as<int32_t>(), nl32, c->d_a, c->d_inc);
-                }
-                LAUNCHED(c);
-            }
-            if ((rc = allreduce(c, c->d_inc, F, ncclFloat64, ncclSum))) return rc;
-            double delta = 0;
-            if (F) {
-                em_update_kernel<<<nb, 256, 0, c->stream>>>(c->d_U, c->d_inc, c->d_a, c->d_partial, F); LAUNCHED(c);
-                em_delta_kernel<<<1, 256, 0, c->stream>>>(c->d_partial, nb, F, c->d_delta + (k - 1)); LAUNCHED(c);
-                CU(cudaMemcpyAsync(&delta, c->d_delta + (k - 1), 8, cudaMemcpyDeviceToHost, c->stream));
-                CU(cudaStreamSynchronize(c->stream));
-                c->d2h_bytes += 8;
-            } else delta = nan("");                                                           // reference divides by n_features == 0
-            s.em_delta[k - 1] = delta; s.em_iterations = k;
-            if (delta < 1e-10) { s.em_converged = 1; break; }                                     // :383
-        }
-        const bool coop = looped;
-        if (!purged_done) {
-        CU(cudaMemsetAsync(c->d_purged, 0, 4, c->stream));
-        if (nl32) { em_purged_kernel<<<em_grid, 256, 0, c->stream>>>(c->csr_off.as<uint32_t>(), c->csr_len.as<uint32_t>(), c->csr_fid.as<int32_t>(), nl32, c->d_a, c->d_purged); LAUNCHED(c); }
-        if ((rc = allreduce(c, c->d_purged, 1, ncclUint32, ncclSum))) return rc;
-        CU(cudaMemcpyAsync(h_purged, c->d_purged, 4, cudaMemcpyDeviceToHost, c->stream));
-        }
-        if (abundance && F) CU(cudaMemcpyAsync(c->h_ab, c->d_a, (size_t)F * 8, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaMemcpyAsync(c->h_pin + 8, c->d_err, 8, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaStreamSynchronize(c->stream));
-        if (coop) {
-            if (g.n_ranks > 1 && res[2]) return fail(c, MSG_ENCCL, "timed out waiting for a peer GPU inside the PropSharing loop");
-            s.em_iterations = res[0]; s.em_converged = res[1]; s.purged_insert_count = (uint32_t)res[3];
-            memcpy(s.em_delta, h_delta, sizeof s.em_delta);
-        } else s.purged_insert_count = *h_purged;
-    } else {
-        if (abundance && F) CU(cudaMemcpyAsync(c->h_ab, c->d_a, (size_t)F * 8, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaMemcpyAsync(c->h_pin + 8, c->d_err, 8, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaStreamSynchronize(c->stream));
-    }
-    if (trace) {
-        tmark(4); cudaEventSynchronize(tev[4]);
-        float ms[4] = {0, 0, 0, 0};
-        for (int k = 0; k < 4; k++) if (tev[k] && tev[k + 1]) cudaEventElapsedTime(&ms[k], tev[k], tev[k + 1]);
-        if (tev[0] && tev[2] && !tev[1]) cudaEventElapsedTime(&ms[1], tev[0], tev[2]);
-        float chunk = 0, gap = 0, dec = 0;
-        if (!c->ev_total.empty()) { cudaEventElapsedTime(&chunk, c->ev_total.back().first, c->ev_total.back().second); cudaEventElapsedTime(&gap, c->ev_total.back().second, tev[0]); }
-        if (!c->ev_decode.empty()) cudaEventElapsedTime(&dec, c->ev_decode.back().first, c->ev_decode.back().second);
-        fprintf(stderr, "[msg finish rank %d] last chunk %.3f ms (decode %.3f), gap %.3f ms, allreduce %.3f ms, init %.3f ms, loop %.3f ms, tail %.3f ms\n",
-                g.rank, chunk, dec, gap, ms[0], ms[1], ms[2], ms[3]);
-        if (g.n_ranks > 1 && F + 8 > EM_XCHG_CTA0 && c->t_ui.p && g.share_type == MSG_MULTI_PROPORTIONAL) {
-            // CTA 0's view of the exchanges (ns): RS stores | fence+flags | owner blocks | announce | AG wait | grid barrier | delta ; gather = gap to the next exchange
-            unsigned long long tr[160]; cudaMemcpy(tr, c->t_ui.p, sizeof tr, cudaMemcpyDeviceToHost);
-            double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}; int nx = 0;
-            for (int k = 1; k < 20 && tr[k * 8 + 7]; k++) {
-                for (int j = 0; j < 7; j++) acc[j] += (double)(tr[k * 8 + j + 1] - tr[k * 8 + j]);
-                if (k + 1 < 20 && tr[(k + 1) * 8]) acc[7] += (double)(tr[(k + 1) * 8] - tr[k * 8 + 7]);
-                nx++;
-            }
-            if (nx) fprintf(stderr, "[msg finish rank %d] rsag exchange, mean over %d (us): rs-store %.1f fence+flags %.1f owner %.1f announce %.1f ag-wait %.1f barrier %.1f delta %.1f | gather+barrier %.1f\n",
-                            g.rank, nx, acc[0] / nx / 1e3, acc[1] / nx / 1e3, acc[2] / nx / 1e3, acc[3] / nx / 1e3, acc[4] / nx / 1e3, acc[5] / nx / 1e3, acc[6] / nx / 1e3, acc[7] / nx / 1e3);
-        }
-        for (auto e : tev) if (e) cudaEventDestroy(e);
-    }
+    tr.mark(2, c->stream);
+    bool looped = false;                              // the cooperative loop ran; it counts the purged lists itself
+    if (coop && (rc = em_coop_loop(c, hc, res, h_delta, tr, &looped))) return rc;
+    if (em && !looped && (rc = em_host_loop(c, s, h_purged))) return rc;
+    if (abundance && F) CU(cudaMemcpyAsync(c->h_ab, c->d_a, (size_t)F * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(c->h_pin + 8, c->d_err, 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (looped) {
+        if (g.n_ranks > 1 && res[2]) return fail(c, MSG_ENCCL, "timed out waiting for a peer GPU inside the PropSharing loop");
+        s.em_iterations = res[0]; s.em_converged = res[1]; s.purged_insert_count = (uint32_t)res[3];
+        memcpy(s.em_delta, h_delta, sizeof s.em_delta);
+    } else if (em) s.purged_insert_count = *h_purged;
+    if (tr.on) finish_trace_report(c, tr, looped && g.n_ranks > 1 && F + 8 > EM_XCHG_CTA0);
     if (abundance && F) memcpy(abundance, c->h_ab, (size_t)F * 8);
     c->d2h_bytes += (size_t)F * 8 + 28;
-    if (g.n_ranks > 1) nl_global = (unsigned long long)hc[4] + ((unsigned long long)hc[5] << 16);
     s.mapped_inserts = hc[0]; s.uniq_mapper_count = hc[1]; s.multi_mapper_count = hc[2];
-    s.multi_lists = nl_global; s.multi_entries = ne_local;
+    s.multi_lists = g.n_ranks > 1 ? (unsigned long long)hc[4] + ((unsigned long long)hc[5] << 16) : c->csr_lists;
+    s.multi_entries = c->csr_ent;
     if (st) *st = s;
     return report_device_errors(c, c->h_pin + 8);
 }

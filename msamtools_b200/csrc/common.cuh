@@ -57,12 +57,6 @@ __device__ __forceinline__ uint4 ldg_stream128_line(const uint4 *p)
     return r;
 }
 
-__device__ __forceinline__ uint32_t warp_sum_u32(uint32_t v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 __device__ __forceinline__ unsigned long long warp_sum_u64(unsigned long long v)
 {
 #pragma unroll

@@ -418,46 +418,15 @@ __global__ void em_init_kernel(const uint32_t *ui, const double *d, int use_d, d
     U[i] = u; a[i] = u;
     if (inc) { inc[i] = 0.0; inc[(size_t)n + i] = 0.0; inc[2 * (size_t)n + i] = 0.0; }      // three buffers (em_loop_smem_kernel)
 }
-__global__ void em_init_from_U_kernel(const double *U, double *a, uint32_t n)
-{
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = U[i];
-}
-
-// one thread per multi-mapper list: s = sum a[f] in list order; inc[f] += a[f]/s   (:341-365)
-// Large catalogs (F up to 1e6): the F-sized vectors live in L2, contention per address is low,
-// so the adds go straight to global memory.
-__global__ void __launch_bounds__(256) em_gather_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
-                                                        const double *a, double *inc)
-{
-    for (uint32_t l = blockIdx.x * blockDim.x + threadIdx.x; l < nlists; l += gridDim.x * blockDim.x) {
-        uint32_t b = mm_off[l], e = b + mm_len[l];
-        double s = 0;
-        for (uint32_t k = b; k < e; k++) s += a[mm_fid[k]];
-        if (s > 0) for (uint32_t k = b; k < e; k++) { int32_t f = mm_fid[k]; atomicAdd(inc + f, a[f] / s); }
-    }
-}
 // Small feature sets (genomes, F <= EM_SMEM_F): millions of lists hit a few hundred addresses.
 // Each CTA keeps a private copy of a[] and inc[] in shared memory and flushes inc once.
+// Large catalogs (F up to 1e6): the F-sized vectors live in L2, contention per address is low,
+// so the adds go straight to global memory.
 constexpr uint32_t EM_SMEM_F = 2048;
-// private inc copies per CTA in the cooperative loop kernels: one per warp while that stays under ~40 KB
+// private inc copies per CTA: one per warp while that stays under ~40 KB
 __host__ __device__ __forceinline__ uint32_t em_copies(uint32_t F) { return F <= 512 ? 8u : 1u; }
-__global__ void __launch_bounds__(256) em_gather_smem_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
-                                                             const double *a, double *inc, uint32_t F)
-{
-    extern __shared__ double s_em[];
-    double *sa = s_em, *si = s_em + F;
-    for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) { sa[i] = a[i]; si[i] = 0.0; }
-    __syncthreads();
-    for (uint32_t l = blockIdx.x * blockDim.x + threadIdx.x; l < nlists; l += gridDim.x * blockDim.x) {
-        uint32_t b = mm_off[l], e = b + mm_len[l];
-        double s = 0;
-        for (uint32_t k = b; k < e; k++) s += sa[mm_fid[k]];
-        if (s > 0) for (uint32_t k = b; k < e; k++) { int32_t f = mm_fid[k]; atomicAdd(si + f, sa[f] / s); }
-    }
-    __syncthreads();
-    for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) { double v = si[i]; if (v != 0.0) atomicAdd(inc + i, v); }
-}
+// dynamic shared memory of a gather that works from shared memory: a[F] | inc copies [em_copies(F)][F]
+__host__ __device__ __forceinline__ size_t em_smem_bytes(uint32_t F) { return F <= EM_SMEM_F ? (size_t)F * 8 * (1 + em_copies(F)) : 0; }
 
 // One multi-mapper list in one PropSharing iteration: s = sum of a[f] in list order, inc[f] += a[f] / s (:341-365).
 // The first four features (almost every list) stay in registers between the two passes; the share is a[f] * (1/s),
@@ -502,112 +471,148 @@ __device__ __forceinline__ void em_share_list_pair(const int32_t *mm_fid, uint32
     }
 }
 
-// a_new = U + inc; flush < 1e-20; per-block partial of sum (a_new - a_old)^2 in a fixed order  (:369-379)
+// The gather of one iteration (:341-365) over this thread's lists of a grid-stride walk (first, first + stride, ...):
+// lists l and l + stride as a pair, then at most one lone list.
+__device__ __forceinline__ void em_share_lists(uint32_t first, uint32_t stride, const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid,
+                                               uint32_t nlists, const double *av, double *iv)
+{
+    uint32_t l = first;
+    for (; l + stride < nlists; l += 2 * stride) em_share_list_pair(mm_fid, mm_off[l], mm_len[l], mm_off[l + stride], mm_len[l + stride], av, iv);
+    if (l < nlists) em_share_list(mm_fid, mm_off[l], mm_len[l], av, iv);
+}
+
+// The gather with F <= EM_SMEM_F: sa[F] holds a[] (written before the call by this CTA), si[] the em_copies(F) private
+// inc copies.  With few features every warp gets a copy of its own, so the (CAS-loop) f64 shared atomics only collide
+// inside a warp.  The summed copies are added to the global inc[] = inc_at() once per CTA.  inc_at is called after the
+// walk: a triple-buffer pointer formed before it and held across it makes em_loop_smem_kernel spill.
+template <class IncAt>
+__device__ __forceinline__ void em_gather_smem(uint32_t first, uint32_t stride, const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid,
+                                               uint32_t nlists, const double *sa, double *si, IncAt inc_at, uint32_t F)
+{
+    const uint32_t ncopy = em_copies(F);
+    for (uint32_t i = threadIdx.x; i < F * ncopy; i += blockDim.x) si[i] = 0.0;
+    __syncthreads();
+    em_share_lists(first, stride, mm_off, mm_len, mm_fid, nlists, sa, si + (size_t)((threadIdx.x >> 5) % ncopy) * F);
+    __syncthreads();
+    double *inc = inc_at();
+    for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) {
+        double v = 0.0;
+        for (uint32_t cp = 0; cp < ncopy; cp++) v += si[(size_t)cp * F + i];
+        if (v != 0.0) atomicAdd(inc + i, v);
+    }
+}
+
+// Sum of v over the 256 threads of the CTA, in one fixed tree order, so that every CTA that sums the same values gets
+// the same bits (and takes the same stop decision).  The caller synchronises before it writes s_red again.
+__device__ __forceinline__ double em_block_sum(double *s_red, double v)
+{
+    s_red[threadIdx.x] = v;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
+    return s_red[0];
+}
+
+// a_new = U + inc, flushed to 0 below 1e-20  (:369-376)
+__device__ __forceinline__ double em_new_abundance(double u, double inc)
+{
+    const double an = u + inc;
+    return an < 1e-20 ? 0.0 : an;
+}
+
+// purged = #lists whose final abundances sum to exactly 0  (:394-404): this thread's lists of a grid-stride walk,
+// one atomic per warp into *purged
+__device__ __forceinline__ void em_count_purged(uint32_t first, uint32_t stride, const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid,
+                                                uint32_t nlists, const double *av, uint32_t *purged)
+{
+    uint32_t z = 0;
+    for (uint32_t l = first; l < nlists; l += stride) {
+        const uint32_t b = mm_off[l], e = b + mm_len[l];
+        double sum = 0;
+        for (uint32_t q = b; q < e; q++) sum += av[mm_fid[q]];
+        z += (sum == 0);
+    }
+    z = __reduce_add_sync(0xffffffffu, z);
+    if ((threadIdx.x & 31u) == 0 && z) atomicAdd(purged, z);
+}
+
+// The host loop (NCCL fallback): one launch per phase.  Gather, with a[] copied into shared memory for F <= EM_SMEM_F.
+__global__ void __launch_bounds__(256) em_gather_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
+                                                        const double *a, double *inc, uint32_t F)
+{
+    extern __shared__ double s_em[];
+    const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
+    if (F <= EM_SMEM_F) {
+        for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) s_em[i] = a[i];
+        em_gather_smem(gtid, gsz, mm_off, mm_len, mm_fid, nlists, s_em, s_em + F, [&] { return inc; }, F);
+    } else em_share_lists(gtid, gsz, mm_off, mm_len, mm_fid, nlists, a, inc);
+}
+// a = U + inc; per-block partial of sum (a_new - a_old)^2 in a fixed order  (:369-379)
 __global__ void __launch_bounds__(256) em_update_kernel(const double *U, const double *inc, double *a, double *partial, uint32_t n)
 {
-    __shared__ double s[256];
+    __shared__ double s_red[256];
     uint32_t i = blockIdx.x * 256 + threadIdx.x;
     double dd = 0;
     if (i < n) {
-        double an = U[i] + inc[i];
-        if (an < 1e-20) an = 0;
-        double diff = an - a[i];
+        const double an = em_new_abundance(U[i], inc[i]);
+        const double diff = an - a[i];
         dd = diff * diff;
         a[i] = an;
     }
-    s[threadIdx.x] = dd;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o]; __syncthreads(); }
-    if (threadIdx.x == 0) partial[blockIdx.x] = s[0];
+    const double sum = em_block_sum(s_red, dd);
+    if (threadIdx.x == 0) partial[blockIdx.x] = sum;
 }
 __global__ void __launch_bounds__(256) em_delta_kernel(const double *partial, uint32_t nblocks, uint32_t n, double *delta_out)
 {
-    __shared__ double s[256];
+    __shared__ double s_red[256];
     double acc = 0;
     for (uint32_t b = threadIdx.x; b < nblocks; b += 256) acc += partial[b];
-    s[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o]; __syncthreads(); }
-    if (threadIdx.x == 0) *delta_out = s[0] / n;                        // :380
+    const double sum = em_block_sum(s_red, acc);
+    if (threadIdx.x == 0) *delta_out = sum / n;                         // :380
 }
+__global__ void __launch_bounds__(256) em_purged_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
+                                                        const double *a, uint32_t *purged)
+{
+    em_count_purged(blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x, mm_off, mm_len, mm_fid, nlists, a, purged);
+}
+
 // The whole PropSharing loop (msam_profile.c:331-389) in ONE cooperative launch (single-GPU case): grid-wide
 // barriers replace the per-iteration launches and the host's read of delta.  Every CTA recomputes delta from the
 // per-CTA partials in the same fixed order, so all of them take the same stop decision.  result[0] = last k,
 // result[1] = converged flag; delta_out[k-1] = DELTA^2 of iteration k.
-template <bool SMEM>
 __global__ void __launch_bounds__(256) em_loop_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
                                                       const double *U, double *a, double *inc, double *partial, uint32_t F,
                                                       double *delta_out, int32_t *result)
 {
     namespace cg = cooperative_groups;
     cg::grid_group grid = cg::this_grid();
-    extern __shared__ double s_em[];
     __shared__ double s_red[256];
-    // shared layout: a[F] | inc copies [ncopy][F].  With few features every warp gets a private copy of inc, so the
-    // (CAS-loop) f64 shared atomics only collide inside a warp.
-    const uint32_t ncopy = SMEM ? em_copies(F) : 1u;
-    double *sa = s_em, *si = s_em + F;
     const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
     int k = 1, conv = 0;
     for (; k < 20; k++) {
-        // gather: s = sum a[f] in list order; inc[f] += a[f]/s            (:341-365)
-        if (SMEM) {
-            for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) sa[i] = a[i];
-            for (uint32_t i = threadIdx.x; i < F * ncopy; i += blockDim.x) si[i] = 0.0;
-            __syncthreads();
-        }
-        const double *av = SMEM ? sa : a;
-        double *iv = SMEM ? si + (size_t)((threadIdx.x >> 5) % ncopy) * F : inc;
-        {
-            uint32_t l = gtid;
-            for (; l + gsz < nlists; l += 2 * gsz) em_share_list_pair(mm_fid, mm_off[l], mm_len[l], mm_off[l + gsz], mm_len[l + gsz], av, iv);
-            if (l < nlists) em_share_list(mm_fid, mm_off[l], mm_len[l], av, iv);
-        }
-        if (SMEM) {
-            __syncthreads();
-            for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) {
-                double v = 0.0;
-                for (uint32_t cp = 0; cp < ncopy; cp++) v += si[(size_t)cp * F + i];
-                if (v != 0.0) atomicAdd(inc + i, v);
-            }
-        }
+        em_share_lists(gtid, gsz, mm_off, mm_len, mm_fid, nlists, a, inc);
         grid.sync();
-        // update: a = U + inc, flush < 1e-20, per-CTA partial of sum diff^2; inc is cleared for the next iteration   (:369-379)
+        // update: a = U + inc, per-CTA partial of sum diff^2; inc is cleared for the next iteration   (:369-379)
         double dd = 0;
         for (uint32_t i = gtid; i < F; i += gsz) {
-            double an = U[i] + inc[i];
-            if (an < 1e-20) an = 0;
+            const double an = em_new_abundance(U[i], inc[i]);
             const double diff = an - a[i];
             dd += diff * diff;
             a[i] = an; inc[i] = 0.0;
         }
-        s_red[threadIdx.x] = dd;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-        if (threadIdx.x == 0) partial[blockIdx.x] = s_red[0];
+        const double part = em_block_sum(s_red, dd);
+        if (threadIdx.x == 0) partial[blockIdx.x] = part;
         grid.sync();
         // delta (every CTA, same order)                                   (:380-383)
         double acc = 0;
         for (uint32_t b = threadIdx.x; b < gridDim.x; b += 256) acc += partial[b];
-        s_red[threadIdx.x] = acc;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-        const double delta = s_red[0] / F;
+        const double delta = em_block_sum(s_red, acc) / F;
         __syncthreads();
         if (gtid == 0) delta_out[k - 1] = delta;
         if (delta < 1e-10) { conv = 1; break; }
     }
     if (gtid == 0) { result[0] = k < 20 ? k : 19; result[1] = conv; }
-    // purged = #lists whose final abundances sum to exactly 0  (:394-404); a[] is final and visible (second grid.sync above)
-    uint32_t z = 0;
-    for (uint32_t l = gtid; l < nlists; l += gsz) {
-        const uint32_t b = mm_off[l], e = b + mm_len[l];
-        double sum = 0;
-        for (uint32_t q = b; q < e; q++) sum += a[mm_fid[q]];
-        z += (sum == 0);
-    }
-    z = warp_sum_u32(z);
-    if ((threadIdx.x & 31) == 0 && z) atomicAdd(reinterpret_cast<uint32_t *>(result + 3), z);
+    // a[] is final and visible (second grid.sync above)
+    em_count_purged(gtid, gsz, mm_off, mm_len, mm_fid, nlists, a, reinterpret_cast<uint32_t *>(result + 3));
 }
 
 // Single GPU, F <= EM_SMEM_F: the loop with ONE grid barrier per iteration.  Every CTA keeps the whole abundance vector
@@ -624,57 +629,32 @@ __global__ void __launch_bounds__(256) em_loop_smem_kernel(const uint32_t *mm_of
     cg::grid_group grid = cg::this_grid();
     extern __shared__ double s_em[];
     __shared__ double s_red[256];
-    const uint32_t ncopy = em_copies(F);
-    double *sa = s_em, *si = s_em + F;
+    double *sa = s_em;
     const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
     for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) sa[i] = a[i];
     int k = 1, conv = 0;
     for (; k < 20; k++) {
-        for (uint32_t i = threadIdx.x; i < F * ncopy; i += blockDim.x) si[i] = 0.0;
-        __syncthreads();
-        // gather: s = sum a[f] in list order; inc[f] += a[f]/s            (:341-365)
-        double *iv = si + (size_t)((threadIdx.x >> 5) % ncopy) * F;
-        uint32_t l = gtid;
-        for (; l + gsz < nlists; l += 2 * gsz) em_share_list_pair(mm_fid, mm_off[l], mm_len[l], mm_off[l + gsz], mm_len[l + gsz], sa, iv);
-        if (l < nlists) em_share_list(mm_fid, mm_off[l], mm_len[l], sa, iv);
-        __syncthreads();
-        double *inc = inc3 + (size_t)(k % 3) * F;
-        for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) {
-            double v = 0.0;
-            for (uint32_t cp = 0; cp < ncopy; cp++) v += si[(size_t)cp * F + i];
-            if (v != 0.0) atomicAdd(inc + i, v);
-        }
+        em_gather_smem(gtid, gsz, mm_off, mm_len, mm_fid, nlists, sa, s_em + F, [&] { return inc3 + (size_t)(k % 3) * F; }, F);
         grid.sync();
+        const double *inc = inc3 + (size_t)(k % 3) * F;
         if (blockIdx.x == 0) { double *nxt = inc3 + (size_t)((k + 2) % 3) * F; for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) nxt[i] = 0.0; }
-        // update (every CTA, all features): a = U + inc, flush < 1e-20, delta = sum diff^2 / F   (:369-383)
+        // update (every CTA, all features): a = U + inc, delta = sum diff^2 / F   (:369-383)
         double dd = 0;
         for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) {
-            double an = U[i] + __ldcg(inc + i);
-            if (an < 1e-20) an = 0;
+            const double an = em_new_abundance(U[i], __ldcg(inc + i));
             const double diff = an - sa[i];
             dd += diff * diff;
             sa[i] = an;
         }
-        s_red[threadIdx.x] = dd;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-        const double delta = s_red[0] / F;
+        const double delta = em_block_sum(s_red, dd) / F;
         __syncthreads();
         if (gtid == 0) delta_out[k - 1] = delta;
         if (delta < 1e-10) { conv = 1; break; }
     }
     if (blockIdx.x == 0) for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) a[i] = sa[i];
     if (gtid == 0) { result[0] = k < 20 ? k : 19; result[1] = conv; }
-    // purged = #lists whose final abundances sum to exactly 0  (:394-404), from this CTA's own (identical) copy of a[]
-    uint32_t z = 0;
-    for (uint32_t l = gtid; l < nlists; l += gsz) {
-        const uint32_t b = mm_off[l], e = b + mm_len[l];
-        double sum = 0;
-        for (uint32_t q = b; q < e; q++) sum += sa[mm_fid[q]];
-        z += (sum == 0);
-    }
-    z = warp_sum_u32(z);
-    if ((threadIdx.x & 31) == 0 && z) atomicAdd(reinterpret_cast<uint32_t *>(result + 3), z);
+    // from this CTA's own (identical) copy of a[]
+    em_count_purged(gtid, gsz, mm_off, mm_len, mm_fid, nlists, sa, reinterpret_cast<uint32_t *>(result + 3));
 }
 
 // Multi-GPU PropSharing: counts exchange + the whole loop + the purged total in ONE cooperative kernel per GPU, with
@@ -722,8 +702,7 @@ __global__ void __launch_bounds__(256) em_loop_multi_kernel(const uint32_t *mm_o
     cg::grid_group grid = cg::this_grid();
     extern __shared__ double s_em[];
     __shared__ double s_red[256];
-    const uint32_t ncopy = SMEM ? em_copies(F) : 1u;
-    double *sa = s_em, *si = s_em + F;
+    double *sa = s_em;
     const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
     const uint32_t V = F + 8;
     // who takes part in the exchanges
@@ -769,7 +748,7 @@ __global__ void __launch_bounds__(256) em_loop_multi_kernel(const uint32_t *mm_o
                  [&](uint32_t i, double tot) { if (i < F) { const double u = tot / 2; U[i] = u; a[i] = u; inc[i] = 0.0; } else hc_out[i - F] = (uint32_t)tot; });
     grid.sync();
     int k = 1, conv = 0;
-    if (SMEM) {
+    if constexpr (SMEM) {
         // F <= EM_SMEM_F: ONE grid barrier per iteration.  After the barrier that completes inc[], CTA 0 exchanges the
         // increments with the peers and broadcasts the rank-ordered totals through totbuf[k & 1] + a release flag; every
         // CTA then redoes the F-sized update and the delta reduction from its own shared-memory a[] (same data, same order:
@@ -777,18 +756,7 @@ __global__ void __launch_bounds__(256) em_loop_multi_kernel(const uint32_t *mm_o
         // next gather (which starts only after they have seen the flag) adds into zeros.
         for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) sa[i] = __ldcg(a + i);
         for (; k < 20; k++) {
-            for (uint32_t i = threadIdx.x; i < F * ncopy; i += blockDim.x) si[i] = 0.0;
-            __syncthreads();
-            double *iv = si + (size_t)((threadIdx.x >> 5) % ncopy) * F;
-            uint32_t l = gtid;
-            for (; l + gsz < nlists; l += 2 * gsz) em_share_list_pair(mm_fid, mm_off[l], mm_len[l], mm_off[l + gsz], mm_len[l + gsz], sa, iv);
-            if (l < nlists) em_share_list(mm_fid, mm_off[l], mm_len[l], sa, iv);
-            __syncthreads();
-            for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) {
-                double v = 0.0;
-                for (uint32_t cp = 0; cp < ncopy; cp++) v += si[(size_t)cp * F + i];
-                if (v != 0.0) atomicAdd(inc + i, v);
-            }
+            em_gather_smem(gtid, gsz, mm_off, mm_len, mm_fid, nlists, sa, s_em + F, [&] { return inc; }, F);
             grid.sync();
             double *tb = totbuf + (size_t)(k & 1) * F;
             if (blockIdx.x == 0) {
@@ -812,79 +780,45 @@ __global__ void __launch_bounds__(256) em_loop_multi_kernel(const uint32_t *mm_o
                 dd += diff * diff;
                 sa[i] = an;
             }
-            s_red[threadIdx.x] = dd;
-            __syncthreads();
-            for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-            const double delta = s_red[0] / F;
+            const double delta = em_block_sum(s_red, dd) / F;
             __syncthreads();
             if (gtid == 0) delta_out[k - 1] = delta;
             if (delta < 1e-10) { conv = 1; break; }
         }
         if (blockIdx.x == 0) for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) a[i] = sa[i];
-    } else
-    for (; k < 20; k++) {
-        if (SMEM) {
-            for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) sa[i] = a[i];
-            for (uint32_t i = threadIdx.x; i < F * ncopy; i += blockDim.x) si[i] = 0.0;
-            __syncthreads();
-        }
-        const double *av = SMEM ? sa : a;
-        double *iv = SMEM ? si + (size_t)((threadIdx.x >> 5) % ncopy) * F : inc;
-        {
-            uint32_t l = gtid;
-            for (; l + gsz < nlists; l += 2 * gsz) em_share_list_pair(mm_fid, mm_off[l], mm_len[l], mm_off[l + gsz], mm_len[l + gsz], av, iv);
-            if (l < nlists) em_share_list(mm_fid, mm_off[l], mm_len[l], av, iv);
-        }
-        if (SMEM) {
-            __syncthreads();
-            for (uint32_t i = threadIdx.x; i < F; i += blockDim.x) {
-                double v = 0.0;
-                for (uint32_t cp = 0; cp < ncopy; cp++) v += si[(size_t)cp * F + i];
-                if (v != 0.0) atomicAdd(inc + i, v);
+    } else {
+        for (; k < 20; k++) {
+            em_share_lists(gtid, gsz, mm_off, mm_len, mm_fid, nlists, a, inc);
+            grid.sync();
+            // exchange the increments; a = U + total, flush < 1e-20, per-CTA partial of sum diff^2   (:369-379)
+            if (part) {
+                double dd = 0;
+                exchange((uint32_t)k, (uint32_t)k & 1u,
+                         [&](uint32_t i) -> double { if (i >= F) return 0.0; const double v = inc[i]; inc[i] = 0.0; return v; },
+                         [&](uint32_t i, double tot) {
+                             if (i >= F) return;
+                             double an = U[i] + tot;
+                             if (an < 1e-20) an = 0;
+                             const double diff = an - a[i];
+                             dd += diff * diff;
+                             a[i] = an;
+                         });
+                const double sum = em_block_sum(s_red, dd);
+                if (threadIdx.x == 0) partial[blockIdx.x] = sum;
             }
-        }
-        grid.sync();
-        // exchange the increments; a = U + total, flush < 1e-20, per-CTA partial of sum diff^2   (:369-379)
-        if (part) {
-            double dd = 0;
-            exchange((uint32_t)k, (uint32_t)k & 1u,
-                     [&](uint32_t i) -> double { if (i >= F) return 0.0; const double v = inc[i]; inc[i] = 0.0; return v; },
-                     [&](uint32_t i, double tot) {
-                         if (i >= F) return;
-                         double an = U[i] + tot;
-                         if (an < 1e-20) an = 0;
-                         const double diff = an - a[i];
-                         dd += diff * diff;
-                         a[i] = an;
-                     });
-            s_red[threadIdx.x] = dd;
+            grid.sync();
+            // delta (every CTA, same order)                                   (:380-383)
+            double acc = 0;
+            for (uint32_t b = threadIdx.x; b < nparts; b += 256) acc += __ldcg(partial + b);
+            const double delta = em_block_sum(s_red, acc) / F;
             __syncthreads();
-            for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-            if (threadIdx.x == 0) partial[blockIdx.x] = s_red[0];
+            if (gtid == 0) delta_out[k - 1] = delta;
+            if (delta < 1e-10) { conv = 1; break; }
         }
-        grid.sync();
-        // delta (every CTA, same order)                                   (:380-383)
-        double acc = 0;
-        for (uint32_t b = threadIdx.x; b < nparts; b += 256) acc += __ldcg(partial + b);
-        s_red[threadIdx.x] = acc;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-        const double delta = s_red[0] / F;
-        __syncthreads();
-        if (gtid == 0) delta_out[k - 1] = delta;
-        if (delta < 1e-10) { conv = 1; break; }
     }
     // ---- purged = #lists whose final abundances sum to exactly 0 (:394-404), summed over ranks through the same regions
     {
-        uint32_t z = 0;
-        for (uint32_t l = gtid; l < nlists; l += gsz) {
-            const uint32_t b = mm_off[l], e = b + mm_len[l];
-            double sum = 0;
-            for (uint32_t q = b; q < e; q++) sum += SMEM ? sa[mm_fid[q]] : a[mm_fid[q]];
-            z += (sum == 0);
-        }
-        z = __reduce_add_sync(0xffffffffu, z);
-        if ((threadIdx.x & 31u) == 0 && z) atomicAdd(reinterpret_cast<uint32_t *>(result + 3), z);
+        em_count_purged(gtid, gsz, mm_off, mm_len, mm_fid, nlists, SMEM ? sa : a, reinterpret_cast<uint32_t *>(result + 3));
         grid.sync();
         if (blockIdx.x == 0 && threadIdx.x == 0) {
             const unsigned long long want = (unsigned long long)(epoch + 24u);
@@ -1062,10 +996,8 @@ __global__ void __launch_bounds__(256) em_loop_rsag_kernel(const uint32_t *mm_of
             }
             for (uint32_t r = 0; r < N; r++)
                 st_weak_v2f64(reinterpret_cast<double *>(peers.base[r] + L.ag_data()) + (size_t)par * N * S + i0, n0, n1);
-            s_red[threadIdx.x] = dd;
-            __syncthreads();
-            for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-            if (threadIdx.x == 0) s_dd[nmine] = s_red[0];
+            const double bsum = em_block_sum(s_red, dd);
+            if (threadIdx.x == 0) s_dd[nmine] = bsum;
             nmine++;
             if (nmine == RSAG_MAXB) {                       // (huge catalogues only)
                 __syncthreads();
@@ -1103,10 +1035,7 @@ __global__ void __launch_bounds__(256) em_loop_rsag_kernel(const uint32_t *mm_of
                 ll_load(reinterpret_cast<const unsigned long long *>(me + L.dd()) + ((size_t)par * N * nblk + q) * 2, w0, w1);
                 acc += __longlong_as_double((long long)((w1 << 32) | (w0 & 0xffffffffull)));
             }
-        s_red[threadIdx.x] = acc;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) { if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o]; __syncthreads(); }
-        const double delta = s_red[0] / F;
+        const double delta = em_block_sum(s_red, acc) / F;
         __syncthreads();
         stamp(k, 7);
         return delta;
@@ -1142,12 +1071,7 @@ __global__ void __launch_bounds__(256) em_loop_rsag_kernel(const uint32_t *mm_of
     int k = 1, conv = 0;
     for (; k < 20; k++) {
         // gather: s = sum a[f] in list order; inc[f] += a[f]/s            (:341-365)
-        const double *av = a_buf((uint32_t)(k - 1) & 1u);
-        {
-            uint32_t l = gtid;
-            for (; l + gsz < nlists; l += 2 * gsz) em_share_list_pair(mm_fid, mm_off[l], mm_len[l], mm_off[l + gsz], mm_len[l + gsz], av, inc);
-            if (l < nlists) em_share_list(mm_fid, mm_off[l], mm_len[l], av, inc);
-        }
+        em_share_lists(gtid, gsz, mm_off, mm_len, mm_fid, nlists, a_buf((uint32_t)(k - 1) & 1u), inc);
         grid.sync();
         const double delta = exchange((uint32_t)k, false);
         if (gtid == 0) delta_out[k - 1] = delta;
@@ -1159,15 +1083,7 @@ __global__ void __launch_bounds__(256) em_loop_rsag_kernel(const uint32_t *mm_of
         const uint32_t kl = k < 20 ? (uint32_t)k : 19u;
         const double *av = a_buf(kl & 1u);
         for (uint32_t i = gtid; i < F; i += gsz) a_out[i] = av[i];
-        uint32_t z = 0;
-        for (uint32_t l = gtid; l < nlists; l += gsz) {
-            const uint32_t b = mm_off[l], e = b + mm_len[l];
-            double sum = 0;
-            for (uint32_t q = b; q < e; q++) sum += av[mm_fid[q]];
-            z += (sum == 0);
-        }
-        z = __reduce_add_sync(0xffffffffu, z);
-        if ((threadIdx.x & 31u) == 0 && z) atomicAdd(reinterpret_cast<uint32_t *>(result + 3), z);
+        em_count_purged(gtid, gsz, mm_off, mm_len, mm_fid, nlists, av, reinterpret_cast<uint32_t *>(result + 3));
         grid.sync();
         // the purged message also tells the peers that this rank is done reading its copy of a[]: only then may a peer's
         // next call overwrite it
@@ -1177,20 +1093,6 @@ __global__ void __launch_bounds__(256) em_loop_rsag_kernel(const uint32_t *mm_of
             result[0] = (int32_t)kl; result[1] = conv;
         }
     }
-}
-
-// purged = #lists whose final abundances sum to exactly 0  (:394-404)
-__global__ void __launch_bounds__(256) em_purged_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
-                                                        const double *a, uint32_t *purged)
-{
-    uint32_t z = 0;
-    for (uint32_t l = blockIdx.x * blockDim.x + threadIdx.x; l < nlists; l += gridDim.x * blockDim.x) {
-        double s = 0;
-        for (uint32_t k = mm_off[l]; k < mm_off[l] + mm_len[l]; k++) s += a[mm_fid[k]];
-        z += (s == 0);
-    }
-    z = warp_sum_u32(z);
-    if ((threadIdx.x & 31) == 0 && z) atomicAdd(purged, z);
 }
 
 struct InPcountPacked {      // (is_list << 32) | entries, for one packed u64 scan

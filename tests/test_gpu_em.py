@@ -2,10 +2,11 @@
 CPU oracle, on streams built to reach the loop's boundaries.
 
 msg_finish_profile runs the loop in one of four ways: em_loop_smem_kernel with 8 private inc copies per CTA (F <= 512)
-or 1 copy (F <= 2048), em_loop_kernel<false> with a[] and inc[] in global memory (F > 2048), or the host loop of
-em_gather(_smem)_kernel, em_update_kernel, em_delta_kernel and em_purged_kernel (MSG_EM_HOST_LOOP=1, read at every
-finish).  Both cooperative kernels walk the lists in grid stride, a thread taking lists l and l + gsz together and then
-at most one lone list; gsz = grid x 256 and the grid is nsm x min(occupancy, MSG_EM_CTAS or 3 / 4).  The tests cover:
+or 1 copy (F <= 2048), em_loop_kernel with a[] and inc[] in global memory (F > 2048), or the host loop of
+em_gather_kernel, em_update_kernel, em_delta_kernel and em_purged_kernel (MSG_EM_HOST_LOOP=1, read at every finish).
+All of them walk the lists in grid stride (em_share_lists), a thread taking lists l and l + gsz together and then at
+most one lone list; gsz = grid x 256, and the cooperative kernels' grid is nsm x min(occupancy, MSG_EM_CTAS or 3 / 4).
+The tests cover:
 - every implementation at F = 2 ... ~10 000;
 - the pair / lone boundaries with MSG_EM_CTAS=1 (gsz = nsm x 256 exactly), list counts 2 gsz q + r, every list at a
   boundary on features of its own, so that a lost or misweighted list moves abundances by O(1);
@@ -345,8 +346,8 @@ def loop(request, monkeypatch):
 @gpu
 @pytest.mark.parametrize("F", IMPL_F)
 def test_implementations(m, oracle, loop, F):
-    """each F picks em_loop_smem_kernel (8 or 1 inc copies), em_loop_kernel<false> or, with MSG_EM_HOST_LOOP=1, the
-    shared-memory or global host-loop gather; 20 000 lists through an fmap of 2F + 1 targets"""
+    """each F picks em_loop_smem_kernel (8 or 1 inc copies), em_loop_kernel or, with MSG_EM_HOST_LOOP=1, the
+    host-loop gather from shared or global memory; 20 000 lists through an fmap of 2F + 1 targets"""
     exp = run_named(m, oracle, "impl-%d" % F)
     assert exp[1]["iterations"] >= (2 if F == 2 else 5)
 

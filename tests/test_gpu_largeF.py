@@ -1,6 +1,6 @@
 """GPU parity on the feature counts the metric is quoted on: BASELINE.json configs[2] (10 k references)
 and configs[4] (1 M-gene catalogue).  These shapes leave the shared-memory fast paths (F <= 4096
-histograms, F <= 2048 PropSharing loop) and run `em_loop_kernel<false>`, `fused_warp_kernel<false>` and
+histograms, F <= 2048 PropSharing loop) and run `em_loop_kernel`, `fused_warp_kernel<false>` and
 `profile_warp_count_kernel<false>`; every case is compared with the CPU oracle on the same 2 M-record
 seeded stream: integer counts bit-exact, abundances within 1e-9 relative, same PropSharing iteration
 count / purged / list totals (msam_profile.c:331-404).
