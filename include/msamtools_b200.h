@@ -105,7 +105,15 @@ typedef struct msg_config {
                                     msg_finish_profile / msg_finish_coverage after pushes.  Needs want_profile and/or
                                     want_coverage, n_ranks == 1; not with want_records / want_kept / want_stats.
                                     Results equal those of the same records regrouped stably by QNAME (see below).    */
-    uint8_t  reserved0[2];
+    uint8_t  exact;              /* bit-exact abundances: every feature's --multi=equal shares and PropSharing increments
+                                    are added in the input order of their inserts, with the reference's IEEE operations,
+                                    instead of by f64 atomics.  Abundances, EM deltas, iterations and purged count are then
+                                    bit-identical to the reference's (for any chunking and push kind; with collate, to the
+                                    reference on the grouped order).  Effect only with share_type MSG_MULTI_EQUAL or
+                                    MSG_MULTI_PROPORTIONAL.  Needs n_ranks == 1 (msg_create returns MSG_EINVAL otherwise);
+                                    works with collate.  Costs a transposition of the lists per finish after pushes
+                                    and a serial sum per feature in each iteration (DESIGN.md §9).                      */
+    uint8_t  reserved0[1];
     int32_t  min_length;         /* -l  (MIN_LENGTH, msam_filter.c:449-457)            */
     int32_t  ppt;                /* 10*-p or --ppt (PPT, msam_filter.c:420-437)        */
     int32_t  max_clip;           /* 100 - z; 100 when -z absent (MAX_CLIP, :439-447)   */

@@ -21,7 +21,7 @@ class MsgConfig(C.Structure):
     _fields_ = [
         ("abi_version", C.c_uint32),
         ("do_filter", C.c_uint8), ("hit_mode", C.c_uint8), ("invert", C.c_uint8), ("keep_unmapped", C.c_uint8),
-        ("rescore", C.c_uint8), ("collate", C.c_uint8), ("reserved0", C.c_uint8 * 2),
+        ("rescore", C.c_uint8), ("collate", C.c_uint8), ("exact", C.c_uint8), ("reserved0", C.c_uint8 * 1),
         ("min_length", C.c_int32), ("ppt", C.c_int32), ("max_clip", C.c_int32),
         ("want_kept", C.c_uint8), ("want_records", C.c_uint8), ("want_profile", C.c_uint8), ("want_coverage", C.c_uint8),
         ("want_stats", C.c_uint8), ("share_type", C.c_uint8), ("debug_force_slow", C.c_uint8), ("coverage_summary", C.c_uint8),

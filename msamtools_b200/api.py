@@ -38,7 +38,7 @@ class Context:
                  besthit=False, uniqhit=False, do_filter=None,
                  profile=False, multi="proportional", coverage=False, coverage_summary=False, records=False, stats=False, kept=True,
                  n_targets=0, n_features=None, fmap=None, target_len=None,
-                 device=0, n_ranks=1, rank=0, nccl_unique_id=None, force_slow=False, collate=False):
+                 device=0, n_ranks=1, rank=0, nccl_unique_id=None, force_slow=False, collate=False, exact=False):
         self.lib = L.load()
         cfg = L.MsgConfig()
         cfg.abi_version = L.MSG_ABI_VERSION
@@ -51,6 +51,7 @@ class Context:
         cfg.hit_mode = L.HIT_UNIQUE if uniqhit else (L.HIT_BEST if besthit else L.HIT_NONE)
         cfg.invert, cfg.keep_unmapped, cfg.rescore = int(invert), int(keep_unmapped), int(rescore)
         cfg.collate = int(collate)                 # records in any order: grouped by QNAME on the device at finish
+        cfg.exact = int(exact)                     # equal / proportional abundances bit-identical to the reference
         cfg.min_length, cfg.ppt, cfg.max_clip = int(l), int(PPT), int(max_clip)
         cfg.want_kept, cfg.want_records, cfg.want_profile = int(kept), int(records), int(profile)
         cfg.want_coverage, cfg.want_stats = int(coverage), int(stats)

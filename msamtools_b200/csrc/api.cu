@@ -95,6 +95,7 @@ struct Slot {
     const uint8_t *d_raw = nullptr, *h_raw = nullptr; const uint64_t *d_off = nullptr, *h_off = nullptr;
     uint64_t nbytes = 0, readable = 0, n = 0; bool zero_copy = false;
     uint64_t ub_lists = 0, ub_ent = 0;        // list space reserved for it (worst case) until its real counts are known
+    uint64_t key_base = 0;                    // records pushed before it (exact mode: the input order of its lists)
 };
 
 struct msg_ctx {
@@ -136,6 +137,10 @@ struct msg_ctx {
     // profile accumulators
     uint32_t *d_ui = nullptr; double *d_d = nullptr; uint32_t *d_counters = nullptr;   // counters[8]
     DevBuf csr_off, csr_len, csr_fid; uint64_t csr_lists = 0, csr_ent = 0;     // multi-mapper lists (CSR), appended per chunk
+    // exact mode (cfg.exact): the input key of every list, and the per-feature incidence in key order (built at finish)
+    DevBuf csr_key, ex_beg, ex_cur, ex_keys, ex_big, ex_list, ex_sums;
+    uint64_t rec_base = 0, cur_key_base = 0;   // records pushed since the reset / before the chunk being profiled
+    bool ex_ready = false;                     // the incidence (and, equal mode, d) match the lists
     DevBuf t_ui, t_d, t_cnt, t_cov;                                    // allreduce staging (n_ranks > 1)
     uint32_t *d_stamp = nullptr; uint32_t stamp_next = 0;
     double *d_U = nullptr, *d_a = nullptr, *d_inc = nullptr, *d_partial = nullptr, *d_delta = nullptr;
@@ -261,8 +266,10 @@ int profile_stage(msg_ctx *c, const uint32_t *stream, uint64_t m)
     int rc = run_scan<uint32_t>(c, InFlagBit{c->fb.as<uint32_t>(), FB_EQPREV, 0u}, OutInclU32{c->nid.as<uint32_t>()}, n, (uint32_t *)nullptr);
     if (rc) return rc;
 
-    const bool prop = g.share_type == MSG_MULTI_PROPORTIONAL;
-    if (prop) CU(c->pcount.reserve(m * 4));
+    // exact mode also writes lists for the inserts that add 1/n to d (MSG_MULTI_EQUAL); d is then summed at finish
+    const bool ex = g.exact != 0;
+    const bool lists = g.share_type == MSG_MULTI_PROPORTIONAL || (ex && g.share_type == MSG_MULTI_EQUAL);
+    if (lists) CU(c->pcount.reserve(m * 4));
     const uint32_t big_cap = 65536;
     CU(c->biglist.reserve((size_t)big_cap * 4));
     ProfParams p;
@@ -270,22 +277,24 @@ int profile_stage(msg_ctx *c, const uint32_t *stream, uint64_t m)
     p.tid = c->tid.as<int32_t>(); p.nid = c->nid.as<uint32_t>(); p.hash = c->hash.as<uint32_t>();
     p.fmap = c->d_fmap; p.n_targets = g.n_targets; p.n_features = g.n_features; p.share_type = g.share_type;
     p.ui = c->d_ui; p.d = c->d_d; p.counters = c->d_counters;
-    p.pcount = prop ? c->pcount.as<uint32_t>() : nullptr;
+    p.pcount = lists ? c->pcount.as<uint32_t>() : nullptr;
     p.big = c->biglist.as<uint32_t>(); p.big_cap = big_cap; p.big_threshold = 1024; p.err = c->d_err;
+    p.key = nullptr; p.key_base = c->cur_key_base;
     CU(c->worklist.reserve((std::max<uint64_t>(n, m) / 32 + 2) * 4));
-    if (prop) CU(c->gmeta.reserve(m));
+    if (lists) CU(c->gmeta.reserve(m));
     CU(cudaMemsetAsync(c->d_wl + 1, 0, 4, c->stream));
-    uint8_t *gmeta = prop ? c->gmeta.as<uint8_t>() : nullptr;
+    uint8_t *gmeta = lists ? c->gmeta.as<uint8_t>() : nullptr;
     const uint32_t pgrid = std::min<uint32_t>(nblocks(m / 32 + 1, 256), 148u * 4u);
-    if ((uint32_t)g.n_features <= 4096u)
-        profile_warp_count_kernel<true><<<nblocks(m, 256), 256, (size_t)g.n_features * 4, c->stream>>>(p, gmeta, c->worklist.as<uint32_t>(), c->d_wl + 1);
-    else
-        profile_warp_count_kernel<false><<<nblocks(m, 256), 256, 0, c->stream>>>(p, gmeta, c->worklist.as<uint32_t>(), c->d_wl + 1);
-    LAUNCHED(c);
-    profile_walk_count_kernel<<<pgrid, 256, 0, c->stream>>>(p, c->worklist.as<uint32_t>(), c->d_wl + 1); LAUNCHED(c);
+    const bool sh = (uint32_t)g.n_features <= 4096u;
+    auto warp_count = sh ? (ex ? profile_warp_count_kernel<true, true> : profile_warp_count_kernel<true, false>)
+                         : (ex ? profile_warp_count_kernel<false, true> : profile_warp_count_kernel<false, false>);
+    warp_count<<<nblocks(m, 256), 256, sh ? (size_t)g.n_features * 4 : 0, c->stream>>>(p, gmeta, c->worklist.as<uint32_t>(), c->d_wl + 1); LAUNCHED(c);
+    auto walk_count = ex ? profile_walk_count_kernel<true> : profile_walk_count_kernel<false>;
+    walk_count<<<pgrid, 256, 0, c->stream>>>(p, c->worklist.as<uint32_t>(), c->d_wl + 1); LAUNCHED(c);
+    auto big_kernel = ex ? profile_big_kernel<true> : profile_big_kernel<false>;
 
     uint32_t nbig = 0;
-    if (prop) {
+    if (lists) {
         CU(c->scanv.reserve(m * 8));
         unsigned long long tot = 0;
         rc = run_scan<unsigned long long>(c, InPcountPacked{p.pcount}, OutExclU64{c->scanv.as<unsigned long long>()}, m, &tot);
@@ -296,9 +305,10 @@ int profile_stage(msg_ctx *c, const uint32_t *stream, uint64_t m)
             CU(c->csr_off.reserve_keep((c->csr_lists + nl + 1) * 4, c->csr_lists * 4, c->stream));
             CU(c->csr_len.reserve_keep((c->csr_lists + nl + 1) * 4, c->csr_lists * 4, c->stream));
             CU(c->csr_fid.reserve_keep((c->csr_ent + ne + 1) * 4, c->csr_ent * 4, c->stream));
-            profile_warp_fill_kernel<<<nblocks(m, 256), 256, 0, c->stream>>>(p, gmeta, c->scanv.as<unsigned long long>(), c->csr_off.as<uint32_t>(),
+            if (ex) { CU(c->csr_key.reserve_keep((c->csr_lists + nl + 1) * 8, c->csr_lists * 8, c->stream)); p.key = c->csr_key.as<unsigned long long>(); }
+            (ex ? profile_warp_fill_kernel<true> : profile_warp_fill_kernel<false>)<<<nblocks(m, 256), 256, 0, c->stream>>>(p, gmeta, c->scanv.as<unsigned long long>(), c->csr_off.as<uint32_t>(),
                                                                              c->csr_len.as<uint32_t>(), c->csr_fid.as<int32_t>(), (uint32_t)c->csr_lists, (uint32_t)c->csr_ent); LAUNCHED(c);
-            profile_walk_fill_kernel<<<pgrid, 256, 0, c->stream>>>(p, c->scanv.as<unsigned long long>(), c->csr_off.as<uint32_t>(), c->csr_len.as<uint32_t>(),
+            (ex ? profile_walk_fill_kernel<true> : profile_walk_fill_kernel<false>)<<<pgrid, 256, 0, c->stream>>>(p, c->scanv.as<unsigned long long>(), c->csr_off.as<uint32_t>(), c->csr_len.as<uint32_t>(),
                                                                    c->csr_fid.as<int32_t>(), (uint32_t)c->csr_lists, (uint32_t)c->csr_ent, c->worklist.as<uint32_t>(), c->d_wl + 1); LAUNCHED(c);
             c->csr_lists += nl; c->csr_ent += ne;
         }
@@ -311,9 +321,9 @@ int profile_stage(msg_ctx *c, const uint32_t *stream, uint64_t m)
         if (!c->d_stamp) { CU(cudaMalloc(&c->d_stamp, (size_t)(g.n_features > 0 ? g.n_features : 1) * 4));
                            CU(cudaMemsetAsync(c->d_stamp, 0, (size_t)(g.n_features > 0 ? g.n_features : 1) * 4, c->stream)); }
         uint32_t *d_tot = reinterpret_cast<uint32_t *>(c->d_total);
-        profile_big_kernel<<<1, 1, 0, c->stream>>>(p, nbig, c->d_stamp, c->stamp_next, nullptr, nullptr, nullptr, d_tot, 0, 0, 0); LAUNCHED(c);
+        big_kernel<<<1, 1, 0, c->stream>>>(p, nbig, c->d_stamp, c->stamp_next, nullptr, nullptr, nullptr, d_tot, 0, 0, 0); LAUNCHED(c);
         c->stamp_next += nbig + 1;
-        if (prop) {
+        if (lists) {
             uint32_t tot[2];
             CU(cudaMemcpyAsync(tot, d_tot, 8, cudaMemcpyDeviceToHost, c->stream));
             CU(cudaStreamSynchronize(c->stream));
@@ -322,7 +332,8 @@ int profile_stage(msg_ctx *c, const uint32_t *stream, uint64_t m)
                 CU(c->csr_off.reserve_keep((c->csr_lists + tot[0] + 1) * 4, c->csr_lists * 4, c->stream));
                 CU(c->csr_len.reserve_keep((c->csr_lists + tot[0] + 1) * 4, c->csr_lists * 4, c->stream));
                 CU(c->csr_fid.reserve_keep((c->csr_ent + tot[1] + 2) * 4, c->csr_ent * 4, c->stream));
-                profile_big_kernel<<<1, 1, 0, c->stream>>>(p, nbig, c->d_stamp, c->stamp_next, c->csr_off.as<uint32_t>(), c->csr_len.as<uint32_t>(), c->csr_fid.as<int32_t>(),
+                if (ex) { CU(c->csr_key.reserve_keep((c->csr_lists + tot[0] + 1) * 8, c->csr_lists * 8, c->stream)); p.key = c->csr_key.as<unsigned long long>(); }
+                big_kernel<<<1, 1, 0, c->stream>>>(p, nbig, c->d_stamp, c->stamp_next, c->csr_off.as<uint32_t>(), c->csr_len.as<uint32_t>(), c->csr_fid.as<int32_t>(),
                                                            d_tot, 1, (uint32_t)c->csr_lists, (uint32_t)c->csr_ent); LAUNCHED(c);
                 c->stamp_next += nbig + 1;
                 c->csr_lists += tot[0]; c->csr_ent += tot[1];
@@ -363,12 +374,13 @@ int fused_enqueue(msg_ctx *c, const DecodeParams &dp, uint64_t n, Slot &sl, bool
 {
     const msg_config &g = c->cfg;
     *queued = false;
-    const bool prop = g.share_type == MSG_MULTI_PROPORTIONAL;
+    const bool ex = g.exact != 0;
+    const bool lists = g.share_type == MSG_MULTI_PROPORTIONAL || (ex && g.share_type == MSG_MULTI_EQUAL);
     const uint32_t nwin = nblocks(n, 32);
     CU(c->worklist.reserve(((size_t)nwin + 2) * 4));
     CU(c->win.reserve((size_t)nwin * sizeof(WinInfo)));
     sl.ub_lists = sl.ub_ent = 0;
-    if (prop) {
+    if (lists) {
         const uint64_t ul = n / 2 + 2, ue = n + 2;
         if (c->csr_lists + c->inflight_lists + ul >= 0xffffffffull || c->csr_ent + c->inflight_ent + ue >= 0xffffffffull) return MSG_OK;   // general path reports the overflow
         if ((c->csr_lists + c->inflight_lists + ul) * 4 > c->csr_off.cap || (c->csr_ent + c->inflight_ent + ue) * 4 > c->csr_fid.cap || !c->csr_off.p) {
@@ -377,6 +389,10 @@ int fused_enqueue(msg_ctx *c, const DecodeParams &dp, uint64_t n, Slot &sl, bool
             CU(c->csr_off.reserve_keep((c->csr_lists + ul) * 4, c->csr_lists * 4, c->stream));
             CU(c->csr_len.reserve_keep((c->csr_lists + ul) * 4, c->csr_lists * 4, c->stream));
             CU(c->csr_fid.reserve_keep((c->csr_ent + ue) * 4, c->csr_ent * 4, c->stream));
+        }
+        if (ex && (c->csr_lists + c->inflight_lists + ul) * 8 > c->csr_key.cap) {
+            int rc = wait_all(c); if (rc) return rc;
+            CU(c->csr_key.reserve_keep((c->csr_lists + ul) * 8, c->csr_lists * 8, c->stream));
         }
         sl.ub_lists = ul; sl.ub_ent = ue;
     }
@@ -397,10 +413,11 @@ int fused_enqueue(msg_ctx *c, const DecodeParams &dp, uint64_t n, Slot &sl, bool
     p.l_start = c->csr_off.as<uint32_t>(); p.l_len = c->csr_len.as<uint32_t>(); p.l_fid = c->csr_fid.as<int32_t>();
     p.worklist = c->worklist.as<uint32_t>(); p.wl_count = c->d_wl; p.win = c->win.as<WinInfo>();
     p.big_threshold = 1024; p.err = c->d_err;
-    if ((uint32_t)g.n_features <= 4096u) fused_warp_kernel<true><<<nblocks(n, 256), 256, (size_t)g.n_features * 4, c->stream>>>(p);
-    else                                  fused_warp_kernel<false><<<nblocks(n, 256), 256, 0, c->stream>>>(p);
-    LAUNCHED(c);
-    fused_walk_kernel<<<std::min<uint32_t>(nblocks(nwin, 128), 148u * 8u), 128, 0, c->stream>>>(p); LAUNCHED(c);
+    p.l_key = c->csr_key.as<unsigned long long>(); p.key_base = sl.key_base;
+    const bool sh = (uint32_t)g.n_features <= 4096u;
+    auto warp = sh ? (ex ? fused_warp_kernel<true, true> : fused_warp_kernel<true, false>) : (ex ? fused_warp_kernel<false, true> : fused_warp_kernel<false, false>);
+    warp<<<nblocks(n, 256), 256, sh ? (size_t)g.n_features * 4 : 0, c->stream>>>(p); LAUNCHED(c);
+    (ex ? fused_walk_kernel<true> : fused_walk_kernel<false>)<<<std::min<uint32_t>(nblocks(nwin, 128), 148u * 8u), 128, 0, c->stream>>>(p); LAUNCHED(c);
     fused_guard_kernel<<<nblocks(nwin, 256), 256, 0, c->stream>>>(p.win, nwin, c->d_fcnt + 3); LAUNCHED(c);
     const size_t F = (size_t)(g.n_features > 0 ? g.n_features : 1);
     fused_commit_kernel<<<nblocks(F < 3 ? 3 : F, 256), 256, 0, c->stream>>>(c->d_ui, c->d_d, c->d_ui_tmp, c->d_d_tmp, (uint32_t)g.n_features,
@@ -622,6 +639,7 @@ int complete_slot(msg_ctx *c, int s)
         c->h2d_bytes += sl.nbytes;
         d_raw = sl.raw.as<uint8_t>(); readable = sl.nbytes + 64;
     }
+    c->cur_key_base = sl.key_base;                   // the rerun's lists take the declined chunk's keys
     return run_chunk_general(c, d_raw, sl.nbytes, readable, sl.d_off, sl.n, sl.h_raw, sl.h_off);
 }
 
@@ -646,6 +664,8 @@ int push_chunk(msg_ctx *c, const uint8_t *h_raw, const uint8_t *dev_raw, size_t 
     if (rc) return rc;
     Slot &sl = c->slot[fused ? s : 0];
     sl.h_raw = h_raw; sl.h_off = h_off; sl.nbytes = nbytes; sl.n = nrec; sl.zero_copy = false;
+    sl.key_base = c->rec_base; c->rec_base += nrec;     // chunks complete in push order, so this is their input position
+    c->ex_ready = false;
 
     cudaEvent_t t0 = get_event(c), t1 = get_event(c);
     if (dev_raw) {
@@ -711,6 +731,7 @@ int push_chunk(msg_ctx *c, const uint8_t *h_raw, const uint8_t *dev_raw, size_t 
         c->h2d_bytes += nbytes;
         d_raw = sl.raw.as<uint8_t>(); readable = nbytes + 64;
     }
+    c->cur_key_base = sl.key_base;
     return run_chunk_general(c, d_raw, nbytes, readable, sl.d_off, nrec, h_raw, h_off);
 }
 
@@ -916,6 +937,68 @@ int collate_run(msg_ctx *c)
     return MSG_OK;
 }
 
+// Exact mode: the lists that hold each feature, sorted by their input key (profile.cuh, exact mode), built once per
+// finish after pushes -- entries per feature, run_scan, scatter of {key, list}, collate.cuh's bucket sorts (shared memory
+// up to COLL_SMEM_KEYS entries, global memory above) -- and, with MSG_MULTI_EQUAL, d[] summed from them in that order.
+int exact_prepare(msg_ctx *c)
+{
+    const msg_config &g = c->cfg;
+    if (!g.exact || c->ex_ready) return MSG_OK;
+    const bool prop = g.share_type == MSG_MULTI_PROPORTIONAL, eq = g.share_type == MSG_MULTI_EQUAL;
+    if (!prop && !eq) { c->ex_ready = true; return MSG_OK; }
+    const uint32_t F = (uint32_t)g.n_features, nl = (uint32_t)c->csr_lists;
+    const uint64_t ne = c->csr_ent;
+    if (F == 0) { c->ex_ready = true; return MSG_OK; }
+    CU(c->ex_beg.reserve((size_t)F * 4)); CU(c->ex_cur.reserve((size_t)F * 4)); CU(c->ex_big.reserve((size_t)F * 4 + 8));
+    CU(c->ex_keys.reserve((ne + 1) * sizeof(CollKey))); CU(c->ex_list.reserve((ne + 1) * 4));
+    if (prop) CU(c->ex_sums.reserve(((size_t)nl + 1) * 8));
+    uint32_t *beg = c->ex_beg.as<uint32_t>(), *cur = c->ex_cur.as<uint32_t>();
+    const uint32_t *off = c->csr_off.as<uint32_t>(), *len = c->csr_len.as<uint32_t>(); const int32_t *fid = c->csr_fid.as<int32_t>();
+    CollKey *keys = c->ex_keys.as<CollKey>();
+    static const bool trace = getenv("MSG_TRACE_FINISH") != nullptr;
+    cudaEvent_t tev[2] = {nullptr, nullptr};
+    if (trace) for (auto &e : tev) cudaEventCreate(&e);
+    if (trace) cudaEventRecord(tev[0], c->stream);
+    const uint32_t lgrid = std::max<uint32_t>(1u, std::min<uint32_t>(nblocks(nl, 256), 148u * 8u));
+    CU(cudaMemsetAsync(cur, 0, (size_t)F * 4, c->stream));
+    if (nl) { exact_hist_kernel<<<lgrid, 256, 0, c->stream>>>(off, len, fid, nl, cur); LAUNCHED(c); }
+    int rc = run_scan<uint32_t>(c, InU32{cur}, OutExclU32{beg}, F, (uint32_t *)nullptr);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(cur, beg, (size_t)F * 4, cudaMemcpyDeviceToDevice, c->stream));
+    if (nl) {
+        exact_scatter_kernel<<<lgrid, 256, 0, c->stream>>>(off, len, fid, nl, c->csr_key.as<unsigned long long>(), cur, keys); LAUNCHED(c);
+        uint32_t *big = c->ex_big.as<uint32_t>(), *cnt = reinterpret_cast<uint32_t *>(c->d_total);
+        CU(cudaMemsetAsync(cnt, 0, 4, c->stream));
+        collate_bucket_sort_kernel<<<std::min<uint32_t>(F, 148u * 8u), 256, 0, c->stream>>>(keys, beg, F, ne, big, cnt); LAUNCHED(c);
+        uint32_t *h_cnt = c->h_pin + 88;
+        CU(cudaMemcpyAsync(h_cnt, cnt, 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        if (*h_cnt) { collate_sort_global_kernel<<<*h_cnt, 1024, 0, c->stream>>>(keys, beg, F, ne, big, false, nullptr, nullptr); LAUNCHED(c); }
+        exact_lists_kernel<<<std::max<uint32_t>(1u, std::min<uint32_t>(nblocks(ne, 256), 148u * 8u)), 256, 0, c->stream>>>(keys, ne, c->ex_list.as<uint32_t>()); LAUNCHED(c);
+    }
+    if (eq) { em_exact_equal_kernel<<<std::min<uint32_t>(nblocks(F, 256), 148u * 8u), 256, 0, c->stream>>>(beg, c->ex_list.as<uint32_t>(), ne, len, c->d_d, F); LAUNCHED(c); }
+    if (trace) {                           // MSG_TRACE_FINISH: the one-off cost and the longest serial chain of the gather
+        cudaEventRecord(tev[1], c->stream); cudaEventSynchronize(tev[1]);
+        float ms = 0; cudaEventElapsedTime(&ms, tev[0], tev[1]);
+        std::vector<uint32_t> hb(F);
+        cudaMemcpy(hb.data(), beg, (size_t)F * 4, cudaMemcpyDeviceToHost);
+        uint64_t longest = 0;
+        for (uint32_t f = 0; f < F; f++) longest = std::max<uint64_t>(longest, (f + 1 < F ? hb[f + 1] : ne) - hb[f]);
+        fprintf(stderr, "[msg exact] %u lists, %llu entries, longest incidence %llu: transposition%s %.3f ms\n", nl, (unsigned long long)ne,
+                (unsigned long long)longest, eq ? " + equal shares" : "", ms);
+        for (auto e : tev) cudaEventDestroy(e);
+    }
+    c->ex_ready = true;
+    return MSG_OK;
+}
+
+// MSG_EXACT_DELTA=seq (tests): take the sequential delta of the exact loop in every iteration, not only near 1e-10
+bool exact_force_seq()
+{
+    static const bool on = getenv("MSG_EXACT_DELTA") && strcmp(getenv("MSG_EXACT_DELTA"), "seq") == 0;
+    return on;
+}
+
 int allreduce(msg_ctx *c, void *buf, size_t count, ncclDataType_t dt, ncclRedOp_t op)
 {
     if (c->cfg.n_ranks <= 1) return MSG_OK;
@@ -961,6 +1044,8 @@ int msg_create(const msg_config *cfg, msg_ctx **out)
     if (cfg->want_coverage && !cfg->target_len) return fail(c, MSG_EINVAL, "want_coverage requires target_len");
     if (cfg->do_filter && cfg->invert && cfg->hit_mode) return fail(c, MSG_EINVAL, "--invert cannot be combined with --besthit or --uniqhit");
     if (cfg->hit_mode > MSG_HIT_UNIQUE) return fail(c, MSG_EINVAL, "bad hit_mode");
+    if (cfg->exact && cfg->n_ranks > 1)
+        return fail(c, MSG_EINVAL, "exact needs n_ranks == 1: bit-exact sums across GPUs would chain every rank's partial sums after the previous rank's");
     if (cfg->collate) {
         if (!cfg->want_profile && !cfg->want_coverage) return fail(c, MSG_EINVAL, "collate needs want_profile and/or want_coverage");
         if (cfg->want_records || cfg->want_kept || cfg->want_stats)
@@ -1129,7 +1214,7 @@ void msg_destroy(msg_ctx *c)
     if (c->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(c->comm);
     DevBuf *bufs[] = {&c->tid, &c->fb, &c->score, &c->hash, &c->nid, &c->st_alen, &c->st_qlen, &c->st_qclip, &c->st_edit,
                       &c->kbase, &c->worklist, &c->gmeta, &c->out_idx, &c->tile_sums, &c->pcount, &c->scanv, &c->biglist, &c->out_len, &c->out_off, &c->plan, &c->out_rec,
-                      &c->csr_off, &c->csr_len, &c->csr_fid, &c->win, &c->t_ui, &c->t_d, &c->t_cnt, &c->t_cov};
+                      &c->csr_off, &c->csr_len, &c->csr_fid, &c->csr_key, &c->ex_beg, &c->ex_cur, &c->ex_keys, &c->ex_big, &c->ex_list, &c->ex_sums, &c->win, &c->t_ui, &c->t_d, &c->t_cnt, &c->t_cov};
     for (DevBuf *b : bufs) b->release();
     void *ptrs[] = {c->d_fmap, c->d_tlen, c->d_covbase, c->d_err, c->d_acct, c->d_total, c->d_ui, c->d_d, c->d_counters, c->d_stamp, c->d_U, c->d_a,
                     c->d_inc, c->d_partial, c->d_delta, c->d_purged, c->d_bflag, c->d_wl, c->d_ui_tmp, c->d_d_tmp, c->d_fcnt, c->d_cursor, c->d_diff, c->d_depth, c->d_covered, c->d_touched, c->d_sum, c->d_covbits};
@@ -1160,6 +1245,7 @@ int msg_reset(msg_ctx *c)
         CU(cudaMemsetAsync(c->d_counters, 0, 32, c->stream));
         c->csr_lists = c->csr_ent = 0;
     }
+    c->rec_base = 0; c->ex_ready = false;
     if (g.want_coverage) {
         if (c->cov_bits) {
             CU(cudaMemsetAsync(c->d_covbits, 0, (size_t)(c->cov_words ? c->cov_words : 1) * 8, c->stream));
@@ -1333,6 +1419,7 @@ int msg_pull_counts(msg_ctx *c, uint32_t *ui, double *d)
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
     { int crc = collate_run(c); if (crc) return crc; }
+    { int erc = exact_prepare(c); if (erc) return erc; }
     const size_t F = (size_t)c->cfg.n_features;
     if (ui && F) CU(cudaMemcpyAsync(ui, c->d_ui, F * 4, cudaMemcpyDeviceToHost, c->stream));
     if (d && F)  CU(cudaMemcpyAsync(d, c->d_d, F * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -1387,7 +1474,7 @@ static int em_coop_loop(msg_ctx *c, uint32_t *hc, int32_t *res, double *h_delta,
     const uint32_t F = (uint32_t)g.n_features;
     const bool multi = g.n_ranks > 1, sm = F <= EM_SMEM_F;
     const bool rsag = multi && F + 8 > EM_XCHG_CTA0;               // gene catalogues: reduce-scatter / all-gather exchange
-    const size_t shm = em_smem_bytes(F);
+    const size_t shm = g.exact ? 0 : em_smem_bytes(F);
     int rc;
     // the argument arrays below hold the addresses of these; partial is set once the grid size is known
     const uint32_t *a0 = c->csr_off.as<uint32_t>(), *a1 = c->csr_len.as<uint32_t>(); const int32_t *a2 = c->csr_fid.as<int32_t>();
@@ -1413,8 +1500,16 @@ static int em_coop_loop(msg_ctx *c, uint32_t *hc, int32_t *res, double *h_delta,
                      &totbuf, &bflag, &pt, &nr, &rk, &epoch, &timeout_ns};
     void *rargs[] = {&a0, &a1, &a2, &nl_arg, &ui_arg, &cnt_arg, &nl_lo, &nl_hi, &U, &av, &inc, &F_arg, &dout, &d_res, &hc_dev,
                      &pt, &nr, &rk, &epoch, &timeout_ns, &d_trace};
+    // exact (one GPU): incidence from exact_prepare; list sums in ex_sums, the squared differences in the second third of inc
+    const uint32_t *ibeg = c->ex_beg.as<uint32_t>(), *ilist = c->ex_list.as<uint32_t>();
+    unsigned long long nent = c->csr_ent;
+    double *sums = c->ex_sums.as<double>(), *sq = c->d_inc + F;
+    int force_seq = exact_force_seq();
+    void *xargs[] = {&a0, &a1, &a2, &nl_arg, &ibeg, &ilist, &nent, &U, &av, &sums, &sq, &partial, &F_arg, &dout, &d_res, &force_seq};
+    const bool exact = g.exact != 0;
     const void *fn; void **args;
-    if (rsag)       { fn = (const void *)em_loop_rsag_kernel; args = rargs; }
+    if (exact)      { fn = (const void *)em_loop_exact_kernel; args = xargs; }
+    else if (rsag)  { fn = (const void *)em_loop_rsag_kernel; args = rargs; }
     else if (multi) { fn = sm ? (const void *)em_loop_multi_kernel<true> : (const void *)em_loop_multi_kernel<false>; args = margs; }
     else if (sm)    { fn = (const void *)em_loop_smem_kernel; args = sargs; }
     else            { fn = (const void *)em_loop_kernel; args = largs; }
@@ -1425,10 +1520,10 @@ static int em_coop_loop(msg_ctx *c, uint32_t *hc, int32_t *res, double *h_delta,
         if (multi) return fail(c, MSG_ECUDA, "cannot launch the cooperative PropSharing kernel (F = %u needs too much shared memory?)", F);
         return MSG_OK;
     }
-    const int want_ctas = EM_CTAS_ENV > 0 ? EM_CTAS_ENV : (sm ? 3 : 4);
+    const int want_ctas = EM_CTAS_ENV > 0 ? EM_CTAS_ENV : (sm && !exact ? 3 : 4);
     if (per_sm > want_ctas) per_sm = want_ctas;
     const uint32_t grid = (uint32_t)(nsm * per_sm);
-    CU(c->tile_sums.reserve((size_t)grid * 8 + 16));
+    CU(c->tile_sums.reserve((size_t)grid * 8 + 16));                 // + the exact loop's sequential delta
     partial = c->tile_sums.as<double>();
     // one GPU: inc[3F], delta and d_res were cleared by em_init_kernel; the multi-GPU kernels clear their own state
     if (multi) {
@@ -1463,7 +1558,27 @@ static int em_host_loop(msg_ctx *c, msg_profile_stats &s, uint32_t *h_purged)
     const uint32_t em_grid = nl32 ? (nblocks(nl32, 256) < 148u * 8u ? nblocks(nl32, 256) : 148u * 8u) : 0;
     const uint32_t *off = c->csr_off.as<uint32_t>(), *len = c->csr_len.as<uint32_t>(); const int32_t *fid = c->csr_fid.as<int32_t>();
     int rc;
+    const bool exact = c->cfg.exact != 0;
     for (int k = 1; k < 20; k++) {                                                                      // msam_profile.c:331
+        if (exact) {
+            if (!F) { s.em_delta[k - 1] = nan(""); s.em_iterations = k; continue; }
+            if (nl32) { em_exact_sums_kernel<<<em_grid, 256, 0, c->stream>>>(off, len, fid, nl32, c->d_a, c->ex_sums.as<double>()); LAUNCHED(c); }
+            em_exact_gather_kernel<<<nb, 256, 0, c->stream>>>(c->ex_beg.as<uint32_t>(), c->ex_list.as<uint32_t>(), c->csr_ent, c->ex_sums.as<double>(),
+                                                              c->d_U, c->d_a, c->d_inc + F, c->d_partial, F); LAUNCHED(c);
+            em_delta_kernel<<<1, 256, 0, c->stream>>>(c->d_partial, nb, F, c->d_delta + (k - 1)); LAUNCHED(c);
+            double delta = 0;
+            CU(cudaMemcpyAsync(&delta, c->d_delta + (k - 1), 8, cudaMemcpyDeviceToHost, c->stream));
+            CU(cudaStreamSynchronize(c->stream));
+            if (exact_force_seq() || em_exact_near(delta, F)) {              // profile.cuh: the sum in order j = 0 .. F-1
+                em_exact_seq_kernel<<<1, 32, 0, c->stream>>>(c->d_inc + F, F, c->d_delta + (k - 1)); LAUNCHED(c);
+                CU(cudaMemcpyAsync(&delta, c->d_delta + (k - 1), 8, cudaMemcpyDeviceToHost, c->stream));
+                CU(cudaStreamSynchronize(c->stream));
+            }
+            c->d2h_bytes += 8;
+            s.em_delta[k - 1] = delta; s.em_iterations = k;
+            if (delta < 1e-10) { s.em_converged = 1; break; }
+            continue;
+        }
         CU(cudaMemsetAsync(c->d_inc, 0, (size_t)F * 8, c->stream));
         if (nl32) { em_gather_kernel<<<em_grid, 256, em_smem_bytes(F), c->stream>>>(off, len, fid, nl32, c->d_a, c->d_inc, F); LAUNCHED(c); }
         if ((rc = allreduce(c, c->d_inc, F, ncclFloat64, ncclSum))) return rc;
@@ -1519,6 +1634,7 @@ int msg_finish_profile(msg_ctx *c, double *abundance, msg_profile_stats *st)
     CU(cudaSetDevice(c->cfg.device));
     { int wrc = wait_all(c); if (wrc) return wrc; }
     { int crc = collate_run(c); if (crc) return crc; }
+    { int erc = exact_prepare(c); if (erc) return erc; }
     const msg_config &g = c->cfg;
     const uint32_t F = (uint32_t)g.n_features;
     msg_profile_stats s; memset(&s, 0, sizeof s);
@@ -1560,6 +1676,7 @@ int msg_finish_profile(msg_ctx *c, double *abundance, msg_profile_stats *st)
     s.mapped_inserts = hc[0]; s.uniq_mapper_count = hc[1]; s.multi_mapper_count = hc[2];
     s.multi_lists = g.n_ranks > 1 ? (unsigned long long)hc[4] + ((unsigned long long)hc[5] << 16) : c->csr_lists;
     s.multi_entries = c->csr_ent;
+    if (!em) s.multi_lists = s.multi_entries = 0;          // exact --multi=equal keeps lists of its own; they are not PropSharing's
     if (st) *st = s;
     return report_device_errors(c, c->h_pin + 8);
 }

@@ -862,6 +862,8 @@ static int profile_main(int argc, char *argv[])
 
     r.cfg.do_filter = 0; r.cfg.want_profile = 1; r.cfg.share_type = (uint8_t)share_type;
     r.cfg.collate = a_collate->count > 0;
+    /* MSAMTOOLS_EXACT=1: abundances bit-identical to the reference (--multi=equal / proportional; msg_config.exact) */
+    r.cfg.exact = getenv("MSAMTOOLS_EXACT") && atoi(getenv("MSAMTOOLS_EXACT")) != 0;
     r.cfg.n_targets = n_targets; r.cfg.n_features = n_features; r.cfg.fmap = fmap;
     phase(sub, "pre-flight + feature map");
     msg_ctx *ctx = run_stream(&r);

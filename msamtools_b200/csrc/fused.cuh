@@ -36,11 +36,17 @@ struct FusedParams {
     WinInfo *win;                     // [ceil(n/32)]
     uint32_t big_threshold;
     uint32_t *err;
+    unsigned long long *l_key;        // exact mode: [list] key_base + position of the list's group in the chunk (input order)
+    unsigned long long key_base;      // records pushed before this chunk
 };
+
+// Whether the chunk writes multi-mapper lists: PropSharing always; with EXACT (msg_config.exact) also --multi=equal, whose
+// 1/n shares are then summed at finish in input order instead of by atomics.
+template <bool EXACT> __device__ __forceinline__ bool fused_lists(const FusedParams &p) { return p.share_type == 3 || (EXACT && p.share_type == 2); }
 
 __device__ __forceinline__ int32_t fused_feature(const FusedParams &p, int32_t t) { return p.fmap ? p.fmap[t] : t; }
 
-template <bool SMEM_HIST>
+template <bool SMEM_HIST, bool EXACT>
 __global__ void __launch_bounds__(256) fused_warp_kernel(const FusedParams p)
 {
     extern __shared__ uint32_t s_hist[];
@@ -97,12 +103,13 @@ __global__ void __launch_bounds__(256) fused_warp_kernel(const FusedParams p)
             if (!multi) { if (ghead) atomicAdd(ui + feat, 2u); }
             else if (first && p.share_type != 3) {
                 if (p.share_type == 1) atomicAdd(ui + feat, 2u);
-                else if (p.share_type == 2) { if (size == 2) atomicAdd(ui + feat, 1u); else atomicAdd(p.d + feat, 1.0 / (int)nd); }
+                else if (p.share_type == 2) { if (size == 2) atomicAdd(ui + feat, 1u); else if (!EXACT) atomicAdd(p.d + feat, 1.0 / (int)nd); }
             }
         }
         // proportional: list space for this warp's multi-feature groups = (lists, entries); offsets inside the warp by ballot / scan
-        if (p.share_type == 3) {
-            const bool lhead = ghead && multi;
+        if (fused_lists<EXACT>(p)) {
+            const bool glist = multi && (p.share_type == 3 || size != 2);          // equal: the two-record case adds to ui
+            const bool lhead = ghead && glist;
             const uint32_t lmask = __ballot_sync(0xffffffffu, lhead);
             uint32_t x = lhead ? nd : 0u, incl = x;                                   // inclusive scan of list lengths over lanes
 #pragma unroll
@@ -112,7 +119,7 @@ __global__ void __launch_bounds__(256) fused_warp_kernel(const FusedParams p)
             is_lhead = lhead; my_nd = nd; my_feat = feat;
             const uint32_t gl = gmask ? (uint32_t)__ffs((int)gmask) - 1u : 0u;
             e_off_group = __shfl_sync(0xffffffffu, e_off, (int)gl);                    // entry offset of my group's list (within the warp)
-            if (first && multi) {
+            if (first && glist) {
                 const uint32_t below = (1u << lane) - 1u;
                 const uint32_t f1 = firsts & r1mask, f2 = firsts & ~r1mask;
                 f_rank = r2 ? __popc(f1) + __popc(f2 & below) : __popc(f1 & below);
@@ -144,7 +151,7 @@ __global__ void __launch_bounds__(256) fused_warp_kernel(const FusedParams p)
     }
     // ---- proportional: ONE pair of global atomics per CTA reserves list slots and entries for all of its warps
     __shared__ uint32_t s_wl[8], s_we[8], s_base[2];
-    if (p.share_type == 3) {
+    if (fused_lists<EXACT>(p)) {
         const uint32_t wid = threadIdx.x >> 5;
         if (lane == 0) { s_wl[wid] = w_lists; s_we[wid] = w_ents; }
         __syncthreads();
@@ -156,7 +163,7 @@ __global__ void __launch_bounds__(256) fused_warp_kernel(const FusedParams p)
         }
         __syncthreads();
         const uint32_t lbase = s_base[0] + s_wl[wid], ebase = s_base[1] + s_we[wid];
-        if (is_lhead) { p.l_start[lbase + l_rank] = ebase + e_off; p.l_len[lbase + l_rank] = my_nd; }
+        if (is_lhead) { p.l_start[lbase + l_rank] = ebase + e_off; p.l_len[lbase + l_rank] = my_nd; if (EXACT) p.l_key[lbase + l_rank] = p.key_base + i; }
         if (writes_fid) p.l_fid[ebase + e_off_group + f_rank] = my_feat;
     }
     __syncthreads();
@@ -172,6 +179,7 @@ constexpr int FUSED_MAXM = 48;    // distinct features per walked pool (more: th
 constexpr int FUSED_PF = 8;       // records whose columns are prefetched per walked pool
 constexpr int FUSED_DR = 8;       // distinct features kept in registers
 
+template <bool EXACT>
 __global__ void __launch_bounds__(128) fused_walk_kernel(const FusedParams p)
 {
     const uint32_t nw = *p.wl_count;
@@ -276,12 +284,12 @@ __global__ void __launch_bounds__(128) fused_walk_kernel(const FusedParams p)
             if (p.share_type == 1) { for (uint32_t k = 0; k < nd; k++) atomicAdd(p.ui + feat_at(k), 2u); }
             else if (p.share_type == 2) {
                 if (nm == 2) { atomicAdd(p.ui + dr[0], 1u); atomicAdd(p.ui + dr[1], 1u); }
-                else { const double share = 1.0 / (int)nd; for (uint32_t k = 0; k < nd; k++) atomicAdd(p.d + feat_at(k), share); }
+                else if (!EXACT) { const double share = 1.0 / (int)nd; for (uint32_t k = 0; k < nd; k++) atomicAdd(p.d + feat_at(k), share); }
             }
         }
       }
-      if (p.share_type == 3) {            // one pair of atomics per warp reserves the list slots / entries of its multi-feature groups
-        const bool lhead = emit && nd > 1;
+      if (fused_lists<EXACT>(p)) {        // one pair of atomics per warp reserves the list slots / entries of its multi-feature groups
+        const bool lhead = emit && nd > 1 && (p.share_type == 3 || nm != 2);
         const uint32_t lmask = __ballot_sync(0xffffffffu, lhead);
         uint32_t x = lhead ? nd : 0u, incl = x;
 #pragma unroll
@@ -293,6 +301,7 @@ __global__ void __launch_bounds__(128) fused_walk_kernel(const FusedParams p)
         if (lhead) {
             const uint32_t li = lb + (uint32_t)__popc(lmask & ((1u << lane) - 1u)), base = eb + incl - x;
             p.l_start[li] = base; p.l_len[li] = nd;
+            if (EXACT) p.l_key[li] = p.key_base + i;          // the pool's first record: any position inside the group orders alike
 #pragma unroll
             for (int k = 0; k < FUSED_DR; k++) if ((uint32_t)k < nd) p.l_fid[base + k] = (int32_t)dr[k];
             for (uint32_t k = FUSED_DR; k < nd; k++) p.l_fid[base + k] = df[k];

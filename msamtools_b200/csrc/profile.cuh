@@ -17,6 +17,7 @@
 // lists into a CSR that the EM kernels iterate.
 #pragma once
 #include "common.cuh"
+#include "collate.cuh"
 #include <cooperative_groups.h>
 
 namespace msg {
@@ -40,6 +41,8 @@ struct ProfParams {
     uint32_t big_cap;
     uint32_t big_threshold;
     uint32_t *err;
+    unsigned long long *key;     // exact mode: [list] key_base + stream position of the list's group head (its input order)
+    unsigned long long key_base; // records pushed before this chunk
 };
 
 __device__ __forceinline__ uint32_t stream_at(const ProfParams &p, uint64_t j) { return p.stream ? p.stream[j] : (uint32_t)j; }
@@ -126,6 +129,8 @@ __device__ __forceinline__ bool group_head(const ProfParams &p, uint64_t j, uint
 // ---- head-walks-its-group path (worklist fallback; exact for any group size) ----------------
 // Applies the share rule of the group headed at stream position j; returns list length for
 // proportional mode (0 otherwise).  ins/uq/mu are incremented for the caller's counters.
+// EXACT (msg_config.exact): an insert that would add 1/n to d[] becomes a list instead (d is summed at finish, in order).
+template <bool EXACT>
 __device__ __forceinline__ uint32_t count_group_walk(const ProfParams &p, uint64_t j, uint32_t r, uint32_t &ins, uint32_t &uq, uint32_t &mu)
 {
     int32_t f0 = -1, f1 = -1; uint32_t size = 0, pc = 0;
@@ -142,6 +147,7 @@ __device__ __forceinline__ uint32_t count_group_walk(const ProfParams &p, uint64
             case 1: walk_group(p, j, r, &size, ActAddUi{p.ui, 2u}, p.big_threshold); break;               // :99-102,169-173
             case 2:
                 if (size == 2) { atomicAdd(p.ui + f0, 1u); atomicAdd(p.ui + f1, 1u); }                    // :103-106
+                else if (EXACT) pc = nd;
                 else walk_group(p, j, r, &size, ActAddD{p.d, 1.0 / (int)nd}, p.big_threshold);            // :175-182
                 break;
             case 3: pc = nd; break;                                                                        // :107-121,184-186
@@ -152,13 +158,14 @@ __device__ __forceinline__ uint32_t count_group_walk(const ProfParams &p, uint64
     return pc;
 }
 
+template <bool EXACT>
 __global__ void __launch_bounds__(256) profile_walk_count_kernel(const ProfParams p, const uint32_t *worklist, const uint32_t *wl_count)
 {
     const uint32_t nw = *wl_count;
     uint32_t ins = 0, uq = 0, mu = 0;
     for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < nw; q += gridDim.x * blockDim.x) {
         const uint64_t j = worklist[q];
-        const uint32_t pc = count_group_walk(p, j, stream_at(p, j), ins, uq, mu);
+        const uint32_t pc = count_group_walk<EXACT>(p, j, stream_at(p, j), ins, uq, mu);
         if (p.pcount) p.pcount[j] = pc;
     }
     ins = __reduce_add_sync(0xffffffffu, ins); uq = __reduce_add_sync(0xffffffffu, uq); mu = __reduce_add_sync(0xffffffffu, mu);
@@ -170,6 +177,7 @@ __global__ void __launch_bounds__(256) profile_walk_count_kernel(const ProfParam
 }
 
 // proportional: worklist heads with pcount>0 write their list; scanv[j] = (lists before << 32) | entries before
+template <bool EXACT>
 __global__ void __launch_bounds__(256) profile_walk_fill_kernel(const ProfParams p, const unsigned long long *scanv, uint32_t *mm_off, uint32_t *mm_len, int32_t *mm_fid,
                                                                 uint32_t list_base, uint32_t ent_base, const uint32_t *worklist, const uint32_t *wl_count)
 {
@@ -180,6 +188,7 @@ __global__ void __launch_bounds__(256) profile_walk_fill_kernel(const ProfParams
         const unsigned long long sv = scanv[j];
         const uint32_t li = list_base + (uint32_t)(sv >> 32), eo = ent_base + (uint32_t)sv;
         mm_off[li] = eo; mm_len[li] = p.pcount[j];
+        if (EXACT) p.key[li] = p.key_base + j;
         uint32_t size;
         walk_group(p, j, stream_at(p, j), &size, ActStore{mm_fid + eo}, p.big_threshold);
     }
@@ -256,7 +265,7 @@ __device__ __forceinline__ GroupView group_view(const ProfParams &p, uint64_t j,
     return v;
 }
 
-template <bool SMEM_HIST>
+template <bool SMEM_HIST, bool EXACT>
 __global__ void __launch_bounds__(256) profile_warp_count_kernel(const ProfParams p, uint8_t *gmeta, uint32_t *worklist, uint32_t *wl_count)
 {
     extern __shared__ uint32_t s_hist[];                 // SMEM_HIST: CTA-private ui histogram (small feature sets)
@@ -286,10 +295,11 @@ __global__ void __launch_bounds__(256) profile_warp_count_kernel(const ProfParam
                 if (p.share_type == 1) atomicAdd(ui + v.feat, 2u);                                   // :99-102,169-173
                 else if (p.share_type == 2) {
                     if (size == 2) atomicAdd(ui + v.feat, 1u);                                       // :103-106
-                    else atomicAdd(p.d + v.feat, 1.0 / (int)nd);                                     // :175-182
+                    else if (!EXACT) atomicAdd(p.d + v.feat, 1.0 / (int)nd);                         // :175-182
                 }
             }
             if (v.head && multi && p.share_type == 3) pc = nd;                                       // :107-121,184-186
+            if (EXACT && v.head && multi && p.share_type == 2 && size != 2) pc = nd;
         }
         if (j < p.m) {
             if (p.pcount) p.pcount[j] = pc;
@@ -310,6 +320,7 @@ __global__ void __launch_bounds__(256) profile_warp_count_kernel(const ProfParam
 
 // proportional: first-appearance lanes of in-window multi groups write their feature at
 // (list offset of the head) + (rank among the group's first appearances)
+template <bool EXACT>
 __global__ void __launch_bounds__(256) profile_warp_fill_kernel(const ProfParams p, const uint8_t *gmeta, const unsigned long long *scanv,
                                                                 uint32_t *mm_off, uint32_t *mm_len, int32_t *mm_fid, uint32_t list_base, uint32_t ent_base)
 {
@@ -332,7 +343,7 @@ __global__ void __launch_bounds__(256) profile_warp_fill_kernel(const ProfParams
     sv = __shfl_sync(0xffffffffu, sv, (int)gs);
     if (member && le && hpc) {
         const uint32_t li = list_base + (uint32_t)(sv >> 32), eo = ent_base + (uint32_t)sv;
-        if (head) { mm_off[li] = eo; mm_len[li] = hpc; }
+        if (head) { mm_off[li] = eo; mm_len[li] = hpc; if (EXACT) p.key[li] = p.key_base + j; }
         if (first) {
             const uint32_t rank = __popc(fmask & span & ((1u << lane) - 1u));
             mm_fid[eo + rank] = feature_of(p, p.tid[stream_at(p, j)]);
@@ -342,12 +353,14 @@ __global__ void __launch_bounds__(256) profile_warp_fill_kernel(const ProfParams
 
 // Oversized groups (> big_threshold records): one thread, the reference's own
 // ub_target_hit stamp algorithm (msam_profile.c:131-145) with a u32 stamp per feature.
-// Lists for proportional mode are appended to big_fid / big_off.
+// Lists for proportional mode (and, EXACT, the equal-share lists) are appended to big_fid / big_off.
+template <bool EXACT>
 __global__ void profile_big_kernel(const ProfParams p, uint32_t nbig, uint32_t *stamp, uint32_t stamp_base,
                                    uint32_t *big_off, uint32_t *big_len, int32_t *big_fid, uint32_t *big_tot /*[0]=lists,[1]=entries*/, int fill,
                                    uint32_t list_base, uint32_t ent_base)
 {
     if (blockIdx.x || threadIdx.x) return;
+    const bool lists = p.share_type == 3 || (EXACT && p.share_type == 2);
     uint32_t nl = fill ? list_base : 0, ne = fill ? ent_base : 0;
     for (uint32_t b = 0; b < nbig; b++) {
         const uint64_t j = p.big[b];
@@ -365,7 +378,7 @@ __global__ void profile_big_kernel(const ProfParams p, uint32_t nbig, uint32_t *
             int32_t f = feature_of(p, tt);
             if (stamp[f] != st) {
                 stamp[f] = st;
-                if (fill && p.share_type == 3) big_fid[ne] = f;
+                if (fill && lists) big_fid[ne] = f;
                 ne++; nd++;
             }
         }
@@ -375,7 +388,7 @@ __global__ void profile_big_kernel(const ProfParams p, uint32_t nbig, uint32_t *
             if (nd == 1) { atomicAdd(p.ui + feature_of(p, p.tid[r0]), 2u); atomicAdd(p.counters + 1, 1u); ne = e0; }
             else {
                 atomicAdd(p.counters + 2, 1u);
-                if (p.share_type == 1 || p.share_type == 2) {
+                if (p.share_type == 1 || (!EXACT && p.share_type == 2)) {
                     // second walk with a fresh stamp to apply the adds
                     const uint32_t st2 = st | 0x80000000u;
                     for (uint64_t jj = j; jj < p.m; jj++) {
@@ -392,12 +405,12 @@ __global__ void profile_big_kernel(const ProfParams p, uint32_t nbig, uint32_t *
                         }
                     }
                 }
-                if (p.share_type != 3) ne = e0;
+                if (!lists) ne = e0;
             }
-            if (p.share_type == 3 && nd > 1) nl++;
+            if (lists && nd > 1) nl++;
         } else {
-            if (nd == 1 || p.share_type != 3) ne = e0;
-            else { big_off[nl] = e0; big_len[nl] = ne - e0; nl++; }
+            if (nd == 1 || !lists) ne = e0;
+            else { big_off[nl] = e0; big_len[nl] = ne - e0; if (EXACT) p.key[nl] = p.key_base + j; nl++; }
         }
     }
     if (!fill) { big_tot[0] = nl; big_tot[1] = ne; }
@@ -655,6 +668,201 @@ __global__ void __launch_bounds__(256) em_loop_smem_kernel(const uint32_t *mm_of
     if (gtid == 0) { result[0] = k < 20 ? k : 19; result[1] = conv; }
     // from this CTA's own (identical) copy of a[]
     em_count_purged(gtid, gsz, mm_off, mm_len, mm_fid, nlists, sa, reinterpret_cast<uint32_t *>(result + 3));
+}
+
+// ---------------------------------------------------------------- exact mode (msg_config.exact)
+// The reference adds every feature's shares in the input order of the lists (msam_profile.c:341-365, :175-182).  Exact
+// mode does the same: the per-feature incidence ibeg[f] .. ibeg[f+1] of ilist[] holds the lists that contain f, sorted by
+// their input key (built once per finish after pushes, from a histogram, run_scan, a scatter and collate.cuh's bucket
+// sorts), and each feature's shares are added in that order, one after another.  Every f64 operation is uncontracted
+// (__dadd_rn / __dmul_rn / __ddiv_rn): the reference's x86-64 build does not fuse a*b + c.  With the same IEEE
+// operations in the same order, abundances, deltas and stop decisions are bit-identical to the reference's.
+
+// the incidence of one feature: lists ilist[b .. e); e of the last feature is the entry total
+__device__ __forceinline__ void exact_range(const uint32_t *ibeg, uint32_t F, unsigned long long nent, uint32_t f, uint32_t &b, uint32_t &e)
+{
+    b = ibeg[f]; e = f + 1 < F ? ibeg[f + 1] : (uint32_t)nent;
+}
+
+// transpose, step 1: entries per feature
+__global__ void __launch_bounds__(256) exact_hist_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists, uint32_t *hist)
+{
+    for (uint32_t l = blockIdx.x * blockDim.x + threadIdx.x; l < nlists; l += gridDim.x * blockDim.x)
+        for (uint32_t q = mm_off[l], e = q + mm_len[l]; q < e; q++) atomicAdd(hist + mm_fid[q], 1u);
+}
+// step 2 (after run_scan): {key, list} into the feature's bucket; cursor[] starts as the bucket starts.  The order inside a
+// bucket does not matter: the bucket sort orders it by (key, list index).
+__global__ void __launch_bounds__(256) exact_scatter_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
+                                                            const unsigned long long *key, uint32_t *cursor, CollKey *out)
+{
+    for (uint32_t l = blockIdx.x * blockDim.x + threadIdx.x; l < nlists; l += gridDim.x * blockDim.x) {
+        CollKey k; k.hash = key[l]; k.ord = l; k.pad = 0;
+        for (uint32_t q = mm_off[l], e = q + mm_len[l]; q < e; q++) out[atomicAdd(cursor + mm_fid[q], 1u)] = k;
+    }
+}
+// step 3 (after the bucket sorts): the list indices alone
+__global__ void __launch_bounds__(256) exact_lists_kernel(const CollKey *keys, unsigned long long n, uint32_t *ilist)
+{
+    for (unsigned long long q = blockIdx.x * blockDim.x + threadIdx.x; q < n; q += (unsigned long long)gridDim.x * blockDim.x) ilist[q] = keys[q].ord;
+}
+
+// Phase 1: s_l = sum of a[f] in list order, from 0 (:341-350)
+__device__ __forceinline__ void em_exact_list_sums(uint32_t first, uint32_t stride, const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid,
+                                                   uint32_t nlists, const double *av, double *sums)
+{
+    for (uint32_t l = first; l < nlists; l += stride) {
+        double s = 0.0;
+        for (uint32_t q = mm_off[l], e = q + mm_len[l]; q < e; q++) s = __dadd_rn(s, __ldcg(av + mm_fid[q]));
+        sums[l] = s;
+    }
+}
+
+// The share list l gives feature f: PropSharing a[f] / s_l for s_l > 0 (:351-365), a true division; equal 1 / n (:175-182)
+struct ExactShareProp { const double *sums, *av;
+    __device__ __forceinline__ bool operator()(uint32_t l, uint32_t f, double &v) const {
+        const double s = __ldcg(sums + l);
+        if (!(s > 0)) return false;
+        v = __ddiv_rn(__ldcg(av + f), s); return true;
+    } };
+struct ExactShareEqual { const uint32_t *mm_len;
+    __device__ __forceinline__ bool operator()(uint32_t l, uint32_t, double &v) const { v = __ddiv_rn(1.0, (double)mm_len[l]); return true; } };
+
+// Incidences longer than this are summed by the whole warp: the lanes compute 32 quotients at once and every lane then
+// carries the same chain of adds over them, in order.  Shorter ones are summed by their own lane.
+constexpr uint32_t EXACT_WARP_CHAIN = 32;
+
+// Phase 2: inc[f] = the serial sum, in key order, of the shares of f's lists; put(f, inc) is called once per feature by
+// the lane that owns f.  Features are taken 32 at a time by warps first_warp, first_warp + warp_stride, ...
+template <class Share, class Put>
+__device__ __forceinline__ void em_exact_gather(uint32_t first_warp, uint32_t warp_stride, const uint32_t *ibeg, const uint32_t *ilist,
+                                                uint32_t F, unsigned long long nent, Share share, Put put)
+{
+    const uint32_t lane = threadIdx.x & 31u;
+    for (uint32_t f0 = first_warp * 32u; f0 < F; f0 += warp_stride * 32u) {
+        const uint32_t f = f0 + lane;
+        const bool own = f < F;
+        uint32_t b = 0, e = 0;
+        if (own) exact_range(ibeg, F, nent, f, b, e);
+        const bool chain = e - b > EXACT_WARP_CHAIN;
+        double acc = 0.0;
+        if (!chain)
+            for (uint32_t q = b; q < e; q++) { double v; if (share(ilist[q], f, v)) acc = __dadd_rn(acc, v); }
+        for (uint32_t lm = __ballot_sync(0xffffffffu, chain); lm; lm &= lm - 1u) {
+            const int src = __ffs((int)lm) - 1;
+            const uint32_t fs = __shfl_sync(0xffffffffu, f, src), bs = __shfl_sync(0xffffffffu, b, src), es = __shfl_sync(0xffffffffu, e, src);
+            double cs = 0.0;
+            for (uint32_t q0 = bs; q0 < es; q0 += 32u) {
+                double v = 0.0;
+                const bool ok = q0 + lane < es && share(ilist[q0 + lane], fs, v);
+                const uint32_t okm = __ballot_sync(0xffffffffu, ok);
+                for (int k = 0; k < 32; k++) {
+                    const double vk = __shfl_sync(0xffffffffu, v, k);
+                    if ((okm >> k) & 1u) cs = __dadd_rn(cs, vk);
+                }
+            }
+            if ((int)lane == src) acc = cs;
+        }
+        if (own) put(f, acc);
+    }
+}
+
+// Phase 3 for feature f: a = U + inc, flushed below 1e-20 (em_new_abundance); sq[f] = (a_new - a_old)^2 (:369-379)
+__device__ __forceinline__ double em_exact_update(const double *U, double *a, double *sq, uint32_t f, double inc)
+{
+    const double an = em_new_abundance(U[f], inc);
+    const double diff = __dsub_rn(an, a[f]);
+    const double d2 = __dmul_rn(diff, diff);
+    a[f] = an; sq[f] = d2;
+    return d2;
+}
+
+// Phase 4, the stop decision.  The grid sums the sq[] terms in a tree (em_block_sum) to D_tree = fl(S_tree / F); the
+// reference sums them in order j = 0 .. F-1 to D_seq = fl(S_seq / F).  For F non-negative terms with true sum S, every
+// summation order gives |S_hat - S| <= gamma_{F-1} S, gamma_k = k u / (1 - k u), u = 2^-53 (Higham, Accuracy and
+// Stability, (4.4)).  So S_seq / S_tree lies in [(1-g)/(1+g), (1+g)/(1-g)], g = gamma_{F-1}, and the two correctly
+// rounded divisions by F add a factor (1 +- u) each: D_seq / D_tree lies within 1 +- r, r = 2g + 2u + O(u^2).  For
+// F < 2^31, g <= (F-1) u (1 + 2^-21), so r <= 3 (F + 2) u, with room left for the rounding of D_tree * (1 +- r) below.
+// Outside [D_tree (1 - r), D_tree (1 + r)] the threshold cannot separate the two sums: D_tree decides as D_seq would.
+// Inside it (rare), the sequential sum is taken and used for the decision and for delta.
+__host__ __device__ __forceinline__ bool em_exact_near(double delta_tree, uint32_t F)
+{
+    const double r = 3.0 * ((double)F + 2.0) * 0x1p-53;
+    return delta_tree * (1.0 - r) < 1e-10 && delta_tree * (1.0 + r) >= 1e-10;
+}
+// D_seq: one thread, j = 0 .. F-1 (:377-380)
+__device__ __forceinline__ double em_exact_seq_delta(const double *sq, uint32_t F)
+{
+    double s = 0.0;
+    for (uint32_t j = 0; j < F; j++) s = __dadd_rn(s, __ldcg(sq + j));
+    return __ddiv_rn(s, (double)F);
+}
+
+// The exact loop in one cooperative launch: list sums | barrier | gather + update + per-CTA partial | barrier | every CTA
+// sums the partials in the same order (D_tree) and takes the same decision; near the threshold (or with force_seq, the
+// tests' MSG_EXACT_DELTA=seq) CTA 0 takes D_seq, which every CTA reads after one more barrier.  partial has gridDim.x + 1
+// slots.  result / delta_out as em_loop_kernel.
+__global__ void __launch_bounds__(256) em_loop_exact_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
+                                                            const uint32_t *ibeg, const uint32_t *ilist, unsigned long long nent,
+                                                            const double *U, double *a, double *sums, double *sq, double *partial, uint32_t F,
+                                                            double *delta_out, int32_t *result, int force_seq)
+{
+    namespace cg = cooperative_groups;
+    cg::grid_group grid = cg::this_grid();
+    __shared__ double s_red[256];
+    const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
+    int k = 1, conv = 0;
+    for (; k < 20; k++) {
+        em_exact_list_sums(gtid, gsz, mm_off, mm_len, mm_fid, nlists, a, sums);
+        grid.sync();
+        double dd = 0;
+        em_exact_gather(gtid >> 5, gsz >> 5, ibeg, ilist, F, nent, ExactShareProp{sums, a},
+                        [&](uint32_t f, double inc) { dd = __dadd_rn(dd, em_exact_update(U, a, sq, f, inc)); });
+        const double part = em_block_sum(s_red, dd);
+        if (threadIdx.x == 0) partial[blockIdx.x] = part;
+        grid.sync();
+        double acc = 0;
+        for (uint32_t b = threadIdx.x; b < gridDim.x; b += 256) acc = __dadd_rn(acc, __ldcg(partial + b));
+        double delta = em_block_sum(s_red, acc) / F;
+        __syncthreads();
+        if (force_seq || em_exact_near(delta, F)) {                         // the same decision in every CTA
+            if (gtid == 0) partial[gridDim.x] = em_exact_seq_delta(sq, F);
+            grid.sync();
+            delta = __ldcg(partial + gridDim.x);
+        }
+        if (gtid == 0) delta_out[k - 1] = delta;
+        if (delta < 1e-10) { conv = 1; break; }
+    }
+    if (gtid == 0) { result[0] = k < 20 ? k : 19; result[1] = conv; }
+    em_count_purged(gtid, gsz, mm_off, mm_len, mm_fid, nlists, a, reinterpret_cast<uint32_t *>(result + 3));
+}
+
+// The same phases one launch each, for the host loop
+__global__ void __launch_bounds__(256) em_exact_sums_kernel(const uint32_t *mm_off, const uint32_t *mm_len, const int32_t *mm_fid, uint32_t nlists,
+                                                            const double *a, double *sums)
+{
+    em_exact_list_sums(blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x, mm_off, mm_len, mm_fid, nlists, a, sums);
+}
+__global__ void __launch_bounds__(256) em_exact_gather_kernel(const uint32_t *ibeg, const uint32_t *ilist, unsigned long long nent, const double *sums,
+                                                              const double *U, double *a, double *sq, double *partial, uint32_t F)
+{
+    __shared__ double s_red[256];
+    const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
+    double dd = 0;
+    em_exact_gather(gtid >> 5, gsz >> 5, ibeg, ilist, F, nent, ExactShareProp{sums, a},
+                    [&](uint32_t f, double inc) { dd = __dadd_rn(dd, em_exact_update(U, a, sq, f, inc)); });
+    const double part = em_block_sum(s_red, dd);
+    if (threadIdx.x == 0) partial[blockIdx.x] = part;
+}
+__global__ void em_exact_seq_kernel(const double *sq, uint32_t F, double *delta_out)
+{
+    if (blockIdx.x == 0 && threadIdx.x == 0) *delta_out = em_exact_seq_delta(sq, F);
+}
+// exact --multi=equal: d[f] = the serial sum, in key order, of 1 / n over f's lists
+__global__ void __launch_bounds__(256) em_exact_equal_kernel(const uint32_t *ibeg, const uint32_t *ilist, unsigned long long nent, const uint32_t *mm_len,
+                                                             double *d, uint32_t F)
+{
+    const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
+    em_exact_gather(gtid >> 5, gsz >> 5, ibeg, ilist, F, nent, ExactShareEqual{mm_len}, [&](uint32_t f, double v) { d[f] = v; });
 }
 
 // Multi-GPU PropSharing: counts exchange + the whole loop + the purged total in ONE cooperative kernel per GPU, with
