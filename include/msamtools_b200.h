@@ -34,7 +34,7 @@
  * boundary (see msg_split_point) so that no read group straddles chunks/GPUs --
  * except on a context created with `collate`, which takes records in any order.
  *
- * Collating contexts (msg_config.collate = 1)
+ * Collating contexts (msg_config.collate = 1 or MSG_COLLATE_RANKS)
  *   - chunks need not end on a QNAME boundary; a read's records may be spread over any number of pushes, and a read
  *     may have any number of records.
  *   - msg_push* append the records' heads (everything but SEQ/QUAL) to device memory and complete before returning.
@@ -47,6 +47,25 @@
  *   - msg_kept_count, msg_pull_kept, msg_pull_records and msg_pull_stats return MSG_ESTATE.
  *   - errors found after grouping (MSG_ENOTAG, MSG_ENOAS, MSG_EFORMAT) name the record's input ordinal (0-based,
  *     counted over the scope's pushes) in msg_last_error.
+ *
+ * Collating across ranks (msg_config.collate = MSG_COLLATE_RANKS, n_ranks > 1)
+ *   - one read's records may be pushed on different ranks, in any order and any number of pushes.  The input is rank
+ *     0's pushes, then rank 1's, and so on: a record's global input ordinal is the number of records pushed by lower
+ *     ranks in this scope plus its ordinal among this rank's pushes.
+ *   - at the first collation point after pushes the ranks exchange record heads over NCCL (send/recv) so that every
+ *     QNAME lands on exactly one rank (rank floor(hash * n_ranks / 2^64) of its 64-bit QNAME hash); each rank then
+ *     collates and runs the pipeline on what it received, and msg_finish_profile / msg_finish_coverage combine the
+ *     ranks as usual.  Each rank holds about 1/n_ranks of the heads.
+ *   - results equal those of one collating GPU fed the concatenation: integers exactly, f64 values to rounding, the
+ *     same PropSharing iteration count; they are bit-identical on every rank.
+ *   - msg_finish_profile, msg_finish_coverage and msg_pull_counts are COLLECTIVE: every rank must make each such
+ *     call, in the same order, including ranks that pushed nothing.  msg_reset must be called on every rank.
+ *   - more than 2^32-2 records over all ranks in one scope, or 64 GiB of heads for one rank: MSG_ERANGE on every rank
+ *     before any record moves; a rank without room for what it receives: MSG_ENOMEM on every rank, naming that rank.
+ *   - a push-time MSG_EFORMAT names the ordinal within this rank's pushes.  Errors found after grouping name the
+ *     global input ordinal and its source, "(input record G: rank r, record k of its pushes)", on the rank that found
+ *     them; every other rank returns the same code with "record error on rank q".
+ *   - with n_ranks == 1 it is collate = 1.  Not with exact.
  */
 #ifndef MSAMTOOLS_B200_H
 #define MSAMTOOLS_B200_H
@@ -78,6 +97,9 @@ extern "C" {
 #define MSG_HIT_BEST    1  /* mWriteBestHitBamPool        */
 #define MSG_HIT_UNIQUE  2  /* mWriteUniqueBestHitBamPool  */
 
+/* collate: 1 = group by QNAME on one GPU; MSG_COLLATE_RANKS = also across the ranks of a multi-GPU run */
+#define MSG_COLLATE_RANKS      2
+
 /* share_type: msam_profile.c:5-8 (same numeric values) */
 #define MSG_MULTI_ALL          1
 #define MSG_MULTI_EQUAL        2
@@ -103,8 +125,9 @@ typedef struct msg_config {
     uint8_t  collate;            /* records may come in any order (e.g. sorted by coordinate): the context keeps their
                                     heads (no SEQ/QUAL) on the device and groups them by QNAME at the first
                                     msg_finish_profile / msg_finish_coverage after pushes.  Needs want_profile and/or
-                                    want_coverage, n_ranks == 1; not with want_records / want_kept / want_stats.
-                                    Results equal those of the same records regrouped stably by QNAME (see below).    */
+                                    want_coverage; not with want_records / want_kept / want_stats.  1 needs
+                                    n_ranks == 1; MSG_COLLATE_RANKS (2) also groups across ranks (see above).
+                                    Results equal those of the same records regrouped stably by QNAME (see above).    */
     uint8_t  exact;              /* bit-exact abundances: every feature's --multi=equal shares and PropSharing increments
                                     are added in the input order of their inserts, with the reference's IEEE operations,
                                     instead of by f64 atomics.  Abundances, EM deltas, iterations and purged count are then
@@ -238,7 +261,9 @@ int  msg_pull_stats(msg_ctx *ctx, size_t nrec, int32_t *alen, int32_t *qlen, int
 int  msg_pull_counts(msg_ctx *ctx, uint32_t *ui, double *d);
 /* mInsertCountToAbundanceMatrix: U = ui/2 (+ d | proportional loop).  With n_ranks > 1 every rank
  * must call it and gets the same result: proportional mode combines the ranks inside one
- * cooperative kernel over CUDA-IPC peer memory, the other modes (or MSG_NO_P2P=1) through NCCL.  */
+ * cooperative kernel over CUDA-IPC peer memory, the other modes (or MSG_NO_P2P=1) through NCCL.
+ * On a MSG_COLLATE_RANKS context with n_ranks > 1, msg_pull_counts and msg_finish_coverage are
+ * collective too (the first of these calls after pushes exchanges the records).                  */
 int  msg_finish_profile(msg_ctx *ctx, double *abundance /*[n_features]*/, msg_profile_stats *st);
 /* per target: covered flag, #positions with depth != 0, sum of depths
  * (msam_coverage.c:189-219).  With n_ranks > 1: allreduce first.             */

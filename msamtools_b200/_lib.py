@@ -15,6 +15,7 @@ MSG_OK, MSG_EINVAL, MSG_ENODEV, MSG_ECUDA, MSG_ENOMEM = 0, -1, -2, -3, -4
 MSG_ENOTAG, MSG_ENOAS, MSG_EFORMAT, MSG_ERANGE, MSG_ENCCL, MSG_ESTATE = -5, -6, -7, -8, -9, -10
 HIT_NONE, HIT_BEST, HIT_UNIQUE = 0, 1, 2
 MULTI_ALL, MULTI_EQUAL, MULTI_PROPORTIONAL, MULTI_IGNORE = 1, 2, 3, 4
+MSG_COLLATE_RANKS = 2       # msg_config.collate: group by QNAME across the ranks of a multi-GPU run
 
 
 class MsgConfig(C.Structure):

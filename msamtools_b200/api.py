@@ -50,7 +50,9 @@ class Context:
         cfg.do_filter = int(any_filter if do_filter is None else do_filter)
         cfg.hit_mode = L.HIT_UNIQUE if uniqhit else (L.HIT_BEST if besthit else L.HIT_NONE)
         cfg.invert, cfg.keep_unmapped, cfg.rescore = int(invert), int(keep_unmapped), int(rescore)
-        cfg.collate = int(collate)                 # records in any order: grouped by QNAME on the device at finish
+        # records in any order, grouped by QNAME on the device at finish: True / 1 on one GPU; L.MSG_COLLATE_RANKS (2)
+        # also across ranks (the records are exchanged by QNAME hash; finish, finish_coverage and pull_counts are collective)
+        cfg.collate = int(collate)
         cfg.exact = int(exact)                     # equal / proportional abundances bit-identical to the reference
         cfg.min_length, cfg.ppt, cfg.max_clip = int(l), int(PPT), int(max_clip)
         cfg.want_kept, cfg.want_records, cfg.want_profile = int(kept), int(records), int(profile)

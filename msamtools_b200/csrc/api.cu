@@ -66,6 +66,11 @@ struct NcclApi {
     ncclResult_t (*AllGather)(const void *, void *, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
     const char *(*GetErrorString)(ncclResult_t) = nullptr;
+    // point-to-point, for the record exchange of collation across ranks (MSG_COLLATE_RANKS)
+    ncclResult_t (*Send)(const void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*Recv)(void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*GroupStart)() = nullptr;
+    ncclResult_t (*GroupEnd)() = nullptr;
     bool load(std::string &err) {
         if (h) return true;
         const char *names[] = {"libnccl.so.2", "libnccl.so", nullptr};
@@ -77,6 +82,10 @@ struct NcclApi {
         AllGather = (decltype(AllGather))dlsym(h, "ncclAllGather");
         CommDestroy = (decltype(CommDestroy))dlsym(h, "ncclCommDestroy");
         GetErrorString = (decltype(GetErrorString))dlsym(h, "ncclGetErrorString");
+        Send = (decltype(Send))dlsym(h, "ncclSend");
+        Recv = (decltype(Recv))dlsym(h, "ncclRecv");
+        GroupStart = (decltype(GroupStart))dlsym(h, "ncclGroupStart");
+        GroupEnd = (decltype(GroupEnd))dlsym(h, "ncclGroupEnd");
         if (!GetUniqueId || !CommInitRank || !AllReduce || !CommDestroy) { err = "libnccl is missing required symbols"; return false; }
         return true;
     }
@@ -170,6 +179,11 @@ struct msg_ctx {
     uint64_t coll_n = 0, coll_bytes = 0;       // records and head bytes held in this scope
     bool coll_dirty = false;                   // pushes since the last collation
     bool coll_done = false;                    // a finish collated this scope: the next push starts a new one
+    // collation across ranks (MSG_COLLATE_RANKS, n_ranks > 1): the agreed size matrix and small flags, and the global
+    // input ordinal where each rank's records start in the last exchange (n_ranks + 1 entries); coll_len then holds the
+    // global ordinal of every received record
+    DevBuf coll_xchg;
+    std::vector<unsigned long long> coll_base;
     double decode_ms = 0, total_ms = 0; uint64_t decode_launches = 0, kernel_launches = 0;
     uint64_t h2d_bytes = 0, d2h_bytes = 0;
 };
@@ -819,11 +833,11 @@ uint64_t coll_chunk_records()
     return (uint64_t)std::min<long long>(std::max<long long>(env, 1), 1ll << 24);
 }
 
-// Group everything held by QNAME and run the pipeline over it once (first finish after pushes).
-int collate_run(msg_ctx *c)
+bool coll_across_ranks(const msg_ctx *c) { return c->cfg.collate == MSG_COLLATE_RANKS && c->cfg.n_ranks > 1; }
+
+// Group everything held by QNAME and run the pipeline over it once.
+int collate_local(msg_ctx *c)
 {
-    if (!c->coll_dirty) return MSG_OK;
-    c->coll_dirty = false; c->coll_done = true;
     const uint64_t n = c->coll_n;
     if (n == 0) return MSG_OK;
     static const bool trace = getenv("MSG_TRACE_FINISH") != nullptr;
@@ -836,6 +850,12 @@ int collate_run(msg_ctx *c)
     // ---- partition by the top bits of the hash
     uint32_t bits = 0;
     while (bits < 24 && ((uint64_t)COLL_BUCKET_AVG << bits) < n) bits++;
+    if (coll_across_ranks(c)) {
+        // this rank holds 1/N of the hash space: ceil(log2 N) more bits keep its occupied buckets near COLL_BUCKET_AVG keys
+        uint32_t lg = 0;
+        while ((1u << lg) < (uint32_t)c->cfg.n_ranks) lg++;
+        bits = std::min<uint32_t>(24, bits + lg);
+    }
     const uint32_t nb = 1u << bits;
     if ((rc = coll_grow(c, c->coll_keys2, n * sizeof(CollKey), 0, n, c->coll_bytes))) return rc;
     CU(c->coll_hist.reserve((size_t)nb * 4)); CU(c->coll_bstart.reserve((size_t)nb * 4));
@@ -919,8 +939,14 @@ int collate_run(msg_ctx *c)
             // errors found after grouping name the record's input ordinal, not its grouped position
             if ((rc == MSG_ENOTAG || rc == MSG_ENOAS || rc == MSG_EFORMAT) && c->err_rec != 0xffffffffu && lo + c->err_rec < n) {
                 CollKey k;
-                if (cudaMemcpy(&k, keys + lo + c->err_rec, sizeof k, cudaMemcpyDeviceToHost) == cudaSuccess)
-                    c->err += " (input record " + std::to_string(k.ord) + ")";
+                uint32_t G = 0;
+                if (cudaMemcpy(&k, keys + lo + c->err_rec, sizeof k, cudaMemcpyDeviceToHost) != cudaSuccess) {}
+                else if (!coll_across_ranks(c)) c->err += " (input record " + std::to_string(k.ord) + ")";
+                else if (cudaMemcpy(&G, c->coll_len.as<uint32_t>() + k.ord, 4, cudaMemcpyDeviceToHost) == cudaSuccess) {
+                    const size_t r = std::upper_bound(c->coll_base.begin(), c->coll_base.end(), (unsigned long long)G) - c->coll_base.begin() - 1;
+                    c->err += " (input record " + std::to_string(G) + ": rank " + std::to_string(r) + ", record " +
+                              std::to_string(G - c->coll_base[r]) + " of its pushes)";
+                }
             }
             return rc;
         }
@@ -935,6 +961,184 @@ int collate_run(msg_ctx *c)
         for (auto e : tev) if (e) cudaEventDestroy(e);
     }
     return MSG_OK;
+}
+
+// The sender's half of the exchange: partition this rank's n held keys by destination rank, stably (collate.cuh), into
+// coll_keys2 with each head length in the key's pad word, count records and head bytes per destination into row[], and
+// gather the heads in that order into coll_grouped.  coll_keys2 and coll_grouped are otherwise only used after the
+// exchange, so they are the send buffers.
+int collate_send_prep(msg_ctx *c, uint64_t n, unsigned long long *row)
+{
+    const uint32_t N = (uint32_t)c->cfg.n_ranks, nblk = nblocks(n, COLL_DEST_TILE);
+    const unsigned long long *aoff = c->coll_aoff.as<unsigned long long>();
+    int rc;
+    if ((rc = coll_grow(c, c->coll_keys2, n * sizeof(CollKey), 0, n, c->coll_bytes))) return rc;
+    if ((rc = coll_grow(c, c->coll_goff, (n + 1) * 8, 0, n, c->coll_bytes))) return rc;
+    CU(c->coll_hist.reserve((size_t)N * nblk * 4)); CU(c->coll_bstart.reserve((size_t)N * nblk * 4));
+    uint32_t *cnt = c->coll_hist.as<uint32_t>(), *pos = c->coll_bstart.as<uint32_t>();
+    CollKey *keys2 = c->coll_keys2.as<CollKey>();
+    collate_dest_count_kernel<<<nblk, 256, 12 * (size_t)N, c->stream>>>(c->coll_keys.as<CollKey>(), n, N, aoff, cnt, nblk, row); LAUNCHED(c);
+    if ((rc = run_scan<uint32_t>(c, InU32{cnt}, OutExclU32{pos}, (uint64_t)N * nblk, (uint32_t *)nullptr))) return rc;
+    collate_dest_scatter_kernel<<<nblk, 256, 4 * (size_t)N * (256 / 32 + 1), c->stream>>>(c->coll_keys.as<CollKey>(), n, N, aoff, pos, nblk, keys2); LAUNCHED(c);
+    unsigned long long *goff = c->coll_goff.as<unsigned long long>(), tot = 0;
+    if ((rc = run_scan<unsigned long long>(c, InGroupedLen{keys2, aoff}, OutExclU64{goff}, n, &tot))) return rc;
+    if ((rc = coll_grow(c, c->coll_grouped, tot + 64, 0, n, tot))) return rc;
+    collate_grouped_gather_kernel<<<std::min<uint32_t>(nblocks(n, 8), 148u * 64u), 256, 0, c->stream>>>(keys2, n, c->coll_arena.as<uint8_t>(), aoff, goff,
+                                                                                                         c->coll_grouped.as<uint8_t>()); LAUNCHED(c);
+    return MSG_OK;
+}
+
+// Collation across ranks (MSG_COLLATE_RANKS, n_ranks > 1; DESIGN.md §11): every rank sends each held record head to rank
+// floor(hash * N / 2^64), so that every QNAME ends up on exactly one rank, then collates what it received.  Every
+// decision below is taken from data all ranks share (one allgather, one allreduce), so that no rank enters a collective
+// its peers skip.  *run: some rank pushed since the last collation.  *sent: the send/recv group was issued; an error
+// returned before that is the same on every rank, one after it is not (collate_run_ranks agrees on it).
+int collate_exchange(msg_ctx *c, bool *run, bool *sent)
+{
+    *run = false; *sent = false;
+    const uint32_t N = (uint32_t)c->cfg.n_ranks, me = (uint32_t)c->cfg.rank, R = 2 * N + 2;
+    // a rank without pushes since the last collation sends nothing: its coll_n still counts what it received then
+    const uint64_t n = c->coll_dirty ? c->coll_n : 0;
+    static const bool trace = getenv("MSG_TRACE_FINISH") != nullptr;
+    cudaEvent_t tev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    auto tmark = [&](int k) { if (trace) { cudaEventCreate(&tev[k]); cudaEventRecord(tev[k], c->stream); } };
+    tmark(0);
+    // the size matrix: rank s's row is [records, head bytes] for every destination, then {pushed, failed}
+    CU(c->coll_xchg.reserve((size_t)N * R * 8 + 16));
+    unsigned long long *dm = c->coll_xchg.as<unsigned long long>(), *row = dm + (size_t)me * R;
+    int *d_agree = reinterpret_cast<int *>(dm + (size_t)N * R);
+    CU(cudaMemsetAsync(row, 0, (size_t)R * 8, c->stream));
+    const int prc = n ? collate_send_prep(c, n, row) : MSG_OK;
+    cudaGetLastError();
+    unsigned long long *h_flags = reinterpret_cast<unsigned long long *>(c->h_pin + 100);
+    h_flags[0] = n > 0; h_flags[1] = prc != MSG_OK;
+    CU(cudaMemcpyAsync(row + 2 * N, h_flags, 16, cudaMemcpyHostToDevice, c->stream));
+    tmark(1);
+    NC(g_nccl.AllGather(row, dm, R, ncclUint64, c->comm, c->stream));
+    std::vector<unsigned long long> M((size_t)N * R);
+    CU(cudaMemcpyAsync(M.data(), dm, M.size() * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    auto rec = [&](uint32_t s, uint32_t d) { return M[(size_t)s * R + 2 * d]; };
+    auto byt = [&](uint32_t s, uint32_t d) { return M[(size_t)s * R + 2 * d + 1]; };
+    bool any = false; int failed = -1;
+    for (uint32_t s = 0; s < N; s++) { any = any || M[(size_t)s * R + 2 * N]; if (failed < 0 && M[(size_t)s * R + 2 * N + 1]) failed = (int)s; }
+    if (!any) { for (auto e : tev) if (e) cudaEventDestroy(e); return MSG_OK; }
+    *run = true;
+    c->coll_dirty = false; c->coll_done = true;
+    if (failed >= 0) return prc ? prc : fail(c, MSG_ENOMEM, "collation across ranks: rank %d could not partition its records", failed);
+    std::vector<unsigned long long> base(N + 1, 0);
+    for (uint32_t s = 0; s < N; s++) { unsigned long long t = 0; for (uint32_t d = 0; d < N; d++) t += rec(s, d); base[s + 1] = base[s] + t; }
+    if (base[N] > 0xfffffffeull)                       // input ordinals stay 32-bit
+        return fail(c, MSG_ERANGE, "collation across ranks holds at most 2^32-2 records per scope (%llu pushed over %u ranks)", base[N], N);
+    unsigned long long rn = 0, rb = 0;
+    for (uint32_t d = 0; d < N; d++) {
+        unsigned long long b = 0;
+        for (uint32_t s = 0; s < N; s++) b += byt(s, d);
+        if (b >= (1ull << 36)) return fail(c, MSG_ERANGE, "collation across ranks: rank %u would receive %llu bytes of record heads (at most 64 GiB per rank)", d, b);
+        if (d == me) { rb = b; for (uint32_t s = 0; s < N; s++) rn += rec(s, d); }
+    }
+    // receive buffers: the arena's heads now sit in coll_grouped and the keys in coll_keys2, so the arena, the keys and
+    // the head offsets are free (released first where they must grow, so the peak stays that of one-GPU collation)
+    int arc = MSG_OK;
+    if (rb + 64 > c->coll_arena.cap) c->coll_arena.release();
+    if (rn * sizeof(CollKey) > c->coll_keys.cap) c->coll_keys.release();
+    if ((rn + 1) * 8 > c->coll_aoff.cap) c->coll_aoff.release();
+    arc = coll_grow(c, c->coll_arena, rb + 64, 0, rn, rb);
+    if (!arc) arc = coll_grow(c, c->coll_keys, (rn ? rn : 1) * sizeof(CollKey), 0, rn, rb);
+    if (!arc) arc = coll_grow(c, c->coll_aoff, (rn + 1) * 8, 0, rn, rb);
+    if (!arc && c->coll_len.reserve((rn + 1) * 4) != cudaSuccess) { cudaGetLastError(); arc = fail(c, MSG_ENOMEM, "cannot hold the global ordinals of %llu received records", rn); }
+    int *h_agree = reinterpret_cast<int *>(c->h_pin + 104);
+    *h_agree = arc ? (int)me : (int)N;
+    CU(cudaMemcpyAsync(d_agree, h_agree, 4, cudaMemcpyHostToDevice, c->stream));
+    NC(g_nccl.AllReduce(d_agree, d_agree, 1, ncclInt32, ncclMin, c->comm, c->stream));
+    CU(cudaMemcpyAsync(h_agree, d_agree, 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (*h_agree < (int)N) return arc ? arc : fail(c, MSG_ENOMEM, "collation across ranks: rank %d lacks device memory for the records it receives", *h_agree);
+    if (n) { collate_rebase_kernel<<<nblocks(n, 256), 256, 0, c->stream>>>(c->coll_keys2.as<CollKey>(), n, (uint32_t)base[me]); LAUNCHED(c); }
+    tmark(2);
+    // ---- the exchange: one send / recv pair per peer for keys and for heads, in one group
+    const uint8_t *sk = c->coll_keys2.as<uint8_t>(), *sh = c->coll_grouped.as<uint8_t>();
+    uint8_t *rk = c->coll_keys.as<uint8_t>(), *rh = c->coll_arena.as<uint8_t>();
+    std::vector<unsigned long long> so(N + 1, 0), sb(N + 1, 0), ro(N + 1, 0), rbo(N + 1, 0);
+    for (uint32_t p = 0; p < N; p++) {
+        so[p + 1] = so[p] + rec(me, p); sb[p + 1] = sb[p] + byt(me, p);         // send segments, in destination order
+        ro[p + 1] = ro[p] + rec(p, me); rbo[p + 1] = rbo[p] + byt(p, me);       // receive segments, in source order
+    }
+    const size_t K = sizeof(CollKey);
+    if (rec(me, me)) {
+        CU(cudaMemcpyAsync(rk + ro[me] * K, sk + so[me] * K, rec(me, me) * K, cudaMemcpyDeviceToDevice, c->stream));
+        CU(cudaMemcpyAsync(rh + rbo[me], sh + sb[me], byt(me, me), cudaMemcpyDeviceToDevice, c->stream));
+    }
+    NC(g_nccl.GroupStart());
+    for (uint32_t p = 0; p < N; p++) {
+        if (p == me) continue;
+        if (rec(me, p)) {
+            NC(g_nccl.Send(sk + so[p] * K, rec(me, p) * K, ncclUint8, (int)p, c->comm, c->stream));
+            NC(g_nccl.Send(sh + sb[p], byt(me, p), ncclUint8, (int)p, c->comm, c->stream));
+        }
+        if (rec(p, me)) {
+            NC(g_nccl.Recv(rk + ro[p] * K, rec(p, me) * K, ncclUint8, (int)p, c->comm, c->stream));
+            NC(g_nccl.Recv(rh + rbo[p], byt(p, me), ncclUint8, (int)p, c->comm, c->stream));
+        }
+    }
+    NC(g_nccl.GroupEnd());
+    *sent = true;
+    tmark(3);
+    // ---- what this rank now holds: keys with their receive position as ordinal, head offsets from the carried lengths
+    CollKey *keys = c->coll_keys.as<CollKey>();
+    unsigned long long *aoff = c->coll_aoff.as<unsigned long long>(), tot = 0;
+    if (rn) { collate_recv_kernel<<<nblocks(rn, 256), 256, 0, c->stream>>>(keys, rn, c->coll_len.as<uint32_t>()); LAUNCHED(c); }
+    int rc = run_scan<unsigned long long>(c, InKeyPadLen{keys}, OutExclU64{aoff}, rn, &tot);
+    if (rc) return rc;
+    unsigned long long *h_end = reinterpret_cast<unsigned long long *>(c->h_pin + 84);
+    *h_end = tot;
+    CU(cudaMemcpyAsync(aoff + rn, h_end, 8, cudaMemcpyHostToDevice, c->stream));
+    tmark(4);
+    CU(cudaStreamSynchronize(c->stream));
+    c->coll_n = rn; c->coll_bytes = tot;
+    c->coll_base.assign(base.begin(), base.end());
+    if (trace) {
+        float ms[4] = {0, 0, 0, 0};
+        for (int k = 0; k < 4; k++) cudaEventElapsedTime(&ms[k], tev[k], tev[k + 1]);
+        fprintf(stderr, "[msg collate rank %u] exchange: partition + send gather %.3f ms, agree %.3f ms, send/recv %.3f ms, receive scan %.3f ms; "
+                "sent %llu records, %llu head bytes (%llu to peers); received %llu records, %llu head bytes (%llu from peers)\n",
+                me, ms[0], ms[1], ms[2], ms[3], so[N], sb[N], sb[N] - byt(me, me), rn, tot, tot - byt(me, me));
+        for (auto e : tev) if (e) cudaEventDestroy(e);
+    }
+    return MSG_OK;
+}
+
+// Collation across ranks: the exchange, the local collation and pipeline, then one allreduce (min) of {return code,
+// failing rank}, so that all ranks return the same code before any combine of the counts and no rank's error leaves its
+// peers waiting in a later collective.  The failing rank keeps its own message.
+int collate_run_ranks(msg_ctx *c)
+{
+    bool run = false, sent = false;
+    int rc = collate_exchange(c, &run, &sent);
+    if (!run || (rc && !sent)) return rc;
+    if (!rc) rc = collate_local(c);
+    cudaGetLastError();
+    const int N = c->cfg.n_ranks;
+    int *h = reinterpret_cast<int *>(c->h_pin + 104), *d = reinterpret_cast<int *>(c->coll_xchg.as<unsigned long long>() + (size_t)N * (2 * N + 2));
+    h[0] = rc; h[1] = rc ? c->cfg.rank : N;
+    CU(cudaMemcpyAsync(d, h, 8, cudaMemcpyHostToDevice, c->stream));
+    NC(g_nccl.AllReduce(d, d, 2, ncclInt32, ncclMin, c->comm, c->stream));
+    CU(cudaMemcpyAsync(h, d, 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (h[0] == MSG_OK) return MSG_OK;
+    if (rc) return h[0];
+    const bool record = h[0] == MSG_ENOTAG || h[0] == MSG_ENOAS || h[0] == MSG_EFORMAT;
+    return fail(c, h[0], "%s on rank %d while collating across ranks (see that rank's error)", record ? "record error" : "error", h[1]);
+}
+
+// The first msg_finish_profile / msg_finish_coverage / msg_pull_counts after pushes groups everything held by QNAME and
+// runs the pipeline once; across ranks every such call is collective.
+int collate_run(msg_ctx *c)
+{
+    if (coll_across_ranks(c)) return collate_run_ranks(c);
+    if (!c->coll_dirty) return MSG_OK;
+    c->coll_dirty = false; c->coll_done = true;
+    return collate_local(c);
 }
 
 // Exact mode: the lists that hold each feature, sorted by their input key (profile.cuh, exact mode), built once per
@@ -1046,11 +1250,13 @@ int msg_create(const msg_config *cfg, msg_ctx **out)
     if (cfg->hit_mode > MSG_HIT_UNIQUE) return fail(c, MSG_EINVAL, "bad hit_mode");
     if (cfg->exact && cfg->n_ranks > 1)
         return fail(c, MSG_EINVAL, "exact needs n_ranks == 1: bit-exact sums across GPUs would chain every rank's partial sums after the previous rank's");
+    if (cfg->collate > MSG_COLLATE_RANKS) return fail(c, MSG_EINVAL, "bad collate value %u (0, 1 or MSG_COLLATE_RANKS = 2)", cfg->collate);
     if (cfg->collate) {
         if (!cfg->want_profile && !cfg->want_coverage) return fail(c, MSG_EINVAL, "collate needs want_profile and/or want_coverage");
         if (cfg->want_records || cfg->want_kept || cfg->want_stats)
             return fail(c, MSG_EINVAL, "collate cannot be combined with want_records, want_kept or want_stats: results come per grouped chunk, not per pushed one");
-        if (cfg->n_ranks > 1) return fail(c, MSG_EINVAL, "collate needs n_ranks == 1");
+        if (cfg->n_ranks > 1 && cfg->collate != MSG_COLLATE_RANKS)
+            return fail(c, MSG_EINVAL, "collate = 1 needs n_ranks == 1; with n_ranks > 1 use collate = MSG_COLLATE_RANKS (2), which exchanges records between the ranks");
     }
     int ndev = 0;
     cudaError_t ce = cudaGetDeviceCount(&ndev);
@@ -1153,6 +1359,10 @@ int msg_create(const msg_config *cfg, msg_ctx **out)
         std::string e;
         if (!cfg->nccl_unique_id) { int rc = fail(nullptr, MSG_EINVAL, "n_ranks > 1 requires nccl_unique_id"); msg_destroy(ctx); return rc; }
         if (!g_nccl.load(e)) { int rc = fail(nullptr, MSG_ENCCL, "%s", e.c_str()); msg_destroy(ctx); return rc; }
+        if (g.collate == MSG_COLLATE_RANKS && (!g_nccl.Send || !g_nccl.Recv || !g_nccl.GroupStart || !g_nccl.GroupEnd || !g_nccl.AllGather)) {
+            int rc = fail(nullptr, MSG_ENCCL, "libnccl lacks ncclSend / ncclRecv / ncclGroupStart / ncclGroupEnd / ncclAllGather, which collation across ranks needs");
+            msg_destroy(ctx); return rc;
+        }
         ncclUniqueId id; memcpy(&id, cfg->nccl_unique_id, 128);
         ncclResult_t r = g_nccl.CommInitRank(&ctx->comm, g.n_ranks, id, g.rank);
         if (r != ncclSuccess) { int rc = fail(nullptr, MSG_ENCCL, "ncclCommInitRank failed: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "?"); msg_destroy(ctx); return rc; }
@@ -1214,7 +1424,9 @@ void msg_destroy(msg_ctx *c)
     if (c->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(c->comm);
     DevBuf *bufs[] = {&c->tid, &c->fb, &c->score, &c->hash, &c->nid, &c->st_alen, &c->st_qlen, &c->st_qclip, &c->st_edit,
                       &c->kbase, &c->worklist, &c->gmeta, &c->out_idx, &c->tile_sums, &c->pcount, &c->scanv, &c->biglist, &c->out_len, &c->out_off, &c->plan, &c->out_rec,
-                      &c->csr_off, &c->csr_len, &c->csr_fid, &c->csr_key, &c->ex_beg, &c->ex_cur, &c->ex_keys, &c->ex_big, &c->ex_list, &c->ex_sums, &c->win, &c->t_ui, &c->t_d, &c->t_cnt, &c->t_cov};
+                      &c->csr_off, &c->csr_len, &c->csr_fid, &c->csr_key, &c->ex_beg, &c->ex_cur, &c->ex_keys, &c->ex_big, &c->ex_list, &c->ex_sums, &c->win, &c->t_ui, &c->t_d, &c->t_cnt, &c->t_cov,
+                      &c->coll_arena, &c->coll_aoff, &c->coll_keys, &c->coll_keys2, &c->coll_len, &c->coll_hist, &c->coll_bstart, &c->coll_list,
+                      &c->coll_grouped, &c->coll_goff, &c->coll_xchg};
     for (DevBuf *b : bufs) b->release();
     void *ptrs[] = {c->d_fmap, c->d_tlen, c->d_covbase, c->d_err, c->d_acct, c->d_total, c->d_ui, c->d_d, c->d_counters, c->d_stamp, c->d_U, c->d_a,
                     c->d_inc, c->d_partial, c->d_delta, c->d_purged, c->d_bflag, c->d_wl, c->d_ui_tmp, c->d_d_tmp, c->d_fcnt, c->d_cursor, c->d_diff, c->d_depth, c->d_covered, c->d_touched, c->d_sum, c->d_covbits};

@@ -235,6 +235,100 @@ __global__ void __launch_bounds__(256) collate_grouped_gather_kernel(const CollK
     }
 }
 
+// ---------------------------------------------------------------- across ranks (MSG_COLLATE_RANKS, DESIGN.md §11)
+// A record goes to rank floor(hash * N / 2^64): every rank holds one contiguous range of the hash space, so every QNAME
+// (and every run of one hash) lands whole on one rank, and the ranks' ranges follow hash order.
+__device__ __forceinline__ uint32_t coll_dest(unsigned long long h, uint32_t nr) { return (uint32_t)__umul64hi(h, (unsigned long long)nr); }
+
+constexpr uint32_t COLL_DEST_TILE = 2048;         // keys per CTA of the destination partition (8 rounds of 256)
+
+// Records and head bytes per destination: cnt[d * nblk + b] = records of tile b for rank d (for the stable scatter), and
+// row[2d], row[2d + 1] += records, head bytes for rank d.  Dynamic shared memory: 12 * nr bytes.
+__global__ void __launch_bounds__(256) collate_dest_count_kernel(const CollKey *keys, uint64_t n, uint32_t nr, const unsigned long long *aoff,
+                                                                 uint32_t *cnt, uint32_t nblk, unsigned long long *row)
+{
+    extern __shared__ unsigned long long s_dyn[];
+    unsigned long long *s_bytes = s_dyn;
+    uint32_t *s_cnt = reinterpret_cast<uint32_t *>(s_dyn + nr);
+    for (uint32_t t = threadIdx.x; t < nr; t += blockDim.x) { s_cnt[t] = 0; s_bytes[t] = 0; }
+    __syncthreads();
+    const uint64_t lo = (uint64_t)blockIdx.x * COLL_DEST_TILE;
+    for (uint32_t r = 0; r < COLL_DEST_TILE; r += blockDim.x) {
+        const uint64_t i = lo + r + threadIdx.x;
+        if (i >= n) break;
+        const uint32_t d = coll_dest(keys[i].hash, nr);
+        atomicAdd(s_cnt + d, 1u);
+        atomicAdd(s_bytes + d, aoff[i + 1] - aoff[i]);
+    }
+    __syncthreads();
+    for (uint32_t t = threadIdx.x; t < nr; t += blockDim.x) {
+        cnt[(uint64_t)t * nblk + blockIdx.x] = s_cnt[t];
+        if (s_cnt[t]) { atomicAdd(row + 2 * t, (unsigned long long)s_cnt[t]); atomicAdd(row + 2 * t + 1, s_bytes[t]); }
+    }
+}
+
+// Stable partition by destination: pos[] is the exclusive scan of collate_dest_count_kernel's cnt[], so the keys of one
+// destination keep their input order (the receiver relies on it, see collate_recv_kernel).  out[] gets {hash, ord, head
+// length in pad}.  Dynamic shared memory: 4 * nr * (blockDim / 32 + 1) bytes.
+__global__ void __launch_bounds__(256) collate_dest_scatter_kernel(const CollKey *keys, uint64_t n, uint32_t nr, const unsigned long long *aoff,
+                                                                   const uint32_t *pos, uint32_t nblk, CollKey *out)
+{
+    extern __shared__ uint32_t s_u32[];
+    const uint32_t nwarp = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
+    uint32_t *s_off = s_u32, *s_w = s_u32 + nr;                     // s_w[w * nr + d]: keys of warp w for d in this round
+    for (uint32_t t = threadIdx.x; t < nr; t += blockDim.x) {
+        s_off[t] = pos[(uint64_t)t * nblk + blockIdx.x];
+        for (uint32_t w = 0; w < nwarp; w++) s_w[w * nr + t] = 0;
+    }
+    __syncthreads();
+    const uint64_t lo = (uint64_t)blockIdx.x * COLL_DEST_TILE;
+    for (uint32_t r = 0; r < COLL_DEST_TILE && lo + r < n; r += blockDim.x) {
+        const uint64_t i = lo + r + threadIdx.x;
+        CollKey k; uint32_t d = 0xffffffffu;
+        if (i < n) { k = keys[i]; d = coll_dest(k.hash, nr); }
+        const uint32_t same = __match_any_sync(0xffffffffu, d);
+        const uint32_t rank = __popc(same & ((1u << lane) - 1u));
+        if (i < n && rank == 0) s_w[warp * nr + d] = __popc(same);
+        __syncthreads();
+        if (i < n) {
+            uint32_t p = s_off[d] + rank;
+            for (uint32_t w = 0; w < warp; w++) p += s_w[w * nr + d];
+            k.pad = (uint32_t)(aoff[i + 1] - aoff[i]);
+            out[p] = k;
+        }
+        __syncthreads();
+        for (uint32_t t = threadIdx.x; t < nr; t += blockDim.x) {
+            uint32_t s = 0;
+            for (uint32_t w = 0; w < nwarp; w++) { s += s_w[w * nr + t]; s_w[w * nr + t] = 0; }
+            s_off[t] += s;
+        }
+        __syncthreads();
+    }
+}
+
+// After the send gather: input ordinals of this rank's records become global ones (records pushed by lower ranks + k).
+__global__ void __launch_bounds__(256) collate_rebase_kernel(CollKey *keys, uint64_t n, uint32_t base)
+{
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) keys[i].ord += base;
+}
+
+// Received keys sit in source-rank order, and in input order within each source (stable scatter), so the receive
+// position orders them exactly as their global ordinals do: the position becomes the key's ordinal (the arena index the
+// sorts and gathers use), and gord[] keeps the global ordinal for error messages.
+__global__ void __launch_bounds__(256) collate_recv_kernel(CollKey *keys, uint64_t n, uint32_t *gord)
+{
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    gord[i] = keys[i].ord;
+    keys[i].ord = (uint32_t)i;
+}
+
+struct InKeyPadLen {           // head length carried in a received key's pad word
+    const CollKey *keys;
+    __device__ __forceinline__ unsigned long long operator()(uint64_t i) const { return keys[i].pad; }
+};
+
 // Chunk cuts: the largest grouped position s in (lo, hi] that starts a run of equal hash (*best, atomicMax), and the
 // smallest such start in (hi, end) (*next, atomicMin).
 __global__ void __launch_bounds__(256) collate_cut_kernel(const CollKey *keys, uint64_t lo, uint64_t hi, uint64_t end,
